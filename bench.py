@@ -250,8 +250,18 @@ class Runner:
     def step_device(self, i):
         self._begin()
         a = self.env.SH_step()[0] if self.sh_loop else self.act_dev[i % self.pool]
-        _, rew, _, _, _ = self.env.step(a)
+        _, rew, self.done, _, _ = self.env.step(a)
         self._end(rew)
+
+    def outputs(self):
+        """What the last ``step_device`` handed its caller, on the host: float16 obs widened to float32, the done mask
+        as 0 / 1, the Shack-Hartmann action when the integrator drives the mirror."""
+        e = self.env
+        out = {'obs': e.obs.float(), 'obs_f64': e.obs_f64, 'reward': e.reward, 'power': e.power,
+               'done': self.done.float()}
+        if self.sh_loop:
+            out['sh_action'] = e.sh_action
+        return {k: v.cpu().numpy() for k, v in out.items()}
 
     def step_e2e(self, i):
         self._begin()
@@ -298,6 +308,24 @@ def timed(r, fn, steps, warmup, world, dist):
     return ms, launches, r.resets - r0
 
 
+DUMP_LIMIT = 64 * 10 ** 6     # bytes written by --dump-outputs, .npy headers included
+
+
+def dump_outputs(arrays, out_dir):
+    """Write each [B, ...] array as out_dir/<name>.npy.  When they would exceed DUMP_LIMIT, every array keeps the same
+    fixed, seeded sample of env rows, whose indices go to env_index.npy."""
+    import numpy as np
+    B = len(next(iter(arrays.values())))
+    row = sum(a.nbytes for a in arrays.values()) // B
+    if B * row > DUMP_LIMIT - 4096:
+        keep = np.sort(np.random.default_rng(0).choice(B, (DUMP_LIMIT - 4096) // (row + 8), replace=False))
+        arrays = {k: a[keep] for k, a in arrays.items()}
+        arrays['env_index'] = keep.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + '.npy'), a)
+
+
 def kernel_times(r, prec, n=6):
     """median per-kernel milliseconds of one step (CUDA events on the launch stream inside the library)"""
     import torch
@@ -330,12 +358,17 @@ def main():
     ap.add_argument('--no-cpu-baseline', action='store_true')
     ap.add_argument('--no-mft-arm', action='store_true', help='skip the secondary timing of the tensor-core MFT path')
     ap.add_argument('--no-workloads', action='store_true', help='skip the short runs of the other BASELINE configs')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='write what the last timed step returned (rank 0\'s envs) as DIR/<name>.npy, to compare builds '
+                         'output for output: the inputs depend only on the arguments')
     ap.add_argument('--cpu-worker', action='store_true', help=argparse.SUPPRESS)
     args = ap.parse_args()
     if args.cpu_worker:
         return cpu_worker(args)
     if args.warmup < 3:
         args.warmup = 3
+    if args.dump_outputs and args.impl != 'b200':
+        ap.error('--dump-outputs needs --impl b200')
     if args.impl == 'reference':
         return run_reference(args)
 
@@ -361,6 +394,7 @@ def main():
     if sampler:
         sampler.start()
     ms, launches, resets = timed(run, run.step_device, args.steps, args.warmup, world, dist)
+    outputs = run.outputs() if args.dump_outputs and rank == 0 else None
     value = world * B * args.steps / (ms * 1e-3)
     ms_e2e, _, _ = timed(run, run.step_e2e, args.steps, args.warmup, world, dist)
     e2e = world * B * args.steps / (ms_e2e * 1e-3)
@@ -568,6 +602,8 @@ def main():
         line['mft_gemm_path'] = mft_arm
     if workloads:
         line['workloads'] = workloads
+    if outputs:
+        dump_outputs(outputs, args.dump_outputs)
     print(json.dumps(line), flush=True)
     if world > 1:
         dist.barrier()

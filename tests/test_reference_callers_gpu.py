@@ -6,9 +6,10 @@
 the reference wrote them; only ``ALGORITHM.learn`` is replaced by "one rollout" so the test ends in seconds, and
 ``gymnasium`` / ``matplotlib`` (absent from this image) are stood in for by ``_gym_compat`` and a no-op stub.
 
-The caller files are looked up in ``$AOG_REFERENCE_DIR``, ``/root/reference`` or ``baseline/_ref/callers``
-(``tools/stage_reference_callers.py``; git-ignored, travels to the GPU box) and must match the committed SHA-256
-manifest -- no reference file is edited.  Our ``gym_AO`` sits AHEAD of the reference's on ``sys.path``.
+The caller files are the reference project's own sources, which this repository does not carry: they are looked up
+in ``$AOG_REFERENCE_DIR`` or ``baseline/_ref/callers`` (``tools/stage_reference_callers.py``; git-ignored), the test
+skips without them, and they must match the committed SHA-256 manifest -- no reference file is edited.  Our
+``gym_AO`` sits AHEAD of the reference's on ``sys.path``.
 """
 import argparse
 import hashlib
@@ -27,7 +28,7 @@ CALLERS = ['main.py', 'algorithm.py', 'network.py', 'replay_buffer.py', 'eval_po
 
 
 def _find_callers():
-    for d in (os.environ.get('AOG_REFERENCE_DIR'), '/root/reference', os.path.join(ROOT, 'baseline', '_ref', 'callers')):
+    for d in (os.environ.get('AOG_REFERENCE_DIR'), os.path.join(ROOT, 'baseline', '_ref', 'callers')):
         if d and all(os.path.exists(os.path.join(d, f)) for f in CALLERS):
             return d
     return None
