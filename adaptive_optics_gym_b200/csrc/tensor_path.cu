@@ -31,6 +31,7 @@
 // plane: it projects it on the fibre modes (AO_env.py:471) out of TMEM.
 #include "tensor_path.cuh"
 #include "kernels_f64.cuh"
+#include "phase_round.cuh"
 
 #include <cuda.h>
 #include <algorithm>
@@ -898,10 +899,14 @@ k_dm_phase_tc(const __grid_constant__ CUtensorMap tmAct_hi, const __grid_constan
       mbar_wait(&tmem_full[as], (it >> 1) & 1, p.err_flag, 14);
       tc_fence_after();
       const bool valid = env < p.num_envs;
-      // obs-arm column sums of this item: (re, im) per row; MODE 2: (ac, bs, as, bc) per conjugate pair, (ac, as) centre
-      double obs_re[NOBS], obs_im[NOBS];
+      // This item's sums over my chunks (at most 5 = 80 pixels) in FP32, folded into FP64 once per item: obs-arm
+      // (re, im) per row, MODE 2: (ac, bs, as, bc) per conjugate pair, (ac, as) centre; fibre projections; Strehl.
+      constexpr int NPP = SYM ? 4 * (NOBS / 2) + 2 * (NOBS & 1) : 2 * NOBS;
+      float pp[NPP], fre[FK_JT], fim[FK_JT];
 #pragma unroll
-      for (int v = 0; v < NOBS; ++v) obs_re[v] = obs_im[v] = 0.0;
+      for (int v = 0; v < NPP; ++v) pp[v] = 0.f;
+#pragma unroll
+      for (int k = 0; k < FK_JT; ++k) fre[k] = fim[k] = 0.f;
       constexpr int kmask = 0x7FFFFF, kexp = 0x4B000000;
       float sre = 0.f, sim = 0.f;
       const int run_first = run_s[2 * x], run_end = run_first + run_s[2 * x + 1];
@@ -942,11 +947,6 @@ k_dm_phase_tc(const __grid_constant__ CUtensorMap tmAct_hi, const __grid_constan
           const float4* tab = reinterpret_cast<const float4*>(pf_warp_ptr + cb * PF_SLOT + FK_PF_TILE);   // [16 y][NF / 4]
           const int32_t q31 = (int32_t)(p.sci_ratio_q32 >> 1);
           const int32_t sci_bias = (1 << 22) - 2 * (int32_t)(((long long)(1 << 22) * (long long)q31) >> 32);
-          float pp[4 * NP2 + 2 * NC + 1], fre[FK_JT], fim[FK_JT];
-#pragma unroll
-          for (int v = 0; v < 4 * NP2 + 2 * NC + 1; ++v) pp[v] = 0.f;
-#pragma unroll
-          for (int k = 0; k < FK_JT; ++k) fre[k] = fim[k] = 0.f;
 #pragma unroll
           for (int j = 0; j < 16; ++j) {
             if (LATE_TILE && j == 8) {
@@ -956,7 +956,7 @@ k_dm_phase_tc(const __grid_constant__ CUtensorMap tmAct_hi, const __grid_constan
                 t[4 * jj] = h.x; t[4 * jj + 1] = h.y; t[4 * jj + 2] = h.z; t[4 * jj + 3] = h.w;
               }
             }
-            const int32_t tb = t[j] + __float2int_rn(d[j] * PHI_ONE) + (1 << 22);
+            const int32_t tb = t[j] + phase_fixed_rn(d[j]) + (1 << 22);
             float c0, s0;
             sincos_biased_fma(tb, kmask, kexp, &s0, &c0);
             float4 rec[NF / 4];
@@ -987,32 +987,16 @@ k_dm_phase_tc(const __grid_constant__ CUtensorMap tmAct_hi, const __grid_constan
               sim = fmaf(m[2 * NP2 + NC + FK_JT], ss, sim);
             }
           }
-          // pair v: row v = (ac - bs, as + bc), row n-1-v = (ac + bs, as - bc)
-#pragma unroll
-          for (int v = 0; v < NP2; ++v) {
-            obs_re[v] += (double)pp[4 * v + 0] - (double)pp[4 * v + 1];
-            obs_im[v] += (double)pp[4 * v + 2] + (double)pp[4 * v + 3];
-            obs_re[NOBS - 1 - v] += (double)pp[4 * v + 0] + (double)pp[4 * v + 1];
-            obs_im[NOBS - 1 - v] += (double)pp[4 * v + 2] - (double)pp[4 * v + 3];
-          }
-          if (NC) { obs_re[NP2] += (double)pp[4 * NP2]; obs_im[NP2] += (double)pp[4 * NP2 + 1]; }
-#pragma unroll
-          for (int k = 0; k < FK_JT; ++k) { fb_re[k] += (double)fre[k]; fb_im[k] += (double)fim[k]; }
         } else if constexpr (FUSED) {
           // ---- fused kernel: the whole optics chain of these 16 pixels, nothing leaves the SM
           const float4* tab = reinterpret_cast<const float4*>(pf_warp_ptr + cb * PF_SLOT + FK_PF_TILE);   // [16 y][NT / 2]
           const int32_t q31 = (int32_t)(p.sci_ratio_q32 >> 1);
           // 2 mulhi(tb, q31) + sci_bias = (t lambda_wfs / lambda_sci) + 2^22, with tb = t + 2^22
           const int32_t sci_bias = (1 << 22) - 2 * (int32_t)(((long long)(1 << 22) * (long long)q31) >> 32);
-          float ore[NOBS], oim[NOBS], fre[FK_JT], fim[FK_JT];
-#pragma unroll
-          for (int v = 0; v < NOBS; ++v) ore[v] = oim[v] = 0.f;
-#pragma unroll
-          for (int k = 0; k < FK_JT; ++k) fre[k] = fim[k] = 0.f;
 #pragma unroll
           for (int j = 0; j < 16; ++j) {
             // atmosphere + DM in fixed point (2^22 per half-turn, unreduced), biased by half a turn
-            const int32_t tb = t[j] + __float2int_rn(d[j] * PHI_ONE) + (1 << 22);
+            const int32_t tb = t[j] + phase_fixed_rn(d[j]) + (1 << 22);
             float c0, s0;
             sincos_biased(tb, &s0, &c0);
             float4 rec[NT / 2];
@@ -1021,8 +1005,8 @@ k_dm_phase_tc(const __grid_constant__ CUtensorMap tmAct_hi, const __grid_constan
             const float2* m = reinterpret_cast<const float2*>(rec);   // [obs rows | fibre modes | (aperture, 0)]
 #pragma unroll
             for (int v = 0; v < NOBS; ++v) {
-              ore[v] = fmaf(m[v].x, c0, fmaf(-m[v].y, s0, ore[v]));
-              oim[v] = fmaf(m[v].x, s0, fmaf(m[v].y, c0, oim[v]));
+              pp[2 * v] = fmaf(m[v].x, c0, fmaf(-m[v].y, s0, pp[2 * v]));
+              pp[2 * v + 1] = fmaf(m[v].x, s0, fmaf(m[v].y, c0, pp[2 * v + 1]));
             }
             // c_j = sum_pixels E . G_j (AO_env.py:471 through the back-projected mode)
 #pragma unroll
@@ -1043,15 +1027,11 @@ k_dm_phase_tc(const __grid_constant__ CUtensorMap tmAct_hi, const __grid_constan
               sim = fmaf(m[NOBS + FK_JT].x, ss, sim);
             }
           }
-#pragma unroll
-          for (int v = 0; v < NOBS; ++v) { obs_re[v] += (double)ore[v]; obs_im[v] += (double)oim[v]; }
-#pragma unroll
-          for (int k = 0; k < FK_JT; ++k) { fb_re[k] += (double)fre[k]; fb_im[k] += (double)fim[k]; }
         } else {
           float ph[16];                                                     // total phase at lambda_wfs, [-pi, pi)
 #pragma unroll
           for (int j = 0; j < 16; ++j) {
-            t[j] += __float2int_rn(d[j] * PHI_ONE);                         // atmosphere + DM, fixed point, unreduced
+            t[j] += phase_fixed_rn(d[j]);                                   // atmosphere + DM, fixed point, unreduced
             ph[j] = small_int_to_float((t[j] << 9) >> 9) * (3.14159265358979323846f / PHI_ONE);
           }
           if (!(p.dbg & 1)) {
@@ -1077,10 +1057,6 @@ k_dm_phase_tc(const __grid_constant__ CUtensorMap tmAct_hi, const __grid_constan
             }
           }
           if constexpr (!PHASE_ONLY) {
-            // obs arm: 16-pixel partial sums in FP32, folded into FP64 per chunk
-            float ore[NOBS], oim[NOBS];
-#pragma unroll
-            for (int v = 0; v < NOBS; ++v) ore[v] = oim[v] = 0.f;
 #pragma unroll
             for (int j = 0; j < 16; ++j) {
               float c0, s0;
@@ -1090,12 +1066,10 @@ k_dm_phase_tc(const __grid_constant__ CUtensorMap tmAct_hi, const __grid_constan
 #pragma unroll
               for (int v = 0; v < NOBS; ++v) {
                 const float2 m = m1o_s[v * Np + y0 + j];
-                ore[v] = fmaf(m.x, c0, fmaf(-m.y, s0, ore[v]));
-                oim[v] = fmaf(m.x, s0, fmaf(m.y, c0, oim[v]));
+                pp[2 * v] = fmaf(m.x, c0, fmaf(-m.y, s0, pp[2 * v]));
+                pp[2 * v + 1] = fmaf(m.x, s0, fmaf(m.y, c0, pp[2 * v + 1]));
               }
             }
-#pragma unroll
-            for (int v = 0; v < NOBS; ++v) { obs_re[v] += (double)ore[v]; obs_im[v] += (double)oim[v]; }
           }
           if (STREHL) {
 #pragma unroll
@@ -1114,8 +1088,24 @@ k_dm_phase_tc(const __grid_constant__ CUtensorMap tmAct_hi, const __grid_constan
       if (lane == 0) mbar_arrive(&tmem_empty[as]);       // this warp is done with the accumulator
       if (valid && !PHASE_ONLY) {
         float2* r = p.R4 + (((size_t)env * Np + x) * FK_PARTS + q) * NOBS;
+        if constexpr (SYM) {
+          // pair v: row v = (ac - bs, as + bc), row n-1-v = (ac + bs, as - bc)
+          constexpr int NP2 = NOBS / 2;
 #pragma unroll
-        for (int v = 0; v < NOBS; ++v) r[v] = make_float2((float)obs_re[v], (float)obs_im[v]);
+          for (int v = 0; v < NP2; ++v) {
+            const double ac = pp[4 * v], bs = pp[4 * v + 1], as_ = pp[4 * v + 2], bc = pp[4 * v + 3];
+            r[v] = make_float2((float)(ac - bs), (float)(as_ + bc));
+            r[NOBS - 1 - v] = make_float2((float)(ac + bs), (float)(as_ - bc));
+          }
+          if (NOBS & 1) r[NP2] = make_float2(pp[4 * NP2], pp[4 * NP2 + 1]);
+        } else {
+#pragma unroll
+          for (int v = 0; v < NOBS; ++v) r[v] = make_float2(pp[2 * v], pp[2 * v + 1]);
+        }
+      }
+      if (FUSED) {
+#pragma unroll
+        for (int k = 0; k < FK_JT; ++k) { fb_re[k] += (double)fre[k]; fb_im[k] += (double)fim[k]; }
       }
       if (STREHL) { st_re += (double)sre; st_im += (double)sim; }
     }
