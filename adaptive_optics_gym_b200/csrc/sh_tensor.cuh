@@ -861,7 +861,7 @@ int sh_tensor_optics(aog_env* env, TensorState* ts, int e0, int nB, cudaStream_t
     fp.env0 = e0;
     fp.dbg = 0;
     fp.sci_ratio_q32 = 0;
-    fp.hwt = ts->hwt; fp.apmask = ts->apmask; fp.m1o32 = ts->m1o32; fp.phi = ts->phi; fp.R4 = ts->R4;
+    fp.apmask = ts->apmask; fp.m1o32 = ts->m1o32; fp.phi = ts->phi; fp.R4 = ts->R4;
     fp.strehl_part = env->strehl_part; fp.gfib = nullptr; fp.fib_part = nullptr; fp.err_flag = ts->err_flag;
     int rc = launch_phase<false, 1, 3>(env, ts, fp, cdiv(fp.num_items, fp.items_per_cta), st);
     if (rc) return rc;

@@ -64,6 +64,9 @@ struct TensorState {
   // [env / 32][Np xp][Np / 16 chunks][32 envs][16 pixels], ring-buffered in xp, the four 16-byte pieces of
   // each env row pre-swizzled (piece j at j ^ ((env >> 1) & 3)) so the shared-memory image is conflict free.
   int32_t* hwt = nullptr;
+  // the same tiles as a 5-D tensor [env / 32][Np xp][Np / 16][32][16]: one box = the four 32-env tiles of a 128-env
+  // block at one (column, chunk), 8 KB, for the shared prefetch of the phase kernel's lane groups
+  CUtensorMap tmHwt;
   // total wavefront phase (atmosphere + DM) at lambda_wfs reduced to [-pi, pi) radians, FP32,
   // [chunk][Np / 16 (y chunk)][Np x][16 y] (the 120 columns x 16 pixels one CTA needs per K block are one
   // contiguous 7.5 KB run): written by the phase kernel, read by the stage-1 kernel's field warps, which form
@@ -592,8 +595,12 @@ __host__ __device__ constexpr int FK_NF(int nobs) { return (2 * (nobs / 2) + (no
 __host__ __device__ constexpr int FK_TAB_TILE(int nobs, int mode) {
   return mode == 1 ? 16 * FK_NT(nobs) * 8 : (mode == 2 ? 16 * FK_NF(nobs) * 4 : 0);
 }
-__host__ __device__ constexpr int FK_PF_SLOT(int nobs, int mode) { return FK_PF_TILE + FK_TAB_TILE(nobs, mode); }
-__host__ __device__ constexpr int FK_PF_BYTES(int nobs, int mode) { return FK_EPI_WARPS * 2 * FK_PF_SLOT(nobs, mode); }
+// Prefetch ring of one q group (the four warps, one per TMEM lane group, that walk the same chunk stream): a slot
+// holds one chunk's four 2 KB phase tiles (lane group lg at lg x 2 KB, one tensor copy) and its one record tile.
+constexpr int FK_PF_STAGES = 3;
+constexpr int FK_PF_PHASE = 4 * FK_PF_TILE;             // 8 KB
+__host__ __device__ constexpr int FK_PF_SLOT(int nobs, int mode) { return (FK_PF_PHASE + FK_TAB_TILE(nobs, mode) + 127) & ~127; }
+__host__ __device__ constexpr int FK_PF_BYTES(int nobs, int mode) { return FK_PARTS * FK_PF_STAGES * FK_PF_SLOT(nobs, mode); }
 constexpr int FK_AUX_BAR = 512;
 
 __device__ __forceinline__ uint64_t umma_desc_sw128(uint32_t smem_addr) {
@@ -656,7 +663,6 @@ struct FieldParams {
   int env0;              // first env of the chunk (index into the tiles)
   int dbg;               // AOG_FK_DEBUG bits (tuning experiments only): 1 no phi stores, 2 no prefetch, 4 no TMEM load
   uint32_t sci_ratio_q32; // lambda_wfs / lambda_sci in 0.32 fixed point
-  const int32_t* hwt;    // tiled atmospheric phase (see TensorState::hwt)
   const uint16_t* apmask;
   const float2* m1o32;   // [n][Np] first obs-arm table, FP32
   float* phi;            // [env][Np / 16][Np x][16 y] total phase out, radians in [-pi, pi)
@@ -676,14 +682,14 @@ template <bool STREHL, int NOBS, int MODE, int NP = TC_NP>
 __global__ void __launch_bounds__(FK_THREADS, 1)
 k_dm_phase_tc(const __grid_constant__ CUtensorMap tmAct_hi, const __grid_constant__ CUtensorMap tmAct_lo,
               const __grid_constant__ CUtensorMap tmM_hi, const __grid_constant__ CUtensorMap tmM_lo,
-              const FieldParams p) {
+              const __grid_constant__ CUtensorMap tmHwt, const FieldParams p) {
   static_assert(NP % 16 == 0 && NP <= 256, "pupil size of the phase kernel");
   constexpr int Np = NP;
   constexpr uint32_t TX_BYTES = 2 * FK_A_TILE + 2 * Np * 64 * 2;
   constexpr uint32_t IDESC = umma_idesc_f16(128, Np);
   extern __shared__ uint8_t smem_raw[];
   uint8_t* base = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);   // stays a shared-space pointer
-  uint8_t* pf = base + FK_STAGES * FK_STAGE_BYTES;                       // phase prefetch ring of the epilogue warps
+  uint8_t* pf = base + FK_STAGES * FK_STAGE_BYTES;                       // phase prefetch rings, [FK_PARTS][FK_PF_STAGES]
   constexpr bool FUSED = MODE == 1 || MODE == 2, SYM = MODE == 2, PHASE_ONLY = MODE == 3;
   constexpr int PF_SLOT = FK_PF_SLOT(NOBS, MODE);
   constexpr int NT = FK_NT(NOBS);
@@ -692,8 +698,9 @@ k_dm_phase_tc(const __grid_constant__ CUtensorMap tmAct_hi, const __grid_constan
   uint64_t* empty = full + FK_STAGES;
   uint64_t* tmem_full = empty + FK_STAGES;       // [2]
   uint64_t* tmem_empty = tmem_full + 2;          // [2]
-  uint64_t* pfbar = tmem_empty + 2;              // [FK_EPI_WARPS][2]
-  uint32_t* tmem_ptr = reinterpret_cast<uint32_t*>(pfbar + 2 * FK_EPI_WARPS);
+  uint64_t* pf_full = tmem_empty + 2;            // [FK_PARTS][FK_PF_STAGES]
+  uint64_t* pf_empty = pf_full + FK_PARTS * FK_PF_STAGES;
+  uint32_t* tmem_ptr = reinterpret_cast<uint32_t*>(pf_empty + FK_PARTS * FK_PF_STAGES);
   constexpr int NRED = FUSED ? 1 + FK_JT : 1;                            // Strehl sum + fibre projections
   double2* sred = reinterpret_cast<double2*>(aux + FK_AUX_BAR);          // [NRED][FK_PARTS][128 envs]
   float2* m1o_s = reinterpret_cast<float2*>(sred + NRED * FK_PARTS * 128);   // [n][Np] (not used by the fused kernel)
@@ -715,7 +722,8 @@ k_dm_phase_tc(const __grid_constant__ CUtensorMap tmAct_hi, const __grid_constan
     run_s[2 * xx + 1] = (uint8_t)cnt;     // the aperture is convex: the lit chunks are contiguous
   }
   if (warp == 0 && lane == 0) {
-    for (int s = 0; s < 2 * FK_EPI_WARPS; ++s) mbar_init(&pfbar[s], 1);
+    for (int s = 0; s < FK_PARTS * FK_PF_STAGES; ++s) { mbar_init(&pf_full[s], 1); mbar_init(&pf_empty[s], 4); }
+    asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&tmHwt)) : "memory");
     asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&tmAct_hi)) : "memory");
     asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&tmAct_lo)) : "memory");
     asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&tmM_hi)) : "memory");
@@ -807,16 +815,21 @@ k_dm_phase_tc(const __grid_constant__ CUtensorMap tmAct_hi, const __grid_constan
     int cur_eb = -1;
     int it = 0;
 
-    // Phase prefetch: the warp's 32 envs x 16 pixels of atmospheric phase are one contiguous, pre-swizzled
-    // 2 KB tile: a single cp.async.bulk one chunk ahead of the arithmetic.
-    const uint32_t pf_warp = smem_u32(pf + ew * (2 * PF_SLOT));
-    const uint8_t* pf_warp_ptr = pf + ew * (2 * PF_SLOT);
-    uint64_t* pbar = pfbar + 2 * ew;
-    uint32_t pphase0 = 0, pphase1 = 0;
-    int buf = 0;
     // The lit chunks of all of the CTA's items form ONE stream dealt round-robin to the FK_PARTS warps of a lane
     // group (chunk g of the stream -> warp g % FK_PARTS), so the warps stay within one chunk of each other over
     // the whole kernel instead of per item; the double-buffered accumulator absorbs the per-item difference.
+    //
+    // Phase prefetch: the four warps of a q group (one per lane group) walk the same sub-stream, so they share a
+    // ring of FK_PF_STAGES slots.  Fill k of the group's sub-stream (its four 2 KB phase tiles, one tensor copy, and
+    // its record tile) is issued by the group's warp with lg == k % 4, when that warp starts chunk k - 1; every warp
+    // waits on full[k % S] before it reads chunk k and arrives once on empty[k % S] after it.
+    // Progress: the issue of fill k waits on empty for chunk k - S <= k - 2, which every warp of the group reaches
+    // before chunk k - 1; a warp waits on full[k] only after it has itself passed chunk k - 1, and so has issued
+    // fill k if it is the issuer.  Take the group's lowest chunk m: its warps wait either on full[m] (issued, as the
+    // issuer is at >= m), on empty for chunk m + 1 - S < m (read by all), on tmem_full (items before its own), or at
+    // flush_strehl's bar.sync 1.  None of these waits on a warp that is parked at a later chunk or at bar.sync 1:
+    // the bar.sync before item i needs only the chunks of items < i and the one fill issued ahead across it, whose
+    // empty wait covers chunks of items < i.
     int n_item = item_lo - 1, n_ci = 0, n_end = 0;       // prefetch cursor: chunk n_ci of item n_item
     int n_x = 0, n_base = 0, n_cnt = 0;                  // its column, lit chunks before the item (mod FK_PARTS), its lit count
     auto next_lit = [&]() -> bool {
@@ -831,26 +844,36 @@ k_dm_phase_tc(const __grid_constant__ CUtensorMap tmAct_hi, const __grid_constan
       }
       return true;
     };
-    auto issue_prefetch = [&](int b) {
-      if (lane == 0) {
-        const int eb2 = n_item / Np, x2 = n_x;
-        int xp2 = x2 + p.col_origin;
+    uint8_t* const ring = pf + q * (FK_PF_STAGES * PF_SLOT);
+    uint64_t* const rfull = pf_full + q * FK_PF_STAGES;
+    uint64_t* const rempty = pf_empty + q * FK_PF_STAGES;
+    int r_slot = 0, f_slot = 0, f_turn = 0;              // slot of the chunk being read; slot and issuer (k % 4) of fill k
+    uint32_t r_phase = 0, f_phase = 0;
+    // fill for the chunk at the cursor
+    auto issue_fill = [&]() {
+      if (f_turn == lg && lane == 0) {
+        mbar_wait(&rempty[f_slot], f_phase ^ 1, p.err_flag, 16);
+        int xp2 = n_x + p.col_origin;
         if (xp2 >= Np) xp2 -= Np;
-        const size_t eb32 = (size_t)(p.env0 + eb2 * 128 + lg * 32) >> 5;
-        const int32_t* src = p.hwt + ((eb32 * Np + xp2) * (Np / 16) + n_ci) * (32 * 16);
+        const int eb32 = (p.env0 + (n_item / Np) * 128) >> 5;
+        const uint32_t dst = smem_u32(ring + f_slot * PF_SLOT);
         asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-        mbar_expect_tx(&pbar[b], PF_SLOT);
-        asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                     ::"r"(pf_warp + b * PF_SLOT), "l"(src), "r"((uint32_t)FK_PF_TILE), "r"(smem_u32(&pbar[b])) : "memory");
+        mbar_expect_tx(&rfull[f_slot], FK_PF_PHASE + FK_TAB_TILE(NOBS, MODE));
+        asm volatile(
+            "cp.async.bulk.tensor.5d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %3, %4, %5, %6}], [%2];"
+            ::"r"(dst), "l"(reinterpret_cast<uint64_t>(&tmHwt)), "r"(smem_u32(&rfull[f_slot])), "r"(0), "r"(n_ci), "r"(xp2),
+              "r"(eb32) : "memory");
         if (FUSED) {
-          const uint8_t* gsrc = static_cast<const uint8_t*>(p.gfib) + ((size_t)x2 * (Np / 16) + n_ci) * FK_TAB_TILE(NOBS, MODE);
+          const uint8_t* gsrc = static_cast<const uint8_t*>(p.gfib) + ((size_t)n_x * (Np / 16) + n_ci) * FK_TAB_TILE(NOBS, MODE);
           asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                       ::"r"(pf_warp + b * PF_SLOT + FK_PF_TILE), "l"(gsrc), "r"((uint32_t)FK_TAB_TILE(NOBS, MODE)), "r"(smem_u32(&pbar[b])) : "memory");
+                       ::"r"(dst + FK_PF_PHASE), "l"(gsrc), "r"((uint32_t)FK_TAB_TILE(NOBS, MODE)), "r"(smem_u32(&rfull[f_slot])) : "memory");
         }
       }
+      f_turn = (f_turn + 1) & 3;
+      if (++f_slot == FK_PF_STAGES) { f_slot = 0; f_phase ^= 1; }
     };
     bool n_ok = next_lit();
-    if (n_ok && !(p.dbg & 2)) issue_prefetch(0);
+    if (n_ok && !(p.dbg & 2)) issue_fill();
 
     auto flush_strehl = [&](int eb) {
       // combine the thirds of every env, one partial per (env, CTA slot)
@@ -919,17 +942,14 @@ k_dm_phase_tc(const __grid_constant__ CUtensorMap tmAct_hi, const __grid_constan
         float d[16];
         if (!(p.dbg & 4)) tc_ld16(lane_addr + as * 256 + y0, d);
         else { for (int j = 0; j < 16; ++j) d[j] = 0.01f * j; }
-        // this chunk's phases were requested one chunk ago; request the next lit chunk now
-        const int cb = buf;
-        __syncwarp();
+        // this chunk's fill was issued one chunk ago; issue the next lit chunk's fill now if it is this warp's turn
         if (!(p.dbg & 2)) {
           n_ok = next_lit();
-          if (n_ok) issue_prefetch(cb ^ 1);
-          if (cb == 0) { mbar_wait(&pbar[0], pphase0, p.err_flag, 15); pphase0 ^= 1; }
-          else         { mbar_wait(&pbar[1], pphase1, p.err_flag, 16); pphase1 ^= 1; }
+          if (n_ok) issue_fill();
+          mbar_wait(&rfull[r_slot], r_phase, p.err_flag, 15);
         }
-        buf ^= 1;
-        const uint8_t* tile = pf_warp_ptr + cb * PF_SLOT + lane * 64;
+        const uint8_t* const slot_ptr = ring + r_slot * PF_SLOT;
+        const uint8_t* tile = slot_ptr + lg * FK_PF_TILE + lane * 64;
         const int sw = (lane >> 1) & 3;                                   // pieces were stored at j ^ ((env >> 1) & 3)
         // The Strehl + wide-detector variants sit at the 128-register cap of a 448-thread block: they fetch the second
         // half of the phase tile after the first eight pixels instead of holding all 16 values through the loop.
@@ -944,7 +964,7 @@ k_dm_phase_tc(const __grid_constant__ CUtensorMap tmAct_hi, const __grid_constan
         if constexpr (SYM) {
           // ---- fused kernel, symmetric tables: 12 FMAs per pixel for the obs pair, the three fibre modes and Strehl
           constexpr int NP2 = NOBS / 2, NC = NOBS & 1, NF = FK_NF(NOBS);
-          const float4* tab = reinterpret_cast<const float4*>(pf_warp_ptr + cb * PF_SLOT + FK_PF_TILE);   // [16 y][NF / 4]
+          const float4* tab = reinterpret_cast<const float4*>(slot_ptr + FK_PF_PHASE);   // [16 y][NF / 4]
           const int32_t q31 = (int32_t)(p.sci_ratio_q32 >> 1);
           const int32_t sci_bias = (1 << 22) - 2 * (int32_t)(((long long)(1 << 22) * (long long)q31) >> 32);
 #pragma unroll
@@ -989,7 +1009,7 @@ k_dm_phase_tc(const __grid_constant__ CUtensorMap tmAct_hi, const __grid_constan
           }
         } else if constexpr (FUSED) {
           // ---- fused kernel: the whole optics chain of these 16 pixels, nothing leaves the SM
-          const float4* tab = reinterpret_cast<const float4*>(pf_warp_ptr + cb * PF_SLOT + FK_PF_TILE);   // [16 y][NT / 2]
+          const float4* tab = reinterpret_cast<const float4*>(slot_ptr + FK_PF_PHASE);   // [16 y][NT / 2]
           const int32_t q31 = (int32_t)(p.sci_ratio_q32 >> 1);
           // 2 mulhi(tb, q31) + sci_bias = (t lambda_wfs / lambda_sci) + 2^22, with tb = t + 2^22
           const int32_t sci_bias = (1 << 22) - 2 * (int32_t)(((long long)(1 << 22) * (long long)q31) >> 32);
@@ -1082,6 +1102,11 @@ k_dm_phase_tc(const __grid_constant__ CUtensorMap tmAct_hi, const __grid_constan
             }
           }
         }
+        if (!(p.dbg & 2)) {
+          __syncwarp();                                                   // every lane has read the slot
+          if (lane == 0) mbar_arrive(&rempty[r_slot]);
+        }
+        if (++r_slot == FK_PF_STAGES) { r_slot = 0; r_phase ^= 1; }
       }
       tc_fence_before();
       __syncwarp();
@@ -1758,6 +1783,23 @@ int make_map_32(aog_env* env, CUtensorMap* map, const void* ptr, uint64_t rows, 
   return AOG_OK;
 }
 
+// the phase tiles [blocks of 32 envs][Np][Np / 16][32][16] int32 (TensorState::hwt) as a 5-D tensor; box = the four
+// 32-env tiles of one (column, chunk), 4 x 2 KB, copied as they are (the tiles are swizzled in memory already)
+int make_map_hwt(aog_env* env, CUtensorMap* map, const int32_t* ptr, uint64_t blocks32, int Np) {
+  EncodeTiledFn enc = get_encode();
+  if (!enc) AOG_FAIL(AOG_ERR_CUDA, "cuTensorMapEncodeTiled entry point not found");
+  const uint64_t tile = 32 * 16 * sizeof(int32_t);
+  cuuint64_t dims[5] = {16, 32, (cuuint64_t)Np / 16, (cuuint64_t)Np, (cuuint64_t)blocks32};
+  cuuint64_t strides[4] = {16 * sizeof(int32_t), tile, tile * (Np / 16), tile * (Np / 16) * Np};
+  cuuint32_t box[5] = {16, 32, 1, 1, 4};
+  cuuint32_t estr[5] = {1, 1, 1, 1, 1};
+  CUresult r = enc(map, CU_TENSOR_MAP_DATA_TYPE_INT32, 5, (void*)ptr, dims, strides, box, estr,
+                   CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
+                   CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  if (r != CUDA_SUCCESS) AOG_FAIL(AOG_ERR_CUDA, "cuTensorMapEncodeTiled (phase tiles) failed: " + std::to_string((int)r));
+  return AOG_OK;
+}
+
 template <typename T>
 int talloc(aog_env* env, T** p, size_t count) {
   if (*p) { cudaFree(*p); *p = nullptr; }
@@ -1830,6 +1872,7 @@ int aog_tensor_create(aog_env* env) {
     const size_t tiles = ((B + 127) / 128) * 4 * NPc * (NPc / 16);       // whole 128-env blocks: the prefetch reads them all
     A(talloc(env, &ts->hwt, tiles * 512));
     AOG_CUDA(cudaMemset(ts->hwt, 0, tiles * 512 * sizeof(int32_t)));
+    A(make_map_hwt(env, &ts->tmHwt, ts->hwt, tiles / ((size_t)NPc * (NPc / 16)), NPc));
     env->phase_tiles = ts->hwt;
     env->phase_tiles_unit = (double)PHI_ONE;
   }
@@ -2242,16 +2285,18 @@ namespace {
 template <bool STREHL, int NOBS, int MODE, int NP = TC_NP>
 int launch_phase(aog_env* env, TensorState* ts, const FieldParams& p, int grid, cudaStream_t st) {
   constexpr bool FUSED = MODE == 1 || MODE == 2;
-  const int smem = FK_STAGES * FK_STAGE_BYTES + FK_PF_BYTES(NOBS, MODE) + 1024 + FK_AUX_BAR +
-                   (FUSED ? 1 + FK_JT : 1) * FK_PARTS * 128 * (int)sizeof(double2) +
-                   (FUSED ? 0 : NOBS * NP * (int)sizeof(float2)) + NP * (NP / 16) * (int)sizeof(uint16_t) + 2 * NP;
+  constexpr int smem = FK_STAGES * FK_STAGE_BYTES + FK_PF_BYTES(NOBS, MODE) + 1024 + FK_AUX_BAR +
+                       (FUSED ? 1 + FK_JT : 1) * FK_PARTS * 128 * (int)sizeof(double2) +
+                       (FUSED ? 0 : NOBS * NP * (int)sizeof(float2)) + NP * (NP / 16) * (int)sizeof(uint16_t) + 2 * NP;
+  static_assert(smem <= 227 * 1024, "shared memory of the phase kernel");
   static std::atomic<bool> configured_on[64];   // function attributes are per device: one flag per device ordinal
   std::atomic<bool>& configured = configured_on[env->cfg.device & 63];
   if (!configured.load(std::memory_order_acquire)) {
     AOG_CUDA(cudaFuncSetAttribute(k_dm_phase_tc<STREHL, NOBS, MODE, NP>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
     configured.store(true, std::memory_order_release);
   }
-  k_dm_phase_tc<STREHL, NOBS, MODE, NP><<<grid, FK_THREADS, smem, st>>>(ts->tmAct_hi, ts->tmAct_lo, ts->tmModes_hi, ts->tmModes_lo, p);
+  k_dm_phase_tc<STREHL, NOBS, MODE, NP><<<grid, FK_THREADS, smem, st>>>(ts->tmAct_hi, ts->tmAct_lo, ts->tmModes_hi, ts->tmModes_lo,
+                                                                        ts->tmHwt, p);
   AOG_LAUNCH_CHECK();
   return AOG_OK;
 }
@@ -2348,7 +2393,7 @@ int aog_tensor_optics(aog_env* env, bool flat_dm, bool with_reward, const aog_ou
       fp.env0 = e0;
       { const char* d = getenv("AOG_FK_DEBUG"); fp.dbg = d ? atoi(d) : 0; }
       fp.sci_ratio_q32 = (uint32_t)std::llround(c.wavelength_wfs / c.wavelength_sci * 4294967296.0);
-      fp.hwt = ts->hwt; fp.apmask = ts->apmask; fp.m1o32 = ts->m1o32; fp.phi = ts->phi; fp.R4 = ts->R4;
+      fp.apmask = ts->apmask; fp.m1o32 = ts->m1o32; fp.phi = ts->phi; fp.R4 = ts->R4;
       fp.strehl_part = env->strehl_part;
       fp.gfib = ts->gfib; fp.fib_part = ts->fib_part;
       fp.err_flag = ts->err_flag;

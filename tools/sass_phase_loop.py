@@ -4,8 +4,10 @@
 
 The chunk loop is the innermost backward branch around the kernel's tcgen05.ld (LDTM): its body handles one
 16-pixel chunk per epilogue warp.  For each instantiation <STREHL, NOBS, MODE, NP> this prints the loop's instruction
-count, its XU (conversion / transcendental pipe) instructions, MUFU, F2I and F2F separately, and the mix over the
-pipes below.  Counts are static (both sides of a branch count), CPU only: cuobjdump -sass of the sm_100a cubin."""
+count, its XU (conversion / transcendental pipe) instructions, MUFU, F2I and F2F separately, its bulk and tensor
+copy issues (UBLKCP, UTMALDG), the instructions of the fill path (the innermost BSSY .. BSYNC region that holds those
+copies: the prefetch issue, which a warp runs on every chunk in a per-warp ring and on every fourth chunk in a ring
+shared by four warps), and the mix over the pipes below.  Counts are static (both sides of a branch count), CPU only: cuobjdump -sass of the sm_100a cubin."""
 import argparse
 import collections
 import os
@@ -73,6 +75,26 @@ def chunk_loop(body):
     return [(a, op) for a, op, _ in body if best[0] <= a <= best[1]]
 
 
+COPIES = ('UBLKCP', 'UTMALDG')
+
+
+def fill_path(body, loop):
+    """instructions of the innermost BSSY .. BSYNC region of the loop that holds all of its copy issues"""
+    copies = [a for a, op in loop if op.startswith(COPIES)]
+    if not copies:
+        return 0
+    lo, hi = loop[0][0], loop[-1][0]
+    best = None
+    for a, op, args in body:
+        if not (lo <= a <= hi and op.startswith('BSSY')):
+            continue
+        m = re.search(r'(0x[0-9a-f]+)', args)
+        end = int(m.group(1), 16) if m else -1
+        if a < min(copies) and max(copies) < end and (best is None or end - a < best[1] - best[0]):
+            best = (a, end)
+    return sum(1 for a, _ in loop if best[0] <= a < best[1]) if best else 0
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument('lib', nargs='?', default=os.path.join(ROOT, 'adaptive_optics_gym_b200', 'libaogym.so'))
@@ -89,22 +111,24 @@ def main():
         ops = collections.Counter(op.split('.')[0] for _, op in loop)
         pipes = collections.Counter(pipe_of(op) for _, op in loop)
         key = tuple(int(g) for g in m.groups())
-        rows.append((key, len(loop), pipes['xu'], ops['MUFU'], ops['F2I'], ops['F2F'], pipes))
+        copies = sum(1 for _, op in loop if op.startswith(COPIES))
+        rows.append((key, len(loop), pipes['xu'], ops['MUFU'], ops['F2I'], ops['F2F'], copies, fill_path(body, loop), pipes))
     rows.sort()
     cols = ['fma', 'alu', 'xu', 'fp64', 'lsu', 'tmem', 'uniform', 'sync/branch', 'other']
     if args.md:
-        print('| instantiation | loop instr | XU | MUFU | F2I | F2F | ' + ' | '.join(cols) + ' |')
-        print('|---' * (6 + len(cols)) + '|')
+        print('| instantiation | loop instr | XU | MUFU | F2I | F2F | copies | fill path | ' + ' | '.join(cols) + ' |')
+        print('|---' * (8 + len(cols)) + '|')
     else:
-        print('%-16s %6s %4s %4s %4s %4s  ' % ('<S,NOBS,MODE,NP>', 'instr', 'XU', 'MUFU', 'F2I', 'F2F') +
+        print('%-16s %6s %4s %4s %4s %4s %6s %4s  ' % ('<S,NOBS,MODE,NP>', 'instr', 'XU', 'MUFU', 'F2I', 'F2F', 'copies', 'fill') +
               ' '.join('%7s' % c[:7] for c in cols))
-    for key, n, xu, mufu, f2i, f2f, pipes in rows:
+    for key, n, xu, mufu, f2i, f2f, copies, fill, pipes in rows:
         k = '<%d,%d,%d,%d>' % key
         if args.md:
-            print('| `%s` | %d | %d | %d | %d | %d | ' % (k, n, xu, mufu, f2i, f2f) +
+            print('| `%s` | %d | %d | %d | %d | %d | %d | %d | ' % (k, n, xu, mufu, f2i, f2f, copies, fill) +
                   ' | '.join(str(pipes[c]) for c in cols) + ' |')
         else:
-            print('%-16s %6d %4d %4d %4d %4d  ' % (k, n, xu, mufu, f2i, f2f) + ' '.join('%7d' % pipes[c] for c in cols))
+            print('%-16s %6d %4d %4d %4d %4d %6d %4d  ' % (k, n, xu, mufu, f2i, f2f, copies, fill) +
+                  ' '.join('%7d' % pipes[c] for c in cols))
     return 0 if rows else 1
 
 
