@@ -561,7 +561,7 @@ constexpr int FIN_WARPS = 8;
 template <int N, int PARTS> struct FinCfg {
   static constexpr int XS = 32 / N, LANES = XS * N, N2 = N * N, N2P = N2 < 7 ? 7 : N2;
   static constexpr int ITER = N >= 6 ? 4 : 8, TILE_X = XS * ITER, ROW = PARTS * N /* float2 per pupil column */;
-  static constexpr int TAB_MAX = N * 256 * 16;           // the [N][Np] table, Np <= 256 on the tensor / fused paths
+  static constexpr int TAB_MAX = N * 512 * 16;           // the [N][Np] table, Np <= 512 on the tensor / fused paths
   static constexpr int TILE_BYTES = TILE_X * ROW * 8, WARP_BYTES = 2 * TILE_BYTES, SMEM = FIN_WARPS * WARP_BYTES;
   static constexpr int RED_LD = 33;
   static_assert(TILE_BYTES % 16 == 0, "tile size");

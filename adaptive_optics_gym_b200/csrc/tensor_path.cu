@@ -552,29 +552,33 @@ k_mft2(const __grid_constant__ CUtensorMap tmA_hi, const __grid_constant__ CUten
 // total phase (reduced, FP32 radians) for the stage-1 kernel's field warps, and accumulate in registers the
 // obs-arm column sums R[x][v] = sum_y m1o[v][y] E[y][x] (AO_env.py:139; FP32 per 16 pixels, FP64 across)
 // and the Strehl sum sum_ap exp(i phi lambda_wfs / lambda_sci).
-// Work item = (block of 128 envs, column x); each CTA takes a contiguous range of items.
+// Work item = (block of 128 envs, column x, segment s); each CTA takes a contiguous range of items.  A pupil column
+// longer than 256 pixels (NP = 512) is split into NSEG = 2 segments of SEG = 256 pixels, one MMA (N = SEG) each: the
+// N of one MMA, a TMA box and one half of the double-buffered accumulator all stop at 256.
 constexpr int FK_STAGES = 1;                            // the double-buffered TMEM accumulator hides the operand load
 constexpr int FK_A_TILE = 128 * 64 * 2;                 // 16 KB: 128 env rows x 128 B
 constexpr int FK_B_TILE = 256 * 64 * 2;                 // 32 KB slot (240 rows used)
+__host__ __device__ constexpr int FK_NSEG(int np) { return np > 256 ? 2 : 1; }
 constexpr int FK_STAGE_BYTES = 2 * FK_A_TILE + 2 * FK_B_TILE;   // 96 KB
 #ifndef AOG_FK_EPI_WARPS      // tuning builds: 12 or 16
 #define AOG_FK_EPI_WARPS 12
 #endif
 constexpr int FK_EPI_WARPS = AOG_FK_EPI_WARPS;          // 3 per TMEM lane group: 5 of the 15 column chunks each
 constexpr int FK_PARTS = FK_EPI_WARPS / 4;
-// Work item -> pupil column: a CTA's contiguous item range strides through the pupil (53 is coprime with 240), so
-// every CTA sees the same mix of short (edge) and long (centre) aperture chords.
+// Work item -> column segment xs = x NSEG + s: a CTA's contiguous item range strides through the pupil (53 is coprime
+// with 240 and 1024), so every CTA sees the same mix of short (edge) and long (centre) aperture chords.
 // (The tensor path's phase kernel keeps the natural order: its phase stores of neighbouring columns are neighbours
 // in HBM, and striding them costs more DRAM page misses than the imbalance does.)
 constexpr int FK_COL_STRIDE = 53;
 template <int MODE, int NP>
-__device__ __forceinline__ int fk_column(int item_in_block) {
-  return (MODE == 0 || MODE == 3) ? item_in_block : (item_in_block * FK_COL_STRIDE) % NP;   // 53 is prime: coprime with every NP
+__device__ __forceinline__ int fk_segment(int item_in_block) {
+  // 53 is prime: coprime with every NP NSEG
+  return (MODE == 0 || MODE == 3) ? item_in_block : (item_in_block * FK_COL_STRIDE) % (NP * FK_NSEG(NP));
 }
 constexpr int FK_THREADS = (2 + FK_EPI_WARPS) * 32;     // 448
 
 constexpr int FK_SLOTS = 128;                           // Strehl / fibre partial slots per env (>= CTAs touching an env block)
-constexpr int FK_MIN_ITEMS = 2;                         // items per CTA at least (bounds the slots: 240 / 2 + 1 = 121 <= FK_SLOTS); small batches spread over more SMs
+constexpr int FK_MIN_ITEMS = 2;                         // items per CTA at least (with a bound from FK_SLOTS); small batches spread over more SMs
 constexpr int FK_PF_TILE = 32 * 16 * 4;                 // 2 KB: 32 envs x 16 pixels of phase (one bulk copy)
 constexpr int FK_JT = 3;                                // fibre modes of the fused kernel (LP01 + 2 x LP11, AO_env.py:393)
 // Fused kernel: per pixel one record of FK_NT(n) float2 = [n obs-arm twiddles | FK_JT back-projected fibre modes |
@@ -656,7 +660,7 @@ __device__ __forceinline__ void split_pack2(float a, float b, uint32_t& hi, uint
 
 struct FieldParams {
   int num_envs;          // envs in this chunk
-  int num_items;         // env blocks x 240 columns
+  int num_items;         // env blocks x Np NSEG column segments
   int items_per_cta;
   int nkb;               // KPAD / 64
   int col_origin;
@@ -666,15 +670,16 @@ struct FieldParams {
   const uint16_t* apmask;
   const float2* m1o32;   // [n][Np] first obs-arm table, FP32
   float* phi;            // [env][Np / 16][Np x][16 y] total phase out, radians in [-pi, pi)
-  float2* R4;            // [env][Np x][FK_PARTS][n] obs-arm column partial sums out
+  float2* R4;            // [env][Np x][NSEG FK_PARTS][n] obs-arm column partial sums out (part s FK_PARTS + q)
   double2* strehl_part;  // [env][FK_SLOTS]
   const void* gfib;      // fused kernel: [Np x][Np / 16][16 y] per-pixel records (FK_NT float2 or FK_NF floats each)
   double2* fib_part;     // fused kernel: [env][FK_SLOTS][FK_JT] partial projection sums out
   int* err_flag;
 };
 
-// NP = pupil pixels per side: 240 (the reference, AO_env.py:216) for every mode; 128 and 256 for the fused modes
-// (BASELINE configs[4], the pupil-grid axis).  Any multiple of 16 up to 256 fits the tiles (N of the MMA, TMEM columns).
+// NP = pupil pixels per side: 240 (the reference, AO_env.py:216) for every mode; 128, 256 and 512 for the fused modes
+// (BASELINE configs[4], the pupil-grid axis).  Any multiple of 16 up to 256 fits the tiles (N of the MMA, TMEM columns);
+// 512 runs every column as two 256-pixel segments.
 template <bool STREHL, int NOBS, int MODE, int NP = TC_NP>
 // (448 threads x 144 registers would fit the register file on paper, but warps are allocated in groups of four: a
 // build with __maxnreg__(144) fails to launch every variant above 128 registers.  The Strehl + 5x5-detector variant
@@ -683,14 +688,15 @@ __global__ void __launch_bounds__(FK_THREADS, 1)
 k_dm_phase_tc(const __grid_constant__ CUtensorMap tmAct_hi, const __grid_constant__ CUtensorMap tmAct_lo,
               const __grid_constant__ CUtensorMap tmM_hi, const __grid_constant__ CUtensorMap tmM_lo,
               const __grid_constant__ CUtensorMap tmHwt, const FieldParams p) {
-  static_assert(NP % 16 == 0 && NP <= 256, "pupil size of the phase kernel");
+  constexpr bool FUSED = MODE == 1 || MODE == 2, SYM = MODE == 2, PHASE_ONLY = MODE == 3;
+  static_assert(NP % 16 == 0 && (NP <= 256 || (FUSED && NP == 512)), "pupil size of the phase kernel");
   constexpr int Np = NP;
-  constexpr uint32_t TX_BYTES = 2 * FK_A_TILE + 2 * Np * 64 * 2;
-  constexpr uint32_t IDESC = umma_idesc_f16(128, Np);
+  constexpr int NSEG = FK_NSEG(NP), SEG = NP / NSEG, IPB = NP * NSEG;   // segments per column, pixels each, items per env block
+  constexpr uint32_t TX_BYTES = 2 * FK_A_TILE + 2 * SEG * 64 * 2;
+  constexpr uint32_t IDESC = umma_idesc_f16(128, SEG);
   extern __shared__ uint8_t smem_raw[];
   uint8_t* base = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);   // stays a shared-space pointer
   uint8_t* pf = base + FK_STAGES * FK_STAGE_BYTES;                       // phase prefetch rings, [FK_PARTS][FK_PF_STAGES]
-  constexpr bool FUSED = MODE == 1 || MODE == 2, SYM = MODE == 2, PHASE_ONLY = MODE == 3;
   constexpr int PF_SLOT = FK_PF_SLOT(NOBS, MODE);
   constexpr int NT = FK_NT(NOBS);
   uint8_t* aux = pf + FK_PF_BYTES(NOBS, MODE);
@@ -704,8 +710,10 @@ k_dm_phase_tc(const __grid_constant__ CUtensorMap tmAct_hi, const __grid_constan
   constexpr int NRED = FUSED ? 1 + FK_JT : 1;                            // Strehl sum + fibre projections
   double2* sred = reinterpret_cast<double2*>(aux + FK_AUX_BAR);          // [NRED][FK_PARTS][128 envs]
   float2* m1o_s = reinterpret_cast<float2*>(sred + NRED * FK_PARTS * 128);   // [n][Np] (not used by the fused kernel)
-  uint16_t* apmask_s = reinterpret_cast<uint16_t*>(m1o_s + (FUSED ? 0 : NOBS * Np));  // [Np][Np / 16]
-  uint8_t* run_s = reinterpret_cast<uint8_t*>(apmask_s + Np * (Np / 16));   // [Np][2]: first lit chunk, lit count
+  // [Np][Np / 16] (read by the MODE 0 chunk loop only: not staged for the fused kernel)
+  uint16_t* apmask_s = reinterpret_cast<uint16_t*>(m1o_s + (FUSED ? 0 : NOBS * Np));
+  // [Np NSEG][2]: first lit chunk (index within the whole column), lit count of the segment
+  uint8_t* run_s = reinterpret_cast<uint8_t*>(apmask_s + (FUSED ? 0 : Np * (Np / 16)));
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int item_lo = blockIdx.x * p.items_per_cta;
@@ -713,13 +721,15 @@ k_dm_phase_tc(const __grid_constant__ CUtensorMap tmAct_hi, const __grid_constan
 
   if (!FUSED && !PHASE_ONLY)
     for (int i = threadIdx.x; i < NOBS * Np; i += blockDim.x) m1o_s[i] = p.m1o32[i];
-  for (int i = threadIdx.x; i < Np * (Np / 16); i += blockDim.x) apmask_s[i] = p.apmask[i];
-  for (int xx = threadIdx.x; xx < Np; xx += blockDim.x) {
-    int first = 0, cnt = 0;
-    for (int c = 0; c < Np / 16; ++c)
-      if (p.apmask[xx * (Np / 16) + c]) { if (!cnt) first = c; ++cnt; }
-    run_s[2 * xx] = (uint8_t)first;
-    run_s[2 * xx + 1] = (uint8_t)cnt;     // the aperture is convex: the lit chunks are contiguous
+  if (!FUSED)
+    for (int i = threadIdx.x; i < Np * (Np / 16); i += blockDim.x) apmask_s[i] = p.apmask[i];
+  for (int xs = threadIdx.x; xs < Np * NSEG; xs += blockDim.x) {
+    const int c0 = (xs % NSEG) * (SEG / 16);
+    int first = c0, cnt = 0;
+    for (int c = c0; c < c0 + SEG / 16; ++c)
+      if (p.apmask[(xs / NSEG) * (Np / 16) + c]) { if (!cnt) first = c; ++cnt; }
+    run_s[2 * xs] = (uint8_t)first;
+    run_s[2 * xs + 1] = (uint8_t)cnt;     // the aperture is convex: the lit chunks are contiguous
   }
   if (warp == 0 && lane == 0) {
     for (int s = 0; s < FK_PARTS * FK_PF_STAGES; ++s) { mbar_init(&pf_full[s], 1); mbar_init(&pf_empty[s], 4); }
@@ -748,15 +758,16 @@ k_dm_phase_tc(const __grid_constant__ CUtensorMap tmAct_hi, const __grid_constan
       int stage = 0;
       uint32_t phase = 0;
       for (int item = item_lo; item < item_hi; ++item) {
-        const int eb = item / Np, x = fk_column<MODE, NP>(item - eb * Np);
+        const int eb = item / IPB, xs = fk_segment<MODE, NP>(item - eb * IPB);
+        const int row0 = (xs / NSEG) * Np + (xs % NSEG) * SEG;               // modes rows of pixels (x, s SEG ...)
         for (int kb = 0; kb < p.nkb; ++kb) {
           mbar_wait<200>(&empty[stage], phase ^ 1, p.err_flag, 11);
           mbar_expect_tx(&full[stage], TX_BYTES);
           const uint32_t s0 = smem_u32(base + stage * FK_STAGE_BYTES);
           tma_load_2d(s0, &tmAct_hi, &full[stage], kb * 64, eb * 128);
           tma_load_2d(s0 + FK_A_TILE, &tmAct_lo, &full[stage], kb * 64, eb * 128);
-          tma_load_2d(s0 + 2 * FK_A_TILE, &tmM_hi, &full[stage], kb * 64, x * Np);
-          tma_load_2d(s0 + 2 * FK_A_TILE + FK_B_TILE, &tmM_lo, &full[stage], kb * 64, x * Np);
+          tma_load_2d(s0 + 2 * FK_A_TILE, &tmM_hi, &full[stage], kb * 64, row0);
+          tma_load_2d(s0 + 2 * FK_A_TILE + FK_B_TILE, &tmM_lo, &full[stage], kb * 64, row0);
           if (++stage == FK_STAGES) { stage = 0; phase ^= 1; }
         }
       }
@@ -837,10 +848,11 @@ k_dm_phase_tc(const __grid_constant__ CUtensorMap tmAct_hi, const __grid_constan
       while (n_ci >= n_end) {
         n_base = (n_base + n_cnt) % FK_PARTS;
         if (++n_item >= item_hi) return false;
-        n_x = fk_column<MODE, NP>(n_item - (n_item / Np) * Np);
-        n_cnt = run_s[2 * n_x + 1];
-        n_ci = run_s[2 * n_x] + (q + FK_PARTS - n_base) % FK_PARTS;
-        n_end = run_s[2 * n_x] + n_cnt;
+        const int n_xs = fk_segment<MODE, NP>(n_item - (n_item / IPB) * IPB);
+        n_x = n_xs / NSEG;
+        n_cnt = run_s[2 * n_xs + 1];
+        n_ci = run_s[2 * n_xs] + (q + FK_PARTS - n_base) % FK_PARTS;
+        n_end = run_s[2 * n_xs] + n_cnt;
       }
       return true;
     };
@@ -855,7 +867,7 @@ k_dm_phase_tc(const __grid_constant__ CUtensorMap tmAct_hi, const __grid_constan
         mbar_wait(&rempty[f_slot], f_phase ^ 1, p.err_flag, 16);
         int xp2 = n_x + p.col_origin;
         if (xp2 >= Np) xp2 -= Np;
-        const int eb32 = (p.env0 + (n_item / Np) * 128) >> 5;
+        const int eb32 = (p.env0 + (n_item / IPB) * 128) >> 5;
         const uint32_t dst = smem_u32(ring + f_slot * PF_SLOT);
         asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
         mbar_expect_tx(&rfull[f_slot], FK_PF_PHASE + FK_TAB_TILE(NOBS, MODE));
@@ -886,7 +898,7 @@ k_dm_phase_tc(const __grid_constant__ CUtensorMap tmAct_hi, const __grid_constan
       if (q == 0) {
         const int env = eb * 128 + row;
         if (env < p.num_envs) {
-          const int slot = blockIdx.x - (eb * Np) / p.items_per_cta;
+          const int slot = blockIdx.x - (eb * IPB) / p.items_per_cta;
           if (STREHL) {
             double2 a = sred[row];
             for (int k = 1; k < FK_PARTS; ++k) { a.x += sred[k * 128 + row].x; a.y += sred[k * 128 + row].y; }
@@ -912,7 +924,8 @@ k_dm_phase_tc(const __grid_constant__ CUtensorMap tmAct_hi, const __grid_constan
     };
 
     for (int item = item_lo; item < item_hi; ++item, ++it) {
-      const int eb = item / Np, x = fk_column<MODE, NP>(item - eb * Np);
+      const int eb = item / IPB, xs = fk_segment<MODE, NP>(item - eb * IPB);
+      const int x = xs / NSEG, seg = xs % NSEG;
       if ((STREHL || FUSED) && eb != cur_eb) {
         if (cur_eb >= 0) flush_strehl(cur_eb);
         cur_eb = eb;
@@ -932,15 +945,16 @@ k_dm_phase_tc(const __grid_constant__ CUtensorMap tmAct_hi, const __grid_constan
       for (int k = 0; k < FK_JT; ++k) fre[k] = fim[k] = 0.f;
       constexpr int kmask = 0x7FFFFF, kexp = 0x4B000000;
       float sre = 0.f, sim = 0.f;
-      const int run_first = run_s[2 * x], run_end = run_first + run_s[2 * x + 1];
+      const int run_first = run_s[2 * xs], run_end = run_first + run_s[2 * xs + 1];
       const int my_first = run_first + (q + FK_PARTS - m_base) % FK_PARTS;   // my chunks of the stream in this item
-      m_base = (m_base + run_s[2 * x + 1]) % FK_PARTS;
+      m_base = (m_base + run_s[2 * xs + 1]) % FK_PARTS;
 #pragma unroll 1
       for (int ci = my_first; ci < run_end; ci += FK_PARTS) {            // warp-uniform: only lit chunks
-        const uint32_t mask = apmask_s[x * (Np / 16) + ci];
+        const uint32_t mask = FUSED ? 0u : apmask_s[x * (Np / 16) + ci];
         const int y0 = ci * 16;
         float d[16];
-        if (!(p.dbg & 4)) tc_ld16(lane_addr + as * 256 + y0, d);
+        // pixel y of the column is accumulator column y - seg SEG of the segment's MMA
+        if (!(p.dbg & 4)) tc_ld16(lane_addr + as * 256 + y0 - seg * SEG, d);
         else { for (int j = 0; j < 16; ++j) d[j] = 0.01f * j; }
         // this chunk's fill was issued one chunk ago; issue the next lit chunk's fill now if it is this warp's turn
         if (!(p.dbg & 2)) {
@@ -1112,7 +1126,7 @@ k_dm_phase_tc(const __grid_constant__ CUtensorMap tmAct_hi, const __grid_constan
       __syncwarp();
       if (lane == 0) mbar_arrive(&tmem_empty[as]);       // this warp is done with the accumulator
       if (valid && !PHASE_ONLY) {
-        float2* r = p.R4 + (((size_t)env * Np + x) * FK_PARTS + q) * NOBS;
+        float2* r = p.R4 + (((size_t)env * Np + x) * (NSEG * FK_PARTS) + seg * FK_PARTS + q) * NOBS;
         if constexpr (SYM) {
           // pair v: row v = (ac - bs, as + bc), row n-1-v = (ac + bs, as - bc)
           constexpr int NP2 = NOBS / 2;
@@ -1829,10 +1843,12 @@ int aog_tensor_create(aog_env* env) {
   const int NPc = c.num_pupil_pixels;
   if (c.precision == AOG_PRECISION_TENSOR && (NPc != TC_NP || c.num_focal_pixels != TC_NF))
     AOG_FAIL(AOG_ERR_UNSUPPORTED, "precision='tensor' (matrix-Fourier-transform GEMMs) is built for num_pupil_pixels=240, "
-                                  "num_focal_pixels=128; use precision='fused' (pupil 128 / 240 / 256, any focal grid) or 'f64'");
-  if (c.precision == AOG_PRECISION_FUSED && NPc != TC_NP && !((NPc == 128 || NPc == 256) && (c.obs_dim == 2 || c.obs_dim == 5)))
-    AOG_FAIL(AOG_ERR_UNSUPPORTED, "precision='fused' supports num_pupil_pixels=240 (any obs_dim <= 8) and 128 / 256 (obs_dim 2 "
-                                  "or 5), with any focal grid; use precision='f64' for other grids");
+                                  "num_focal_pixels=128; use precision='fused' (pupil 128 / 240 / 256 / 512, any focal grid) "
+                                  "or 'f64'");
+  if (c.precision == AOG_PRECISION_FUSED && NPc != TC_NP &&
+      !((NPc == 128 || NPc == 256 || NPc == 512) && (c.obs_dim == 2 || c.obs_dim == 5)))
+    AOG_FAIL(AOG_ERR_UNSUPPORTED, "precision='fused' supports num_pupil_pixels=240 (any obs_dim <= 8) and 128 / 256 / 512 "
+                                  "(obs_dim 2 or 5), with any focal grid; use precision='f64' for other grids");
   TensorState* ts = new TensorState();
   env->tensor_state = ts;
   ts->fused = c.precision == AOG_PRECISION_FUSED;
@@ -1884,7 +1900,7 @@ int aog_tensor_create(aog_env* env) {
   AOG_CUDA(cudaMemset(ts->act_lo, 0, (size_t)ts->act_rows * ts->kpad * sizeof(__half)));
   A(talloc(env, &ts->apmask, (size_t)NPc * (NPc / 16)));
   A(talloc(env, &ts->m1o32, (size_t)c.obs_dim * NPc));
-  A(talloc(env, &ts->R4, ch * NPc * FK_PARTS * c.obs_dim));
+  A(talloc(env, &ts->R4, ch * NPc * FK_NSEG(NPc) * FK_PARTS * c.obs_dim));
   A(talloc(env, &ts->m2oT, (size_t)c.obs_dim * NPc));
   // barrier-timeout code: mapped pinned HOST memory, so that the host can still read it after the trap that follows
   // a timeout has poisoned the CUDA context (aog_health)
@@ -1904,8 +1920,9 @@ int aog_tensor_create(aog_env* env) {
   }
   A(make_map(env, &ts->tmAct_hi, ts->act_hi, ts->act_rows, 128, ts->kpad, 64));
   A(make_map(env, &ts->tmAct_lo, ts->act_lo, ts->act_rows, 128, ts->kpad, 64));
-  A(make_map(env, &ts->tmModes_hi, ts->modesK_hi, P, NPc, ts->kpad, 64));
-  A(make_map(env, &ts->tmModes_lo, ts->modesK_lo, P, NPc, ts->kpad, 64));
+  // B operand of the phase kernel: one column segment of pixels (a TMA box holds at most 256 rows)
+  A(make_map(env, &ts->tmModes_hi, ts->modesK_hi, P, NPc / FK_NSEG(NPc), ts->kpad, 64));
+  A(make_map(env, &ts->tmModes_lo, ts->modesK_lo, P, NPc / FK_NSEG(NPc), ts->kpad, 64));
 #undef A
   AOG_CUDA(cudaFuncSetAttribute(k_mft2<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, M2_SMEM_BYTES));
   AOG_CUDA(cudaFuncSetAttribute(k_mft2<AOG_MAX_LP>, cudaFuncAttributeMaxDynamicSharedMemorySize, M2_SMEM_BYTES));
@@ -2287,7 +2304,8 @@ int launch_phase(aog_env* env, TensorState* ts, const FieldParams& p, int grid, 
   constexpr bool FUSED = MODE == 1 || MODE == 2;
   constexpr int smem = FK_STAGES * FK_STAGE_BYTES + FK_PF_BYTES(NOBS, MODE) + 1024 + FK_AUX_BAR +
                        (FUSED ? 1 + FK_JT : 1) * FK_PARTS * 128 * (int)sizeof(double2) +
-                       (FUSED ? 0 : NOBS * NP * (int)sizeof(float2)) + NP * (NP / 16) * (int)sizeof(uint16_t) + 2 * NP;
+                       (FUSED ? 0 : NOBS * NP * (int)sizeof(float2) + NP * (NP / 16) * (int)sizeof(uint16_t)) +
+                       2 * NP * FK_NSEG(NP);
   static_assert(smem <= 227 * 1024, "shared memory of the phase kernel");
   static std::atomic<bool> configured_on[64];   // function attributes are per device: one flag per device ordinal
   std::atomic<bool>& configured = configured_on[env->cfg.device & 63];
@@ -2304,14 +2322,16 @@ template <bool STREHL, int MODE>
 int launch_phase_n(aog_env* env, TensorState* ts, const FieldParams& p, int n, int grid, cudaStream_t st) {
   const int Np = env->cfg.num_pupil_pixels;
   if (Np != TC_NP) {
-    // the pupil-grid axis of BASELINE configs[4]: fused kernels for 128^2 and 256^2 pupils, detectors 2x2 and 5x5
+    // the pupil-grid axis of BASELINE configs[4]: fused kernels for 128^2, 256^2 and 512^2 pupils, detectors 2x2 and 5x5
     if constexpr (MODE == 1 || MODE == 2) {
       if (Np == 128 && n == 2) return launch_phase<STREHL, 2, MODE, 128>(env, ts, p, grid, st);
       if (Np == 128 && n == 5) return launch_phase<STREHL, 5, MODE, 128>(env, ts, p, grid, st);
       if (Np == 256 && n == 2) return launch_phase<STREHL, 2, MODE, 256>(env, ts, p, grid, st);
       if (Np == 256 && n == 5) return launch_phase<STREHL, 5, MODE, 256>(env, ts, p, grid, st);
+      if (Np == 512 && n == 2) return launch_phase<STREHL, 2, MODE, 512>(env, ts, p, grid, st);
+      if (Np == 512 && n == 5) return launch_phase<STREHL, 5, MODE, 512>(env, ts, p, grid, st);
     }
-    AOG_FAIL(AOG_ERR_UNSUPPORTED, "fused kernels for pupils other than 240^2 are built for 128^2 / 256^2 with obs_dim 2 or 5");
+    AOG_FAIL(AOG_ERR_UNSUPPORTED, "fused kernels for pupils other than 240^2 are built for 128^2 / 256^2 / 512^2 with obs_dim 2 or 5");
   }
   switch (n) {
     case 1: return launch_phase<STREHL, 1, MODE>(env, ts, p, grid, st);
@@ -2342,20 +2362,22 @@ int launch_small(aog_env* env, const SmallParams& sp, int n, cudaStream_t st) {
   AOG_LAUNCH_CHECK();
   return AOG_OK;
 }
-// k_finalize_tcw<n, FK_PARTS>: one warp per env, dynamic shared memory above 48 KB (opt-in once per device)
-template <int N>
+// k_finalize_tcw<n, PARTS>: one warp per env, dynamic shared memory above 48 KB (opt-in once per device).
+// PARTS = a.r4_parts: FK_PARTS, or 2 FK_PARTS for the two column segments of a 512^2 pupil.
+template <int N, int PARTS = FK_PARTS>
 cudaError_t launch_finalize(int device, const FinalizeArgs& a, int nB, cudaStream_t st) {
-  using Cfg = FinCfg<N, FK_PARTS>;
+  using Cfg = FinCfg<N, PARTS>;
+  static_assert(Cfg::SMEM + Cfg::TAB_MAX <= 227 * 1024, "shared memory of k_finalize_tcw");
   static std::atomic<bool> configured_on[64];
   std::atomic<bool>& configured = configured_on[device & 63];
   if (!configured.load(std::memory_order_acquire)) {
-    const cudaError_t e = cudaFuncSetAttribute(k_finalize_tcw<N, FK_PARTS>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+    const cudaError_t e = cudaFuncSetAttribute(k_finalize_tcw<N, PARTS>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                                Cfg::SMEM + Cfg::TAB_MAX);
     if (e != cudaSuccess) return e;
     configured.store(true, std::memory_order_release);
   }
-  if (a.Np > 256) return cudaErrorInvalidValue;
-  k_finalize_tcw<N, FK_PARTS><<<cdiv(nB, FIN_WARPS), FIN_WARPS * 32, Cfg::SMEM + N * a.Np * 16, st>>>(a, nB);
+  if (a.Np > 512 || a.r4_parts != PARTS) return cudaErrorInvalidValue;
+  k_finalize_tcw<N, PARTS><<<cdiv(nB, FIN_WARPS), FIN_WARPS * 32, Cfg::SMEM + N * a.Np * 16, st>>>(a, nB);
   return cudaSuccess;
 }
 }  // namespace
@@ -2371,6 +2393,7 @@ int aog_tensor_optics(aog_env* env, bool flat_dm, bool with_reward, const aog_ou
   const int Np = c.num_pupil_pixels, n = c.obs_dim, K = c.num_modes, J = c.num_lp_modes, B = c.num_envs;
   const bool strehl = with_reward && c.rew_type == AOG_REW_STREHL_RATIO;
   const double2 norm = make_double2(c.mft_norm_re * c.amp_fiber, c.mft_norm_im * c.amp_fiber);
+  const int nseg = FK_NSEG(Np), items_per_block = Np * nseg;      // phase-kernel work items: column segments
   int slot_ipc = 1;
   for (int e0 = 0; e0 < B; e0 += env->chunk) {
     const int nB = std::min(env->chunk, B - e0);
@@ -2386,8 +2409,9 @@ int aog_tensor_optics(aog_env* env, bool flat_dm, bool with_reward, const aog_ou
       ts->packed_valid = false;                      // good for the one optics pass that follows k_actuators_pack
       FieldParams fp{};
       fp.num_envs = nB;
-      fp.num_items = cdiv(nB, 128) * Np;
-      fp.items_per_cta = std::max(Np / FK_MIN_ITEMS + 1 <= FK_SLOTS ? FK_MIN_ITEMS : FK_MIN_ITEMS + 1, cdiv(fp.num_items, ts->num_sms));   // CTAs per env block <= FK_SLOTS
+      fp.num_items = cdiv(nB, 128) * items_per_block;
+      // an env block's items touch at most cdiv(items_per_block, items_per_cta) + 1 <= FK_SLOTS CTAs
+      fp.items_per_cta = std::max(std::max(FK_MIN_ITEMS, cdiv(items_per_block, FK_SLOTS - 1)), cdiv(fp.num_items, ts->num_sms));
       fp.nkb = ts->kpad / 64;
       fp.col_origin = (int)env->cnt.column_origin;
       fp.env0 = e0;
@@ -2455,7 +2479,7 @@ int aog_tensor_optics(aog_env* env, bool flat_dm, bool with_reward, const aog_ou
     }
     if (env->timing) { AOG_CUDA(cudaEventRecord(env->ev1, st)); env->ev_valid = true; }
     FinalizeArgs a{};
-    a.R = nullptr; a.R4 = ts->R4; a.r4_parts = FK_PARTS; a.m1o = ts->m2oT;
+    a.R = nullptr; a.R4 = ts->R4; a.r4_parts = nseg * FK_PARTS; a.m1o = ts->m2oT;
     {
       // coef holds the raw projection sums (re, im): scale = norm * amp * pupil weight * table scale
       const double sc = fused ? c.amp_fiber * ts->gfib_scale : c.amp_fiber * ts->pupil_weight * ts->lpw_scale;
@@ -2464,7 +2488,7 @@ int aog_tensor_optics(aog_env* env, bool flat_dm, bool with_reward, const aog_ou
       a.fib_part = ts->fib_part; a.fib_slots = FK_SLOTS; a.fib_stride = FK_JT;
     } a.coef = nullptr; a.coef4 = ts->coef4; a.lpphase = fused ? ts->lpphase_f : env->t_lpphase; a.lpgram = env->t_lpgram;
     a.strehl_part = env->strehl_part; a.strehl_blocks = FK_SLOTS;
-    a.slot_ipc = slot_ipc; a.slot_items = Np;
+    a.slot_ipc = slot_ipc; a.slot_items = items_per_block;
     a.act = env->act + (size_t)e0 * K; a.K = K;      // (a flattened mirror has zero, not NaN, actuators)
     a.Np = Np; a.n = n; a.J = J; a.rew_type = c.rew_type; a.has_thr = c.has_rew_threshold;
     a.compute_reward = with_reward ? 1 : 0;
@@ -2480,7 +2504,11 @@ int aog_tensor_optics(aog_env* env, bool flat_dm, bool with_reward, const aog_ou
     a.ssim = out.ssim ? out.ssim + e0 : nullptr;
     static const bool fin_block = getenv("AOG_FINALIZE_BLOCK") != nullptr;     // A/B switch: the block-per-env form
     if (fin_block || n > 8) k_finalize_tc<<<nB, 128, (size_t)Np * n * sizeof(double2), st>>>(a);
-    else switch (n) {
+    else if (nseg == 2) {
+      if (n == 2) AOG_CUDA((launch_finalize<2, 2 * FK_PARTS>(c.device, a, nB, st)));
+      else if (n == 5) AOG_CUDA((launch_finalize<5, 2 * FK_PARTS>(c.device, a, nB, st)));
+      else AOG_FAIL(AOG_ERR_UNSUPPORTED, "fused kernels for 512^2 pupils are built for obs_dim 2 or 5");
+    } else switch (n) {
       case 1: AOG_CUDA(launch_finalize<1>(c.device, a, nB, st)); break;
       case 2: AOG_CUDA(launch_finalize<2>(c.device, a, nB, st)); break;
       case 3: AOG_CUDA(launch_finalize<3>(c.device, a, nB, st)); break;

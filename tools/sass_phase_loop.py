@@ -3,7 +3,8 @@
     python tools/sass_phase_loop.py [libaogym.so] [--md]
 
 The chunk loop is the innermost backward branch around the kernel's tcgen05.ld (LDTM): its body handles one
-16-pixel chunk per epilogue warp.  For each instantiation <STREHL, NOBS, MODE, NP> this prints the loop's instruction
+16-pixel chunk per epilogue warp.  For each instantiation <STREHL, NOBS, MODE, NP> (NP = 240 for every mode and detector
+size; 128, 256 and 512 for the fused modes 1 and 2 with NOBS 2 and 5) this prints the loop's instruction
 count, its XU (conversion / transcendental pipe) instructions, MUFU, F2I and F2F separately, its bulk and tensor
 copy issues (UBLKCP, UTMALDG), the instructions of the fill path (the innermost BSSY .. BSYNC region that holds those
 copies: the prefetch issue, which a warp runs on every chunk in a per-warp ring and on every fourth chunk in a ring
