@@ -78,26 +78,12 @@ int extrude_once(aog_env* env, bool positive, const double* noise_dev, long long
                                     flipped, c.sqrt_cn2, noise_stride, c.seed, (unsigned long long)c.env_id_base,
                                     (unsigned long long)env->cnt.extrusions);
     AOG_LAUNCH_CHECK();
-    static const bool split = getenv("AOG_AR_SPLIT") != nullptr;     // tuning: the three-kernel form
-    if (split) {
-      dim3 g2(cdiv(Np, 64), cdiv(nB, 64));
-      k_dgemm<<<g2, 256, 0, st>>>(env->arZ, env->t_arW, env->arNew, nB, Np, Ns + Np, Ns + Np, Np, Np);
-      AOG_LAUNCH_CHECK();
-      dim3 g3(cdiv(Np, 128), nB);
-      k_ar_scatter<<<g3, 128, 0, st>>>(env->screens, env->arNew, env->P, Np, e0, phys, flipped);
-      AOG_LAUNCH_CHECK();
-      continue;
-    }
     // GEMM with the scatter into the ring slot (and the phase-tile refresh of the tensor / fused paths) in its epilogue
     dim3 g2(cdiv(Np, 64), cdiv(nB, AR_TM));
     { int rc = dmma_configure(env); if (rc) return rc; }
     k_ar_step<false><<<g2, AR_THREADS, AR_SMEM, st>>>(env->arZ, env->t_arW, env->screens, env->phase_tiles, nB, Np, Ns + Np, env->P, e0, phys,
                                   flipped, 1.0 / (c.wavelength_wfs * 3.14159265358979323846), env->phase_tiles_unit, ArDirect{});
     AOG_LAUNCH_CHECK();
-  }
-  if (getenv("AOG_AR_SPLIT") != nullptr && c.precision != AOG_PRECISION_F64) {
-    int rc = aog_tensor_column_updated(env, phys, st);
-    if (rc) return rc;
   }
   env->cnt.column_origin = positive ? (org + 1) % Np : phys;
   env->cnt.extrusions++;
@@ -153,7 +139,7 @@ int evolve_to(aog_env* env, int64_t new_timestep, int64_t old_timestep, const do
   const int Np = env->cfg.num_pupil_pixels;
   const int64_t n = d < 0 ? -d : d;
   if (n == 0) return AOG_OK;
-  if (env->ar_direct && getenv("AOG_AR_SPLIT") == nullptr && n <= 4096) return extrude_direct(env, d > 0, (int)n, noise_dev, st);
+  if (env->ar_direct && n <= 4096) return extrude_direct(env, d > 0, (int)n, noise_dev, st);
   for (int64_t i = 0; i < n; ++i) {
     const double* nz = noise_dev ? noise_dev + (size_t)i * Np : nullptr;
     int rc = extrude_once(env, d > 0, nz, (long long)n * Np, st);
@@ -379,7 +365,6 @@ int aog_create(const aog_config* cfg, aog_env** out) {
   A(dev_alloc(env, &env->strehl_part, ch * (size_t)env->strehl_blocks));
   if (c.num_stencil > 0) {
     A(dev_alloc(env, &env->arZ, ch * (size_t)(c.num_stencil + Np)));
-    A(dev_alloc(env, &env->arNew, ch * (size_t)Np));
   }
   A(alloc_host_outputs(env));
   if (c.precision != AOG_PRECISION_F64) A(aog_tensor_create(env));
@@ -411,7 +396,7 @@ void aog_destroy(aog_env* env) {
                   env->t_lpw, env->t_lpphase, env->t_lpgram, env->t_stencil, env->t_stencil_perm, env->t_arA, env->t_arB, env->t_arW,
                   env->t_arW_rev, env->t_ar_tail, env->arNZ, env->t_scr_sh, env->t_scr_tw, env->t_scrC1, env->t_scrW1, env->t_scrW1T, env->t_scrC2, env->t_scrW2, env->t_scrW2T,
                   env->screens, env->act, env->bufA, env->bufB, env->bufC, env->bufR, env->coef,
-                  env->strehl_part, env->arZ, env->arNew, env->act_in, env->noise_in, env->o_pack,
+                  env->strehl_part, env->arZ, env->act_in, env->noise_in, env->o_pack,
                   env->t_sh_mla, env->t_sh_C, env->t_sh_CT,
                   env->t_sh_off, env->t_sh_pix, env->t_sh_px, env->t_sh_py, env->t_sh_offset, env->t_sh_recon,
                   env->t_sh_act0, env->act_sh, env->o_action, env->sh_noisy_in, env->t_sh_Cf[0], env->t_sh_Cf[1],
@@ -854,8 +839,7 @@ int aog_step(aog_env* env, const void* actions_dev, int act_dtype, const double*
   if (env->timing) AOG_CUDA(cudaEventRecord(env->tev[0], st));
   const int64_t ext_before = env->cnt.extrusions;
   int rc;
-  static const bool no_overlap = getenv("AOG_NO_OVERLAP") != nullptr;
-  if (env->sh_phase_pending && env->sh_phase_stream == st && c.velocity != 0.0 && !env->timing && !no_overlap) {
+  if (env->sh_phase_pending && env->sh_phase_stream == st && c.velocity != 0.0 && !env->timing) {
     // SH_step's phase kernel was the last reader of the screens: extrude on the side stream, under SH_step's
     // remaining kernels (which are still running or queued on `st`), and join before the optics
     AOG_CUDA(cudaStreamWaitEvent(env->side_stream, env->ev_sh_phase, 0));

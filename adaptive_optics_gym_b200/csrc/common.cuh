@@ -90,7 +90,6 @@ struct aog_env {
   double2* strehl_part = nullptr;  // [chunk][strehl_blocks]
   int strehl_blocks = 0;
   double* arZ = nullptr;           // [chunk][Ns+Np]
-  double* arNew = nullptr;         // [chunk][Np]
   double* arNZ = nullptr;          // [arNZ_cap extrusions][chunk][Np] scaled normals of one step (k_ar_noise)
   int arNZ_cap = 0;
   void* act_in = nullptr;          // [B][K] staging of raw actions (f64-sized)

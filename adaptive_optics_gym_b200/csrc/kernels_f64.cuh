@@ -173,47 +173,6 @@ static __global__ void __launch_bounds__(256) k_zgemm(const double2* __restrict_
     }
 }
 
-// Real FP64 GEMM C (M x N) = A (M x Kd) . B (Kd x N), same tiling (AR extrusion over envs).
-static __global__ void __launch_bounds__(256) k_dgemm(const double* __restrict__ A, const double* __restrict__ B,
-                                               double* __restrict__ C, int M, int N, int Kd, int lda, int ldb,
-                                               int ldc) {
-  __shared__ double As[16][65];
-  __shared__ double Bs[16][64];
-  const int tx = threadIdx.x & 15, ty = threadIdx.x >> 4;
-  const int m0 = blockIdx.y * 64, n0 = blockIdx.x * 64;
-  double acc[4][4] = {};
-  for (int k0 = 0; k0 < Kd; k0 += 16) {
-#pragma unroll
-    for (int i = 0; i < 4; ++i) {
-      const int k = threadIdx.x & 15, m = (threadIdx.x >> 4) + 16 * i;
-      As[k][m] = (m0 + m < M && k0 + k < Kd) ? A[(size_t)(m0 + m) * lda + k0 + k] : 0.0;
-      const int n = threadIdx.x & 63, kb = (threadIdx.x >> 6) + 4 * i;
-      Bs[kb][n] = (n0 + n < N && k0 + kb < Kd) ? B[(size_t)(k0 + kb) * ldb + n0 + n] : 0.0;
-    }
-    __syncthreads();
-#pragma unroll
-    for (int kk = 0; kk < 16; ++kk) {
-      double a[4], b[4];
-#pragma unroll
-      for (int i = 0; i < 4; ++i) a[i] = As[kk][ty + 16 * i];
-#pragma unroll
-      for (int j = 0; j < 4; ++j) b[j] = Bs[kk][tx + 16 * j];
-#pragma unroll
-      for (int i = 0; i < 4; ++i)
-#pragma unroll
-        for (int j = 0; j < 4; ++j) acc[i][j] = fma(a[i], b[j], acc[i][j]);
-    }
-    __syncthreads();
-  }
-#pragma unroll
-  for (int i = 0; i < 4; ++i)
-#pragma unroll
-    for (int j = 0; j < 4; ++j) {
-      const int m = m0 + ty + 16 * i, n = n0 + tx + 16 * j;
-      if (m < M && n < N) C[(size_t)m * ldc + n] = acc[i][j];
-    }
-}
-
 // --------------------------------------------------------------------------------------
 // Fibre-mode projection (AO_env.py:471): c_j = norm * sum_q F[q] (mode_j w)[q].  Block per env.
 // --------------------------------------------------------------------------------------
@@ -275,26 +234,25 @@ static __global__ void k_obs_rows_f64(const double2* __restrict__ E, const doubl
 
 // --------------------------------------------------------------------------------------
 // Per-env epilogue: obs power (second contraction + |.|^2 w), fibre power, Strehl, SSIM,
-// reward, threshold (AO_env.py:142-153, 468-503).  Block per env.
+// reward, threshold (AO_env.py:142-153, 468-503).  k_finalize (FP64 path, block per env) reads R and coef;
+// k_finalize_tcw (tensor / fused paths, warp per env) reads R4 and the partial sums and actuators described below.
 // --------------------------------------------------------------------------------------
 struct FinalizeArgs {
   const double2* R; const float2* R4; const double2* m1o; const double2* coef; const double* coef4; const double2* lpphase; const double* lpgram;
   const double2* strehl_part; int strehl_blocks;
   int Np, n, J, rew_type, has_thr, compute_reward;
-  int r4_parts;        // partial sums per contraction index in R4
-  int coef_is_raw;     // 1: coef holds unscaled (re, im) projection sums; 2: coef4 holds [re|im][2 partials];
-                       // 3: fib_part holds [fib_slots][fib_stride] partial sums per env;  all x coef_scale
+  int coef_is_raw;     // 2: coef4 holds [re|im][2 partials]; 3: fib_part holds [fib_slots][fib_stride] partial sums
+                       // per env;  both x coef_scale
   const double2* fib_part; int fib_slots, fib_stride;
-  // k_finalize_tc: the phase kernel's CTA c takes work items [c slot_ipc, (c + 1) slot_ipc) and the 128-env block eb
-  // owns items [eb slot_items, (eb + 1) slot_items), so only slots 0 .. last - first of an env are written (and
-  // summed): no clearing pass
+  // the phase kernel's CTA c takes work items [c slot_ipc, (c + 1) slot_ipc) and the 128-env block eb owns items
+  // [eb slot_items, (eb + 1) slot_items), so only slots 0 .. last - first of an env are written (and summed): no
+  // clearing pass
   int slot_ipc, slot_items;
-  // k_finalize_tc: the env's normalised actuators [K].  An all-zero action makes them 0/0 = NaN (AO_env.py:119-120)
-  // and the reference then returns NaN observations, reward and power; the fixed-point phase arithmetic of the
-  // tensor / fused kernels would swallow the NaN, so it is re-applied here.
+  // the env's normalised actuators [K].  An all-zero action makes them 0/0 = NaN (AO_env.py:119-120) and the
+  // reference then returns NaN observations, reward and power; the fixed-point phase arithmetic of the tensor / fused
+  // kernels would swallow the NaN, so it is re-applied here.
   const double* act; int K;
   double2 coef_scale;
-  int transpose_out;   // R / table hold the transposed contraction: result (a, b) is obs pixel (v = b, u = a)
   double thr, obs_weight, strehl_scale, ssim_peak;
   double2 norm;
   uint16_t* obs16; double* obs64; double* reward; double* power; double* strehl; double* ssim;
@@ -328,36 +286,20 @@ static __global__ void k_finalize(FinalizeArgs a) {
   for (int t = warp; t < n2; t += nwarps) {
     const int v = t / a.n, u = t - v * a.n;
     double re = 0.0, im = 0.0;
-    if (a.R4) {   // tensor path: r4_parts FP32 partial sums per contraction index
-      const float2* r4 = a.R4 + (size_t)b * a.Np * a.r4_parts * a.n;
-      for (int y = lane; y < a.Np; y += 32) {
-        const double2 m = a.m1o[(size_t)v * a.Np + y];
-        double ex = 0.0, ey = 0.0;
-        for (int qq = 0; qq < a.r4_parts; ++qq) {
-          const float2 t4 = r4[((size_t)y * a.r4_parts + qq) * a.n + u];
-          ex += (double)t4.x;
-          ey += (double)t4.y;
-        }
-        re += m.x * ex - m.y * ey;
-        im += m.x * ey + m.y * ex;
-      }
-    } else {
-      const double2* r = a.R + (size_t)b * a.Np * a.n;
-      for (int y = lane; y < a.Np; y += 32) {
-        const double2 m = a.m1o[(size_t)v * a.Np + y], e = r[(size_t)y * a.n + u];
-        re += m.x * e.x - m.y * e.y;
-        im += m.x * e.y + m.y * e.x;
-      }
+    const double2* r = a.R + (size_t)b * a.Np * a.n;
+    for (int y = lane; y < a.Np; y += 32) {
+      const double2 m = a.m1o[(size_t)v * a.Np + y], e = r[(size_t)y * a.n + u];
+      re += m.x * e.x - m.y * e.y;
+      im += m.x * e.y + m.y * e.x;
     }
     re = warp_sum(re);
     im = warp_sum(im);
     if (lane == 0) {
       const double fr = re * a.norm.x - im * a.norm.y, fi = re * a.norm.y + im * a.norm.x;
       const double pw = (fr * fr + fi * fi) * a.obs_weight;
-      const int to = a.transpose_out ? (u * a.n + v) : t;
-      obs[to] = pw;
-      if (a.obs64) a.obs64[(size_t)b * n2 + to] = pw;
-      if (a.obs16) a.obs16[(size_t)b * n2 + to] = __half_as_ushort(__double2half(pw));
+      obs[t] = pw;
+      if (a.obs64) a.obs64[(size_t)b * n2 + t] = pw;
+      if (a.obs16) a.obs16[(size_t)b * n2 + t] = __half_as_ushort(__double2half(pw));
     }
   }
   __syncthreads();
@@ -365,19 +307,7 @@ static __global__ void k_finalize(FinalizeArgs a) {
   // fibre: out = M (c e^{i beta L});  total power = c'^H G c'
   double2 c[AOG_MAX_LP];
   for (int j = 0; j < a.J; ++j) {
-    double2 cj;
-    if (a.coef_is_raw == 2) {
-      const double* c4 = a.coef4 + ((size_t)b * a.J + j) * 4;
-      cj = make_double2(c4[0] + c4[1], c4[2] + c4[3]);
-    } else if (a.coef_is_raw == 3) {
-      cj = make_double2(0.0, 0.0);
-      const double2* fp = a.fib_part + (size_t)b * a.fib_slots * a.fib_stride + j;
-#pragma unroll 8
-      for (int i = 0; i < a.fib_slots; ++i) { cj.x += fp[i * a.fib_stride].x; cj.y += fp[i * a.fib_stride].y; }
-    } else {
-      cj = a.coef[(size_t)b * a.J + j];
-    }
-    if (a.coef_is_raw) cj = make_double2(cj.x * a.coef_scale.x - cj.y * a.coef_scale.y, cj.x * a.coef_scale.y + cj.y * a.coef_scale.x);
+    const double2 cj = a.coef[(size_t)b * a.J + j];
     const double2 ph = a.lpphase[j];
     c[j] = make_double2(cj.x * ph.x - cj.y * ph.y, cj.x * ph.y + cj.y * ph.x);
   }
@@ -404,151 +334,10 @@ static __global__ void k_finalize(FinalizeArgs a) {
   if (a.power) a.power[b] = power;
 }
 
-// k_finalize for the tensor / fused paths (a.R4 column sums, a.coef_is_raw = 2 | 3): one block per env.
-// The env's partial column sums ([x][parts][n] float2, one contiguous run) are read ONCE, coalesced, summed over
-// the parts in FP64 and kept in shared memory; k_finalize reads them n times with a stride of parts * n * 8 bytes,
-// i.e. every 32-byte sector n times over (62 us for n = 2, 336 us for n = 5 at 4096 envs).  Warp 0 then reduces
-// the per-CTA partial slots of the Strehl sum and the fibre projections across lanes and evaluates the SSIM
-// windows one per lane.
-static __global__ void __launch_bounds__(128) k_finalize_tc(FinalizeArgs a) {
-  extern __shared__ double2 fin_R[];                   // [Np][n] column sums
-  __shared__ double obs[AOG_MAX_OBS * AOG_MAX_OBS];
-  __shared__ double2 pre[AOG_MAX_LP + 1];              // slot sums of the fibre projections and of the Strehl sum
-  const int b = blockIdx.x, n = a.n, n2 = n * n;
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, nwarps = blockDim.x >> 5;
-  if (a.act) {
-    int bad = 0;
-    for (int k = threadIdx.x; k < a.K; k += blockDim.x) bad |= isfinite(a.act[(size_t)b * a.K + k]) ? 0 : 1;   // inf: exp(i inf) = NaN too
-    if (__syncthreads_or(bad)) {
-      const double qnan = __longlong_as_double(0x7ff8000000000000LL);
-      for (int t = threadIdx.x; t < n2; t += blockDim.x) {
-        if (a.obs64) a.obs64[(size_t)b * n2 + t] = qnan;
-        if (a.obs16) a.obs16[(size_t)b * n2 + t] = 0x7e00;
-      }
-      if (threadIdx.x == 0 && a.compute_reward) {
-        if (a.reward) a.reward[b] = qnan;
-        if (a.power) a.power[b] = qnan;
-        if (a.strehl) a.strehl[b] = qnan;
-        if (a.ssim) a.ssim[b] = qnan;
-      }
-      return;
-    }
-  }
-  // The block is one long latency chain (slot sums -> column sums -> contraction -> reward): warps 1 and 2 fetch and
-  // reduce the per-CTA partial slots of the fibre projections / Strehl sum FIRST, so that their DRAM round trips run
-  // under the column-sum loads of the whole block.
-  const int eb = b >> 7;
-  const int nslots = ((eb + 1) * a.slot_items - 1) / a.slot_ipc - (eb * a.slot_items) / a.slot_ipc + 1;
-  if (a.compute_reward && warp == 1) {
-    for (int j = 0; j < a.J; ++j) {
-      double2 cj = make_double2(0.0, 0.0);
-      if (a.coef_is_raw == 2) {
-        const double* c4 = a.coef4 + ((size_t)b * a.J + j) * 4;
-        cj = make_double2(c4[0] + c4[1], c4[2] + c4[3]);
-      } else {
-        const double2* fp = a.fib_part + (size_t)b * a.fib_slots * a.fib_stride + j;
-        for (int i = lane; i < nslots; i += 32) { cj.x += fp[i * a.fib_stride].x; cj.y += fp[i * a.fib_stride].y; }
-        cj.x = warp_sum(cj.x);
-        cj.y = warp_sum(cj.y);
-      }
-      if (lane == 0) pre[j] = cj;
-    }
-  }
-  if (a.compute_reward && warp == 2 && a.rew_type == AOG_REW_STREHL_RATIO) {
-    double sr = 0.0, si = 0.0;
-    const double2* sp = a.strehl_part + (size_t)b * a.strehl_blocks;
-    for (int i = lane; i < nslots; i += 32) { sr += sp[i].x; si += sp[i].y; }
-    sr = warp_sum(sr);
-    si = warp_sum(si);
-    if (lane == 0) pre[AOG_MAX_LP] = make_double2(sr, si);
-  }
-  const float2* r4 = a.R4 + (size_t)b * a.Np * a.r4_parts * n;
-#pragma unroll 2
-  for (int i = threadIdx.x; i < a.Np * n; i += blockDim.x) {
-    const int x = i / n, v = i - x * n;
-    double ex = 0.0, ey = 0.0;
-    for (int qq = 0; qq < a.r4_parts; ++qq) {
-      const float2 t4 = r4[((size_t)x * a.r4_parts + qq) * n + v];
-      ex += (double)t4.x;
-      ey += (double)t4.y;
-    }
-    fin_R[i] = make_double2(ex, ey);
-  }
-  __syncthreads();
-  for (int t = warp; t < n2; t += nwarps) {
-    const int v = t / n, u = t - v * n;
-    double re = 0.0, im = 0.0;
-    const double2* mp = a.m1o + (size_t)v * a.Np + lane;
-    const double2* ep = fin_R + lane * n + u;
-    for (int y = lane; y < a.Np; y += 32, mp += 32, ep += 32 * n) {
-      const double2 m = *mp, e = *ep;
-      re = fma(m.x, e.x, fma(-m.y, e.y, re));
-      im = fma(m.x, e.y, fma(m.y, e.x, im));
-    }
-    re = warp_sum(re);
-    im = warp_sum(im);
-    if (lane == 0) {
-      const double fr = re * a.norm.x - im * a.norm.y, fi = re * a.norm.y + im * a.norm.x;
-      const double pw = (fr * fr + fi * fi) * a.obs_weight;
-      const int to = a.transpose_out ? (u * n + v) : t;
-      obs[to] = pw;
-      if (a.obs64) a.obs64[(size_t)b * n2 + to] = pw;
-      if (a.obs16) a.obs16[(size_t)b * n2 + to] = __half_as_ushort(__double2half(pw));
-    }
-  }
-  __syncthreads();
-  if (warp != 0 || !a.compute_reward) return;
-  // fibre: out = M (c e^{i beta L});  total power = c'^H G c'
-  double2 c[AOG_MAX_LP];
-  for (int j = 0; j < a.J; ++j) {
-    double2 cj = pre[j];
-    cj = make_double2(cj.x * a.coef_scale.x - cj.y * a.coef_scale.y, cj.x * a.coef_scale.y + cj.y * a.coef_scale.x);
-    const double2 ph = a.lpphase[j];
-    c[j] = make_double2(cj.x * ph.x - cj.y * ph.y, cj.x * ph.y + cj.y * ph.x);
-  }
-  double power = 0.0;
-  for (int j = 0; j < a.J; ++j)
-    for (int k = 0; k < a.J; ++k)
-      power += a.lpgram[j * a.J + k] * (c[j].x * c[k].x + c[j].y * c[k].y);
-  double reward;
-  if (a.rew_type == AOG_REW_STREHL_RATIO) {
-    const double sr = pre[AOG_MAX_LP].x, si = pre[AOG_MAX_LP].y;
-    const double strehl = a.strehl_scale * (sr * sr + si * si);
-    if (lane == 0 && a.strehl) a.strehl[b] = strehl;
-    reward = -(100.0 - strehl);
-  } else {
-    // skimage SSIM on 1-D data (ssim_1d above), one window per lane, summed in window order by lane 0
-    const double peak = a.ssim_peak, C1 = (0.01 * peak) * (0.01 * peak), C2 = (0.03 * peak) * (0.03 * peak);
-    const double cov_norm = 7.0 / 6.0;
-    const int ref_idx = n2 / 2;
-    __shared__ double win[AOG_MAX_OBS * AOG_MAX_OBS];
-    for (int cw = 3 + lane; cw < n2 - 3; cw += 32) {
-      double sx = 0, sxx = 0, sy = 0, syy = 0, sxy = 0;
-      for (int i = cw - 3; i <= cw + 3; ++i) {
-        const double x = obs[i], r = (i == ref_idx) ? peak : 0.0;
-        sx += x; sxx += x * x; sy += r; syy += r * r; sxy += x * r;
-      }
-      const double ux = sx / 7, uy = sy / 7, uxx = sxx / 7, uyy = syy / 7, uxy = sxy / 7;
-      const double vx = cov_norm * (uxx - ux * ux), vy = cov_norm * (uyy - uy * uy), vxy = cov_norm * (uxy - ux * uy);
-      win[cw] = ((2 * ux * uy + C1) * (2 * vxy + C2)) / ((ux * ux + uy * uy + C1) * (vx + vy + C2));
-    }
-    __syncwarp();
-    double tot = 0.0;
-    for (int cw = 3; cw < n2 - 3; ++cw) tot += win[cw];      // same summation order as ssim_1d
-    const double sv = tot / (double)(n2 - 6);
-    if (lane == 0 && a.ssim) a.ssim[b] = sv;
-    reward = 0.8 * power + (1.0 - 0.8) * sv;
-  }
-  if (lane != 0) return;
-  if (a.has_thr && reward < a.thr) reward = -1.0;
-  if (a.reward) a.reward[b] = reward;
-  if (a.power) a.power[b] = power;
-}
-
-// k_finalize_tcw<N, PARTS>: the same epilogue with ONE WARP per env and no block-level barrier (round 2; the
-// block-per-env k_finalize_tc above takes 122 us for the 5x5 detector at 4096 envs = 21 % of a configs[1] step, and a
-// first warp-per-env form with plain loads 106 us: the kernel is bound by the LATENCY of fetching the env's 28.8 KB of
-// column partial sums, not by its arithmetic).  So the partial sums stream through shared memory: every warp keeps a
+// k_finalize_tcw<N, PARTS>: the epilogue of the tensor / fused paths, R4 holding PARTS partial column sums per
+// contraction index, with ONE WARP per env and no block-level barrier.  The kernel is bound by the LATENCY of fetching
+// the env's column partial sums (28.8 KB for the 5x5 detector), not by its arithmetic (DESIGN 4.6), so the partial
+// sums stream through shared memory: every warp keeps a
 // double-buffered ring of tiles (8 XS pupil columns = ~6 KB each, 16-byte cp.async, one commit group per tile) in
 // flight ahead of its arithmetic -- 16 warps per SM x 6-12 KB outstanding.
 // Lane (xs, b) = (lane / N, lane % N) owns column b of the column sums and the pupil columns x = xs, xs + XS, ...
@@ -693,7 +482,7 @@ static __global__ void __launch_bounds__(FIN_WARPS * 32, 2) k_finalize_tcw(Final
     for (int s = 0; s < XS; ++s) { re += red[(2 * v) * Cfg::RED_LD + s * N + u]; im += red[(2 * v + 1) * Cfg::RED_LD + s * N + u]; }
     const double fr = re * a.norm.x - im * a.norm.y, fi = re * a.norm.y + im * a.norm.x;
     const double pw = (fr * fr + fi * fi) * a.obs_weight;
-    const int to = a.transpose_out ? (u * N + v) : t;
+    const int to = u * N + v;          // R4 and the table (M2o^T) hold the transposed contraction
     obs_s[to] = pw;
     if (a.obs64) a.obs64[(size_t)b * N2 + to] = pw;
     if (a.obs16) a.obs16[(size_t)b * N2 + to] = __half_as_ushort(__double2half(pw));
@@ -1137,15 +926,6 @@ k_ar_step(const double* __restrict__ Z, const double* __restrict__ W, double* __
         }
       }
   }
-}
-
-static __global__ void k_ar_scatter(double* __restrict__ screens, const double* __restrict__ newcol, int P, int Np,
-                             int env0, int phys_col, int flipped) {
-  const int b = blockIdx.y;
-  const int y = blockIdx.x * blockDim.x + threadIdx.x;
-  if (y >= Np) return;
-  const int src = flipped ? (Np - 1 - y) : y;
-  screens[(size_t)(env0 + b) * P + (size_t)phys_col * Np + y] = newcol[(size_t)b * Np + src];
 }
 
 // --------------------------------------------------------------------------------------

@@ -43,15 +43,15 @@ constexpr int SG_STAGE_BYTES = 2 * A_TILE;           // 16 KB: streamed operand,
 constexpr int SG_OUT_BUFS = 2;
 constexpr int SG_EPI_BYTES = 2 * SG_OUT_BUFS * 2 * M2_OUT_TILE;      // 32 KB: per column half, ring of (hi, lo) store tiles
 constexpr int SG_EPI_WARPS = 8;
-constexpr int SG_THREADS = 512;                      // warpgroups: {TMA, MMA, 2 idle} | 4 + 4 epilogue warps | 4 field warps (ONCHIP)
+// warp 0 TMA, warp 1 MMA, warps 4-11 epilogue; warps 2, 3 and 12-15 are idle.  Fewer threads raise the register cap
+// and change the generated code: a performance question of its own.
+constexpr int SG_THREADS = 512;
 constexpr int SG_SMEM_BYTES = SG_RES_BYTES + SG_STAGES * SG_STAGE_BYTES + SG_EPI_BYTES + 1024 /*align*/ + 1024 /*barriers*/;
 static_assert(SG_SMEM_BYTES <= 232448, "k_sh_gemm shared memory");
 
 struct ShGemmParams {
   int num_envs;          // environments in this chunk: items of each parity
   float* G;              // STAGE 2 output: [env][p][q][128 i'][re 128 u | im 128 u] FP32
-  const float* phi;      // ONCHIP stage 1: total phase [env][y / 16][x][16 y] (k_dm_phase_tc MODE 3)
-  const uint16_t* apmask;// ONCHIP stage 1: aperture bits [x][y / 16]
   int dbg;               // AOG_SH_DEBUG bits (tuning only): 1 no MMA, 4 no epilogue work
   int* err_flag;
 };
@@ -72,12 +72,7 @@ __device__ __forceinline__ void st_global_v8(void* p, const uint32_t* v) {
 // STAGE 2: resident = B (N side: rows [Gr(u) | Gi(u)] of C2_parity, parity = q; CTA r holds re | im), streamed = A
 //          (M side: Y_{p,q}, CTA r stages p = r); D lanes = i' (of block p = rank), columns = (re | im, u).
 //          Epilogue: FP32 -> G[env][p][q][i'][re | im][u].
-// ONCHIP (stage 1 only): the folded field is never written to HBM.  Four field warps (one fold column x per thread,
-// as in k_field_mft1) read the phase at the four mirror images of their 16 fold pixels of a K block, take sin / cos
-// (MUFU), apply the aperture, fold with the signs (p = the cluster's parity, q = the CTA's rank), split to fp16 and
-// write the row straight into the UMMA SWIZZLE_64B image of the ring slot; `full` then counts the 8 field warps of
-// the pair instead of TMA bytes.  Selected by AOG_SH_ONCHIP=1; the default is k_sh_fold + the TMA-streamed variant.
-template <int STAGE, bool ONCHIP>
+template <int STAGE>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(SG_THREADS, 1)
 k_sh_gemm(const __grid_constant__ CUtensorMap tmR_hi, const __grid_constant__ CUtensorMap tmR_lo,
           const __grid_constant__ CUtensorMap tmS_hi, const __grid_constant__ CUtensorMap tmS_lo,
@@ -108,7 +103,7 @@ k_sh_gemm(const __grid_constant__ CUtensorMap tmR_hi, const __grid_constant__ CU
     asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&tmR_lo)) : "memory");
     asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&tmS_hi)) : "memory");
     asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&tmS_lo)) : "memory");
-    for (int s = 0; s < SG_STAGES; ++s) { mbar_init(&full[s], ONCHIP ? 8 : 1); mbar_init(&empty[s], 1); }
+    for (int s = 0; s < SG_STAGES; ++s) { mbar_init(&full[s], 1); mbar_init(&empty[s], 1); }
     mbar_init(res_full, 1);
     for (int s = 0; s < 2; ++s) { mbar_init(&tmem_full[s], 1); mbar_init(&tmem_empty[s], 2 * SG_EPI_WARPS); }
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
@@ -125,9 +120,6 @@ k_sh_gemm(const __grid_constant__ CUtensorMap tmR_hi, const __grid_constant__ CU
   tc_fence_after();
   const uint32_t tmem_base = *tmem_ptr;
 
-  if (warp < 4) {
-    if (ONCHIP) asm volatile("setmaxnreg.dec.sync.aligned.u32 40;");
-  }
   if (warp == 0) {
     // ===================== TMA producer (both CTAs; completion on the leader's barriers) =====================
     if (lane == 0) {
@@ -143,7 +135,6 @@ k_sh_gemm(const __grid_constant__ CUtensorMap tmR_hi, const __grid_constant__ CU
       }
       int stage = 0;
       uint32_t phase = 0;
-      if (!ONCHIP)
       for (int item = first; item < p.num_envs; item += stride) {
         const int srow0 = ((item * 2 + parity) * 2 + (int)rank) * SH_HP;
         for (int kb = 0; kb < SH_NKB; ++kb) {
@@ -192,7 +183,6 @@ k_sh_gemm(const __grid_constant__ CUtensorMap tmR_hi, const __grid_constant__ CU
       }
     }
   } else if (warp >= 4 && warp < 12) {
-    if (ONCHIP) asm volatile("setmaxnreg.dec.sync.aligned.u32 104;");
     // ===================== epilogue: 8 warps, TMEM lane group = warp % 4, column half = (warp - 4) / 4 ========
     const int lg = warp & 3;
     const int half = (warp - 4) >> 2;
@@ -260,105 +250,6 @@ k_sh_gemm(const __grid_constant__ CUtensorMap tmR_hi, const __grid_constant__ CU
       if (lane == 0) mbar_arrive_cluster(tmem_empty_leader + buf * 8);   // this warp is done with the buffer
     }
     if (STAGE == 1 && lg == 0 && lane == 0) asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");   // stores landed
-  } else if (warp >= 12) {
-    if constexpr (ONCHIP) {
-      asm volatile("setmaxnreg.inc.sync.aligned.u32 224;");
-      // ===================== field warps: one fold column x per thread =====================
-      constexpr int Np = TC_NP, NC = TC_NP / 16;
-      const int t = (warp - 12) * 32 + lane;                       // row of the operand tile = fold column x
-      const bool active = t < SH_NH;
-      const int xa = active ? t : 0, xb = Np - 1 - xa;
-      const uint32_t sw = (uint32_t)((t >> 1) & 3);                // SWIZZLE_64B: 16-byte piece ^= (row >> 1) & 3
-      const float sp = parity ? -1.f : 1.f, sq = rank ? -1.f : 1.f;   // the cluster's row parity p, my CTA's column parity q
-      const uint32_t full_leader0 = mapa_rank(smem_u32(&full[0]), 0);
-      int stage = 0;
-      uint32_t phase = 0;
-      // K blocks of all my items as one stream, double-buffered in registers: the 16 float4 of block it + 1 are in
-      // flight while block it is turned into operand rows (a field thread has no other way to hide its loads)
-      const int my_items = first < p.num_envs ? (p.num_envs - first + stride - 1) / stride : 0;
-      const int total = my_items * SH_NKB;
-      float4 bufA[16], bufB[16];
-      auto load = [&](int it, float4 (&buf)[16]) {
-        const int item = first + (it / SH_NKB) * stride, kb = it % SH_NKB;
-        const float* pe = p.phi + (size_t)item * Np * Np;
-        const int ca = kb, cb = NC - 1 - kb;
-        const float4* src[4] = {reinterpret_cast<const float4*>(pe + ((size_t)ca * Np + xa) * 16),
-                                reinterpret_cast<const float4*>(pe + ((size_t)cb * Np + xa) * 16),
-                                reinterpret_cast<const float4*>(pe + ((size_t)ca * Np + xb) * 16),
-                                reinterpret_cast<const float4*>(pe + ((size_t)cb * Np + xb) * 16)};
-#pragma unroll
-        for (int m = 0; m < 4; ++m)
-#pragma unroll
-          for (int k = 0; k < 4; ++k)          // volatile: issued HERE, a K block ahead of their use
-            asm volatile("ld.global.nc.v4.f32 {%0, %1, %2, %3}, [%4];"
-                         : "=f"(buf[4 * m + k].x), "=f"(buf[4 * m + k].y), "=f"(buf[4 * m + k].z), "=f"(buf[4 * m + k].w)
-                         : "l"(src[m] + k));
-      };
-      auto compute = [&](int it, const float4 (&buf)[16]) {
-        const int kb = it % SH_NKB;
-        const int ca = kb, cb = NC - 1 - kb;
-        const float* ph = reinterpret_cast<const float*>(buf);      // [4 mirror images][16 pixels]
-        const uint32_t mk[4] = {__ldg(p.apmask + xa * NC + ca), __ldg(p.apmask + xa * NC + cb),
-                                __ldg(p.apmask + xb * NC + ca), __ldg(p.apmask + xb * NC + cb)};
-        const int nvalid = !active ? 0 : (kb == SH_NKB - 1 ? SH_NH - 16 * (SH_NKB - 1) : 16);
-        uint32_t oh[16], ol[16];                                   // [8 re pairs | 8 im pairs] packed halves
-#pragma unroll
-        for (int j2 = 0; j2 < 8; ++j2) {
-          float fre[2], fim[2];
-#pragma unroll
-          for (int h = 0; h < 2; ++h) {
-            const int j = 2 * j2 + h;
-            float c[4], sn4[4];
-#pragma unroll
-            for (int m = 0; m < 4; ++m) {                          // 0: (row, col); 1: row-mirrored; 2: column-mirrored; 3: both
-              const int jj = (m & 1) ? 15 - j : j;
-              float sn, cs;
-              __sincosf(ph[16 * m + jj], &sn, &cs);
-              const bool lit = ((mk[m] >> jj) & 1u) && j < nvalid;
-              c[m] = lit ? cs : 0.f;
-              sn4[m] = lit ? sn : 0.f;
-            }
-            // E_pq = (E0 + q E2) + p (E1 + q E3)
-            fre[h] = fmaf(sp, fmaf(sq, c[3], c[1]), fmaf(sq, c[2], c[0]));
-            fim[h] = fmaf(sp, fmaf(sq, sn4[3], sn4[1]), fmaf(sq, sn4[2], sn4[0]));
-          }
-          split_pack2(fre[0], fre[1], oh[j2], ol[j2]);
-          split_pack2(fim[0], fim[1], oh[8 + j2], ol[8 + j2]);
-        }
-        mbar_wait(&empty[stage], phase ^ 1, p.err_flag, 26);      // the MMAs that read this slot have retired
-        uint8_t* b_hi = ring + stage * SG_STAGE_BYTES + t * 64;
-        uint8_t* b_lo = b_hi + A_TILE;
-#pragma unroll
-        for (int k = 0; k < 4; ++k) {                              // pieces 0, 1 = 16 re; 2, 3 = 16 im
-          *reinterpret_cast<uint4*>(b_hi + (((uint32_t)k ^ sw) << 4)) = make_uint4(oh[4 * k], oh[4 * k + 1], oh[4 * k + 2], oh[4 * k + 3]);
-          *reinterpret_cast<uint4*>(b_lo + (((uint32_t)k ^ sw) << 4)) = make_uint4(ol[4 * k], ol[4 * k + 1], ol[4 * k + 2], ol[4 * k + 3]);
-        }
-        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-        __syncwarp();
-        if (lane == 0) mbar_arrive_cluster(full_leader0 + stage * 8);   // my 32 rows of the tile are in place
-        if (++stage == SG_STAGES) { stage = 0; phase ^= 1; }
-      };
-      const bool do_load = !(p.dbg & 16);                           // AOG_SH_DEBUG: 16 no phase loads, 8 no field arithmetic
-      if (p.dbg & 8) {
-        for (int it = 0; it < total; ++it) {
-          mbar_wait(&empty[stage], phase ^ 1, p.err_flag, 26);
-          __syncwarp();
-          if (lane == 0) mbar_arrive_cluster(full_leader0 + stage * 8);
-          if (++stage == SG_STAGES) { stage = 0; phase ^= 1; }
-        }
-      } else {
-        if (!do_load)
-          for (int k = 0; k < 16; ++k) bufA[k] = bufB[k] = make_float4(0.1f * k, 0.2f, 0.3f, 0.4f);
-        if (total > 0 && do_load) load(0, bufA);
-#pragma unroll 1
-        for (int it = 0; it < total; it += 2) {                    // SH_NKB is even: blocks come in (A, B) pairs
-          if (do_load) load(it + 1, bufB);
-          compute(it, bufA);
-          if (it + 2 < total && do_load) load(it + 2, bufA);
-          compute(it + 1, bufB);
-        }
-      }
-    }
   }
   tc_fence_before();
   __syncthreads();
@@ -834,9 +725,8 @@ int ensure_sh_tensor_buffers(aog_env* env, TensorState* ts) {
   if ((rc = make_map(env, &ts->tmShYB_lo, ts->shYB_lo, rows, SH_HP, SH_K, KB))) return rc;
   if ((rc = make_map(env, &ts->tmShYout_hi, ts->shYB_hi, rows, SH_HP, SH_K, 16))) return rc;
   if ((rc = make_map(env, &ts->tmShYout_lo, ts->shYB_lo, rows, SH_HP, SH_K, 16))) return rc;
-  AOG_CUDA(cudaFuncSetAttribute(k_sh_gemm<1, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SG_SMEM_BYTES));
-  AOG_CUDA(cudaFuncSetAttribute(k_sh_gemm<1, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SG_SMEM_BYTES));
-  AOG_CUDA(cudaFuncSetAttribute(k_sh_gemm<2, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SG_SMEM_BYTES));
+  AOG_CUDA(cudaFuncSetAttribute(k_sh_gemm<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, SG_SMEM_BYTES));
+  AOG_CUDA(cudaFuncSetAttribute(k_sh_gemm<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, SG_SMEM_BYTES));
   ts->sh_buffers = true;
   return AOG_OK;
 }
@@ -874,33 +764,24 @@ int sh_tensor_optics(aog_env* env, TensorState* ts, int e0, int nB, cudaStream_t
     }
   }
   if (env->timing) AOG_CUDA(cudaEventRecord(env->tev[3], st));
-  // default: k_sh_fold materialises the folded field and the first product streams it by TMA; AOG_SH_ONCHIP=1 forms it
-  // on chip inside the first product instead (measured slower so far: DESIGN.md 4.4)
-  static const bool fold_kernel = getenv("AOG_SH_ONCHIP") == nullptr;
-  if (fold_kernel) {
-    k_sh_fold<<<dim3(SH_NKB, nB), 128, 0, st>>>(ts->phi, ts->apmask, ts->shEB_hi, ts->shEB_lo, nB);
-    AOG_LAUNCH_CHECK();
-  }
+  // k_sh_fold materialises the folded field and the first product streams it by TMA (forming it on chip inside the
+  // first product was measured slower: DESIGN.md 4.4)
+  k_sh_fold<<<dim3(SH_NKB, nB), 128, 0, st>>>(ts->phi, ts->apmask, ts->shEB_hi, ts->shEB_lo, nB);
+  AOG_LAUNCH_CHECK();
   if (env->timing) AOG_CUDA(cudaEventRecord(env->tev[4], st));
   ShGemmParams gp{};
   gp.num_envs = nB;
   gp.G = ts->shG;
   { const char* d = getenv("AOG_SH_DEBUG"); gp.dbg = d ? atoi(d) : 0; }
   gp.err_flag = ts->err_flag;
-  gp.phi = ts->phi;
-  gp.apmask = ts->apmask;
   // clusters come in pairs (one per parity); each takes every (clusters / 2)-th environment
   const int clusters = std::max(2, std::min((ts->num_sms / 2) & ~1, 2 * nB));
-  if (fold_kernel)
-    k_sh_gemm<1, false><<<2 * clusters, SG_THREADS, SG_SMEM_BYTES, st>>>(ts->tmShCE_hi[0], ts->tmShCE_lo[0], ts->tmShEB_hi, ts->tmShEB_lo,
-                                                                         ts->tmShYout_hi, ts->tmShYout_lo, gp);
-  else
-    k_sh_gemm<1, true><<<2 * clusters, SG_THREADS, SG_SMEM_BYTES, st>>>(ts->tmShCE_hi[0], ts->tmShCE_lo[0], ts->tmShEB_hi, ts->tmShEB_lo,
-                                                                        ts->tmShYout_hi, ts->tmShYout_lo, gp);
+  k_sh_gemm<1><<<2 * clusters, SG_THREADS, SG_SMEM_BYTES, st>>>(ts->tmShCE_hi[0], ts->tmShCE_lo[0], ts->tmShEB_hi, ts->tmShEB_lo,
+                                                                ts->tmShYout_hi, ts->tmShYout_lo, gp);
   AOG_LAUNCH_CHECK();
   if (env->timing) AOG_CUDA(cudaEventRecord(env->tev[5], st));
-  k_sh_gemm<2, false><<<2 * clusters, SG_THREADS, SG_SMEM_BYTES, st>>>(ts->tmShCE_hi[1], ts->tmShCE_lo[1], ts->tmShYB_hi, ts->tmShYB_lo,
-                                                                ts->tmShYout_hi, ts->tmShYout_lo, gp);
+  k_sh_gemm<2><<<2 * clusters, SG_THREADS, SG_SMEM_BYTES, st>>>(ts->tmShCE_hi[1], ts->tmShCE_lo[1], ts->tmShYB_hi, ts->tmShYB_lo,
+                                                         ts->tmShYout_hi, ts->tmShYout_lo, gp);
   AOG_LAUNCH_CHECK();
   if (env->timing) AOG_CUDA(cudaEventRecord(env->tev[6], st));
   return AOG_OK;

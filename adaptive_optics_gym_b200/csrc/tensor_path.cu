@@ -590,7 +590,7 @@ __host__ __device__ constexpr int FK_NT(int nobs) { return (nobs + FK_JT + 1 + 1
 //     is real): with m = a + ib and E = c + is the four products ac, bs, as, bc serve both rows of a pair;
 //   * every back-projected fibre mode is a real function times one unit phasor, G_j = e^{i theta_j} R_j (the Fourier
 //     transform of a real mode that is even or odd along each axis): the projection is two real sums and the phasor
-//     joins the mode's propagation phase in k_finalize.
+//     joins the mode's propagation phase in k_finalize_tcw.
 // Record = FK_NF(n) floats: [a, b per pair | centre a | R_0..R_2 | aperture], padded to a multiple of 4.
 // The tables are checked for both properties when they are uploaded; tables without them run kernel MODE 1.
 __host__ __device__ constexpr int FK_NF(int nobs) { return (2 * (nobs / 2) + (nobs & 1) + FK_JT + 1 + 3) & ~3; }
@@ -1734,17 +1734,6 @@ __global__ void k_screens_to_tiles(const double* __restrict__ src, int32_t* __re
   if (env < (size_t)B) v = phase_fixed(src[(env * Np + xp) * Np + y], inv_w);      // screens are [env][x][y]
   hwt[o] = v;
 }
-// one physical column refresh after an extrusion
-__global__ void k_column_to_tiles(const double* __restrict__ src, int32_t* __restrict__ hwt, int Np, int B, int phys_col,
-                                  double inv_w) {
-  const int i = blockIdx.x * blockDim.x + threadIdx.x;      // over B * Np
-  if (i >= B * Np) return;
-  const int env = i / Np, y = i - env * Np;
-  const double S = src[((size_t)env * Np + phys_col) * Np + y];
-  const int l = env & 31, ci = y >> 4, piece = ((y >> 2) & 3) ^ ((l >> 1) & 3), e = y & 3;
-  const size_t tile = (((size_t)(env >> 5) * Np + phys_col) * (Np / 16) + ci) * (32 * 16);
-  hwt[tile + (size_t)l * 16 + piece * 4 + e] = phase_fixed(S, inv_w);
-}
 
 // ----------------------------------------------------------------------------- host helpers
 typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
@@ -2214,16 +2203,6 @@ int aog_tensor_screens_updated(aog_env* env) {
   return AOG_OK;
 }
 
-int aog_tensor_column_updated(aog_env* env, int phys_col, cudaStream_t st) {
-  TensorState* ts = TS(env);
-  const int B = env->cfg.num_envs;
-  const double pi = 3.14159265358979323846;
-  k_column_to_tiles<<<cdiv(B * env->cfg.num_pupil_pixels, 256), 256, 0, st>>>(env->screens, ts->hwt, env->cfg.num_pupil_pixels, B, phys_col,
-                                                          1.0 / (env->cfg.wavelength_wfs * pi));
-  AOG_LAUNCH_CHECK();
-  return AOG_OK;
-}
-
 // Debug read-back (tests): the split-fp16 intermediates of the LAST chunk processed, recombined
 // hi + lo and returned in the FP64 path's conventions.
 //   which = AOG_FIELD_TC_PUPIL : pupil field [y][x] complex (unit modulus x aperture)
@@ -2363,7 +2342,7 @@ int launch_small(aog_env* env, const SmallParams& sp, int n, cudaStream_t st) {
   return AOG_OK;
 }
 // k_finalize_tcw<n, PARTS>: one warp per env, dynamic shared memory above 48 KB (opt-in once per device).
-// PARTS = a.r4_parts: FK_PARTS, or 2 FK_PARTS for the two column segments of a 512^2 pupil.
+// PARTS = partial sums per contraction index in R4: FK_PARTS, or 2 FK_PARTS for the two column segments of a 512^2 pupil.
 template <int N, int PARTS = FK_PARTS>
 cudaError_t launch_finalize(int device, const FinalizeArgs& a, int nB, cudaStream_t st) {
   using Cfg = FinCfg<N, PARTS>;
@@ -2376,7 +2355,7 @@ cudaError_t launch_finalize(int device, const FinalizeArgs& a, int nB, cudaStrea
     if (e != cudaSuccess) return e;
     configured.store(true, std::memory_order_release);
   }
-  if (a.Np > 512 || a.r4_parts != PARTS) return cudaErrorInvalidValue;
+  if (a.Np > 512) return cudaErrorInvalidValue;
   k_finalize_tcw<N, PARTS><<<cdiv(nB, FIN_WARPS), FIN_WARPS * 32, Cfg::SMEM + N * a.Np * 16, st>>>(a, nB);
   return cudaSuccess;
 }
@@ -2423,7 +2402,7 @@ int aog_tensor_optics(aog_env* env, bool flat_dm, bool with_reward, const aog_ou
       fp.err_flag = ts->err_flag;
       const int grid = cdiv(fp.num_items, fp.items_per_cta);
       int rc;
-      slot_ipc = fp.items_per_cta;            // k_finalize_tc sums exactly the slots this launch writes
+      slot_ipc = fp.items_per_cta;            // k_finalize_tcw sums exactly the slots this launch writes
       const bool no_small = getenv("AOG_NO_SMALL") != nullptr;             // A/B switch and test hook: tensor cores for every batch size
       if (fused && ts->sym && B <= SMALL_MAX && !no_small && ts->kpad <= 128 && Np <= 256 && !fp.dbg) {
         SmallParams sp{};
@@ -2479,20 +2458,19 @@ int aog_tensor_optics(aog_env* env, bool flat_dm, bool with_reward, const aog_ou
     }
     if (env->timing) { AOG_CUDA(cudaEventRecord(env->ev1, st)); env->ev_valid = true; }
     FinalizeArgs a{};
-    a.R = nullptr; a.R4 = ts->R4; a.r4_parts = nseg * FK_PARTS; a.m1o = ts->m2oT;
+    a.R4 = ts->R4; a.m1o = ts->m2oT;
     {
       // coef holds the raw projection sums (re, im): scale = norm * amp * pupil weight * table scale
       const double sc = fused ? c.amp_fiber * ts->gfib_scale : c.amp_fiber * ts->pupil_weight * ts->lpw_scale;
       a.coef_scale = make_double2(c.mft_norm_re * sc, c.mft_norm_im * sc);
       a.coef_is_raw = fused ? 3 : 2;
       a.fib_part = ts->fib_part; a.fib_slots = FK_SLOTS; a.fib_stride = FK_JT;
-    } a.coef = nullptr; a.coef4 = ts->coef4; a.lpphase = fused ? ts->lpphase_f : env->t_lpphase; a.lpgram = env->t_lpgram;
+    } a.coef4 = ts->coef4; a.lpphase = fused ? ts->lpphase_f : env->t_lpphase; a.lpgram = env->t_lpgram;
     a.strehl_part = env->strehl_part; a.strehl_blocks = FK_SLOTS;
     a.slot_ipc = slot_ipc; a.slot_items = items_per_block;
     a.act = env->act + (size_t)e0 * K; a.K = K;      // (a flattened mirror has zero, not NaN, actuators)
     a.Np = Np; a.n = n; a.J = J; a.rew_type = c.rew_type; a.has_thr = c.has_rew_threshold;
     a.compute_reward = with_reward ? 1 : 0;
-    a.transpose_out = 1;     // R is [x][v] and the table is M2o^T: results come out as (u, v)
     a.thr = c.rew_threshold; a.obs_weight = c.obs_weight; a.strehl_scale = c.strehl_scale; a.ssim_peak = c.ssim_ref_peak;
     a.norm = norm;
     const size_t n2 = (size_t)env->n2;
@@ -2502,9 +2480,7 @@ int aog_tensor_optics(aog_env* env, bool flat_dm, bool with_reward, const aog_ou
     a.power = out.power ? out.power + e0 : nullptr;
     a.strehl = out.strehl ? out.strehl + e0 : nullptr;
     a.ssim = out.ssim ? out.ssim + e0 : nullptr;
-    static const bool fin_block = getenv("AOG_FINALIZE_BLOCK") != nullptr;     // A/B switch: the block-per-env form
-    if (fin_block || n > 8) k_finalize_tc<<<nB, 128, (size_t)Np * n * sizeof(double2), st>>>(a);
-    else if (nseg == 2) {
+    if (nseg == 2) {
       if (n == 2) AOG_CUDA((launch_finalize<2, 2 * FK_PARTS>(c.device, a, nB, st)));
       else if (n == 5) AOG_CUDA((launch_finalize<5, 2 * FK_PARTS>(c.device, a, nB, st)));
       else AOG_FAIL(AOG_ERR_UNSUPPORTED, "fused kernels for 512^2 pupils are built for obs_dim 2 or 5");

@@ -7,7 +7,6 @@ void aog_tensor_destroy(aog_env* env);
 int aog_tensor_table_updated(aog_env* env, int which, const void* host);
 int aog_tensor_screens_updated(aog_env* env);
 int aog_tensor_optics(aog_env* env, bool flat_dm, bool with_reward, const aog_outputs& out, cudaStream_t st);
-int aog_tensor_column_updated(aog_env* env, int phys_col, cudaStream_t st);
 int aog_tensor_check(aog_env* env);
 int aog_tensor_actuators(aog_env* env, const void* actions_dev, int act_dtype, cudaStream_t st);
 int aog_tensor_get_field(aog_env* env, int which, int env_in_chunk, double* host_out, size_t count);

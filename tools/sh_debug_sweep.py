@@ -1,5 +1,5 @@
-"""Per-kernel times of the tensor-core Shack-Hartmann step (aog_last_timings) under AOG_SH_DEBUG / AOG_SH_ONCHIP:
-which part of k_sh_gemm costs what (bits: 1 no MMA, 4 no epilogue, 8 no field arithmetic, 16 no phase loads)."""
+"""Per-kernel times of the tensor-core Shack-Hartmann step (aog_last_timings) under AOG_SH_DEBUG:
+which part of k_sh_gemm costs what (bits: 1 no MMA, 4 no epilogue work)."""
 import os, sys, torch
 sys.path.insert(0, '.')
 from adaptive_optics_gym_b200 import AOVecEnv
