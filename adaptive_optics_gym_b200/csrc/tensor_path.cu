@@ -31,6 +31,7 @@
 // plane: it projects it on the fibre modes (AO_env.py:471) out of TMEM.
 #include "tensor_path.cuh"
 #include "kernels_f64.cuh"
+#include "fp32x2.cuh"
 #include "phase_round.cuh"
 
 #include <cuda.h>
@@ -650,6 +651,21 @@ __device__ __forceinline__ void sincos_biased_fma(int32_t tb, int32_t kmask, int
   asm("cos.approx.ftz.f32 %0, %1;" : "=f"(*c) : "f"(x));
 }
 
+// sincos_biased_fma of two pixels, the FMA packed: (cos, sin) of each
+__device__ __forceinline__ void sincos_biased_fma2(int32_t tb0, int32_t tb1, int32_t kmask, int32_t kexp, float2* cs0,
+                                                   float2* cs1) {
+  int32_t u0, u1;
+  asm("lop3.b32 %0, %1, %2, %3, 0xEA;" : "=r"(u0) : "r"(tb0), "r"(kmask), "r"(kexp));
+  asm("lop3.b32 %0, %1, %2, %3, 0xEA;" : "=r"(u1) : "r"(tb1), "r"(kmask), "r"(kexp));
+  constexpr float sc = 3.14159265358979323846f / PHI_ONE;
+  const float2 x = f2_fma(make_float2(__int_as_float(u0), __int_as_float(u1)), make_float2(sc, sc),
+                          make_float2(-12582912.f * sc, -12582912.f * sc));
+  asm("sin.approx.ftz.f32 %0, %1;" : "=f"(cs0->y) : "f"(x.x));
+  asm("cos.approx.ftz.f32 %0, %1;" : "=f"(cs0->x) : "f"(x.x));
+  asm("sin.approx.ftz.f32 %0, %1;" : "=f"(cs1->y) : "f"(x.y));
+  asm("cos.approx.ftz.f32 %0, %1;" : "=f"(cs1->x) : "f"(x.y));
+}
+
 __device__ __forceinline__ void split_pack2(float a, float b, uint32_t& hi, uint32_t& lo) {
   const __half2 h = __floats2half2_rn(a, b);
   const float2 f = __half22float2(h);
@@ -976,13 +992,14 @@ k_dm_phase_tc(const __grid_constant__ CUtensorMap tmAct_hi, const __grid_constan
         }
         tc_wait_ld();
         if constexpr (SYM) {
-          // ---- fused kernel, symmetric tables: 12 FMAs per pixel for the obs pair, the three fibre modes and Strehl
+          // ---- fused kernel, symmetric tables: 12 FMAs per pixel for the obs pair, the three fibre modes and Strehl.
+          // The pixels go in pairs: the phase rounding and the angle FMA of the two are packed FP32x2 operations.
           constexpr int NP2 = NOBS / 2, NC = NOBS & 1, NF = FK_NF(NOBS);
           const float4* tab = reinterpret_cast<const float4*>(slot_ptr + FK_PF_PHASE);   // [16 y][NF / 4]
           const int32_t q31 = (int32_t)(p.sci_ratio_q32 >> 1);
           const int32_t sci_bias = (1 << 22) - 2 * (int32_t)(((long long)(1 << 22) * (long long)q31) >> 32);
 #pragma unroll
-          for (int j = 0; j < 16; ++j) {
+          for (int j = 0; j < 16; j += 2) {
             if (LATE_TILE && j == 8) {
 #pragma unroll
               for (int jj = 2; jj < 4; ++jj) {
@@ -990,35 +1007,42 @@ k_dm_phase_tc(const __grid_constant__ CUtensorMap tmAct_hi, const __grid_constan
                 t[4 * jj] = h.x; t[4 * jj + 1] = h.y; t[4 * jj + 2] = h.z; t[4 * jj + 3] = h.w;
               }
             }
-            const int32_t tb = t[j] + phase_fixed_rn(d[j]) + (1 << 22);
-            float c0, s0;
-            sincos_biased_fma(tb, kmask, kexp, &s0, &c0);
-            float4 rec[NF / 4];
+            int32_t tb[2];
+            phase_fixed_rn2(d[j], d[j + 1], &tb[0], &tb[1]);
+            tb[0] += t[j] + (1 << 22);
+            tb[1] += t[j + 1] + (1 << 22);
+            float2 e[2], es[2];                                             // (cos, sin) at lambda_wfs, lambda_sci
+            sincos_biased_fma2(tb[0], tb[1], kmask, kexp, &e[0], &e[1]);
+            if (STREHL)
+              sincos_biased_fma2(2 * __mulhi(tb[0], q31) + sci_bias, 2 * __mulhi(tb[1], q31) + sci_bias, kmask, kexp,
+                                 &es[0], &es[1]);
 #pragma unroll
-            for (int r = 0; r < NF / 4; ++r) rec[r] = tab[j * (NF / 4) + r];
-            const float* m = reinterpret_cast<const float*>(rec);
+            for (int h = 0; h < 2; ++h) {
+              const float c0 = e[h].x, s0 = e[h].y;
+              float4 rec[NF / 4];
 #pragma unroll
-            for (int v = 0; v < NP2; ++v) {
-              pp[4 * v + 0] = fmaf(m[2 * v], c0, pp[4 * v + 0]);
-              pp[4 * v + 1] = fmaf(m[2 * v + 1], s0, pp[4 * v + 1]);
-              pp[4 * v + 2] = fmaf(m[2 * v], s0, pp[4 * v + 2]);
-              pp[4 * v + 3] = fmaf(m[2 * v + 1], c0, pp[4 * v + 3]);
-            }
-            if (NC) {
-              pp[4 * NP2] = fmaf(m[2 * NP2], c0, pp[4 * NP2]);
-              pp[4 * NP2 + 1] = fmaf(m[2 * NP2], s0, pp[4 * NP2 + 1]);
-            }
+              for (int r = 0; r < NF / 4; ++r) rec[r] = tab[(j + h) * (NF / 4) + r];
+              const float* m = reinterpret_cast<const float*>(rec);
 #pragma unroll
-            for (int k = 0; k < FK_JT; ++k) {
-              fre[k] = fmaf(m[2 * NP2 + NC + k], c0, fre[k]);
-              fim[k] = fmaf(m[2 * NP2 + NC + k], s0, fim[k]);
-            }
-            if (STREHL) {
-              const int32_t ts = 2 * __mulhi(tb, q31) + sci_bias;
-              float cs, ss;
-              sincos_biased_fma(ts, kmask, kexp, &ss, &cs);
-              sre = fmaf(m[2 * NP2 + NC + FK_JT], cs, sre);
-              sim = fmaf(m[2 * NP2 + NC + FK_JT], ss, sim);
+              for (int v = 0; v < NP2; ++v) {
+                pp[4 * v + 0] = fmaf(m[2 * v], c0, pp[4 * v + 0]);
+                pp[4 * v + 1] = fmaf(m[2 * v + 1], s0, pp[4 * v + 1]);
+                pp[4 * v + 2] = fmaf(m[2 * v], s0, pp[4 * v + 2]);
+                pp[4 * v + 3] = fmaf(m[2 * v + 1], c0, pp[4 * v + 3]);
+              }
+              if (NC) {
+                pp[4 * NP2] = fmaf(m[2 * NP2], c0, pp[4 * NP2]);
+                pp[4 * NP2 + 1] = fmaf(m[2 * NP2], s0, pp[4 * NP2 + 1]);
+              }
+#pragma unroll
+              for (int k = 0; k < FK_JT; ++k) {
+                fre[k] = fmaf(m[2 * NP2 + NC + k], c0, fre[k]);
+                fim[k] = fmaf(m[2 * NP2 + NC + k], s0, fim[k]);
+              }
+              if (STREHL) {
+                sre = fmaf(m[2 * NP2 + NC + FK_JT], es[h].x, sre);
+                sim = fmaf(m[2 * NP2 + NC + FK_JT], es[h].y, sim);
+              }
             }
           }
         } else if constexpr (FUSED) {

@@ -1,6 +1,7 @@
-// CPU check of csrc/phase_round.cuh: phase_fixed_rn(d) against round-to-nearest-even of d * 2^22 for EVERY float d with
-// |d| < 512, i.e. every input whose rounded fixed-point value fits an int32 (what __float2int_rn returns there).  Prints
-// the number of mismatches and the number of inputs checked.  Built and run by tests/test_phase_round.py.
+// CPU check of csrc/phase_round.cuh: phase_fixed_rn(d) and both lanes of the two-wide phase_fixed_rn2 against
+// round-to-nearest-even of d * 2^22 for EVERY float d with |d| < 512, i.e. every input whose rounded fixed-point value
+// fits an int32 (what __float2int_rn returns there).  Prints the number of inputs with any mismatch and the number of
+// inputs checked.  Built and run by tests/test_phase_round.py.
 #include <cmath>
 #include <cstdio>
 #include "../../adaptive_optics_gym_b200/csrc/phase_round.cuh"
@@ -14,7 +15,10 @@ int main() {
       float d;
       std::memcpy(&d, &bits, sizeof d);
       const double ref = std::nearbyint((double)d * 4194304.0);   // exact product, ties to even
-      bad += (double)phase_fixed_rn(d) != ref;
+      // the two-wide form with d in one lane and -d in the other: over both signs, every input in both lanes
+      int32_t p0, p1;
+      phase_fixed_rn2(d, -d, &p0, &p1);
+      bad += (double)phase_fixed_rn(d) != ref || (double)p0 != ref || (double)p1 != -ref;
       ++n;
     }
   }

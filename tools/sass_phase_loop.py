@@ -5,7 +5,8 @@
 The chunk loop is the innermost backward branch around the kernel's tcgen05.ld (LDTM): its body handles one
 16-pixel chunk per epilogue warp.  For each instantiation <STREHL, NOBS, MODE, NP> (NP = 240 for every mode and detector
 size; 128, 256 and 512 for the fused modes 1 and 2 with NOBS 2 and 5) this prints the loop's instruction
-count, its XU (conversion / transcendental pipe) instructions, MUFU, F2I and F2F separately, its bulk and tensor
+count, its XU (conversion / transcendental pipe) instructions, MUFU, F2I and F2F separately, its packed FP32x2
+instructions (FFMA2, FADD2, FMUL2: one issue slot for two FP32 operations, counted under fma too), its bulk and tensor
 copy issues (UBLKCP, UTMALDG), the instructions of the fill path (the innermost BSSY .. BSYNC region that holds those
 copies: the prefetch issue, which a warp runs on every chunk in a per-warp ring and on every fourth chunk in a ring
 shared by four warps), and the mix over the pipes below.  Counts are static (both sides of a branch count), CPU only: cuobjdump -sass of the sm_100a cubin."""
@@ -77,6 +78,7 @@ def chunk_loop(body):
 
 
 COPIES = ('UBLKCP', 'UTMALDG')
+PACKED = ('FFMA2', 'FADD2', 'FMUL2')
 
 
 def fill_path(body, loop):
@@ -113,22 +115,24 @@ def main():
         pipes = collections.Counter(pipe_of(op) for _, op in loop)
         key = tuple(int(g) for g in m.groups())
         copies = sum(1 for _, op in loop if op.startswith(COPIES))
-        rows.append((key, len(loop), pipes['xu'], ops['MUFU'], ops['F2I'], ops['F2F'], copies, fill_path(body, loop), pipes))
+        packed = sum(ops[o] for o in PACKED)
+        rows.append((key, len(loop), pipes['xu'], ops['MUFU'], ops['F2I'], ops['F2F'], packed, copies, fill_path(body, loop), pipes))
     rows.sort()
     cols = ['fma', 'alu', 'xu', 'fp64', 'lsu', 'tmem', 'uniform', 'sync/branch', 'other']
     if args.md:
-        print('| instantiation | loop instr | XU | MUFU | F2I | F2F | copies | fill path | ' + ' | '.join(cols) + ' |')
-        print('|---' * (8 + len(cols)) + '|')
+        print('| instantiation | loop instr | XU | MUFU | F2I | F2F | packed | copies | fill path | ' + ' | '.join(cols) + ' |')
+        print('|---' * (9 + len(cols)) + '|')
     else:
-        print('%-16s %6s %4s %4s %4s %4s %6s %4s  ' % ('<S,NOBS,MODE,NP>', 'instr', 'XU', 'MUFU', 'F2I', 'F2F', 'copies', 'fill') +
+        print('%-16s %6s %4s %4s %4s %4s %6s %6s %4s  ' % ('<S,NOBS,MODE,NP>', 'instr', 'XU', 'MUFU', 'F2I', 'F2F', 'packed', 'copies',
+                                                             'fill') +
               ' '.join('%7s' % c[:7] for c in cols))
-    for key, n, xu, mufu, f2i, f2f, copies, fill, pipes in rows:
+    for key, n, xu, mufu, f2i, f2f, packed, copies, fill, pipes in rows:
         k = '<%d,%d,%d,%d>' % key
         if args.md:
-            print('| `%s` | %d | %d | %d | %d | %d | %d | %d | ' % (k, n, xu, mufu, f2i, f2f, copies, fill) +
+            print('| `%s` | %d | %d | %d | %d | %d | %d | %d | %d | ' % (k, n, xu, mufu, f2i, f2f, packed, copies, fill) +
                   ' | '.join(str(pipes[c]) for c in cols) + ' |')
         else:
-            print('%-16s %6d %4d %4d %4d %4d %6d %4d  ' % (k, n, xu, mufu, f2i, f2f, copies, fill) +
+            print('%-16s %6d %4d %4d %4d %4d %6d %6d %4d  ' % (k, n, xu, mufu, f2i, f2f, packed, copies, fill) +
                   ' '.join('%7d' % pipes[c] for c in cols))
     return 0 if rows else 1
 
