@@ -83,6 +83,7 @@ def load():
         'aog_get_screens': (C.c_int, [P, P, C.c_int, C.c_int]),
         'aog_generate_screens': (C.c_int, [P, P]),
         'aog_next_extrusions': (C.c_int, [P]),
+        'aog_set_turbulence': (C.c_int, [P, P, C.c_int, P]),
         'aog_reset': (C.c_int, [P, C.POINTER(AogOutputs), P]),
         'aog_reset_host': (C.c_int, [P, C.POINTER(AogOutputs)]),
         'aog_step': (C.c_int, [P, P, C.c_int, P, C.POINTER(AogOutputs), C.POINTER(C.c_int32), P]),
@@ -186,6 +187,14 @@ class Handle:
 
     def generate_screens(self, stream=None):
         self.check(self.lib.aog_generate_screens(self._h, C.c_void_p(stream or 0)), 'aog_generate_screens')
+
+    def set_turbulence(self, sqrt_cn2, rescale=False, stream=None):
+        """Per-env sqrt(Cn^2) [num_envs]; ``rescale`` also multiplies each env's screen by new / old."""
+        v = np.ascontiguousarray(sqrt_cn2, dtype=np.float64)
+        if v.shape != (self.cfg.num_envs,):
+            raise ValueError(f'sqrt_cn2 must have {self.cfg.num_envs} values')
+        self.check(self.lib.aog_set_turbulence(self._h, _ptr(v), int(bool(rescale)), C.c_void_p(stream or 0)),
+                   'aog_set_turbulence')
 
     def next_extrusions(self):
         return self.lib.aog_next_extrusions(self._h)

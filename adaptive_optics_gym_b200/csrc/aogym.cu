@@ -75,7 +75,7 @@ int extrude_once(aog_env* env, bool positive, const double* noise_dev, long long
     const int nB = std::min(env->chunk, B - e0);
     dim3 g1(cdiv(Ns + Np, 256), nB);
     k_ar_gather<<<g1, 256, 0, st>>>(env->screens, env->t_stencil, noise_dev, env->arZ, env->P, Np, Ns, e0, org,
-                                    flipped, c.sqrt_cn2, noise_stride, c.seed, (unsigned long long)c.env_id_base,
+                                    flipped, env->sqrt_cn2, noise_stride, c.seed, (unsigned long long)c.env_id_base,
                                     (unsigned long long)env->cnt.extrusions);
     AOG_LAUNCH_CHECK();
     // GEMM with the scatter into the ring slot (and the phase-tile refresh of the tensor / fused paths) in its epilogue
@@ -107,7 +107,7 @@ int extrude_direct(aog_env* env, bool positive, int n, const double* noise_dev, 
   for (int e0 = 0; e0 < B; e0 += env->chunk) {
     const int nB = std::min(env->chunk, B - e0);
     dim3 gn(cdiv(cdiv(Np, 4), 64), nB, n);
-    k_ar_noise<<<gn, 64, 0, st>>>(noise_dev, env->arNZ, Np, nB, n, e0, c.sqrt_cn2, (long long)n * Np, c.seed,
+    k_ar_noise<<<gn, 64, 0, st>>>(noise_dev, env->arNZ, Np, nB, n, e0, env->sqrt_cn2, (long long)n * Np, c.seed,
                                    (unsigned long long)c.env_id_base, (unsigned long long)env->cnt.extrusions);
     AOG_LAUNCH_CHECK();
     org = (int)env->cnt.column_origin;
@@ -352,6 +352,10 @@ int aog_create(const aog_config* cfg, aog_env** out) {
   A(dev_alloc(env, &env->act, B * K));
   AOG_CUDA(cudaMemset(env->act, 0, B * K * sizeof(double)));
   A(dev_alloc(env, (double**)&env->act_in, B * K));
+  // every env starts at the configured strength (aog_set_turbulence changes it per env)
+  env->sqrt_cn2_host.assign(B, c.sqrt_cn2);
+  A(dev_alloc(env, &env->sqrt_cn2, 2 * B));
+  AOG_CUDA(cudaMemcpy(env->sqrt_cn2, env->sqrt_cn2_host.data(), B * sizeof(double), cudaMemcpyHostToDevice));
   env->chunk = (int)std::min<size_t>(B, 4096);
   env->strehl_blocks = cdiv(env->P, 128);
   const size_t ch = env->chunk;
@@ -395,7 +399,7 @@ void aog_destroy(aog_env* env) {
   void* ptrs[] = {env->t_aperture, env->t_modes, env->t_gram, env->t_m1f, env->t_m2f, env->t_m1o, env->t_m2o,
                   env->t_lpw, env->t_lpphase, env->t_lpgram, env->t_stencil, env->t_stencil_perm, env->t_arA, env->t_arB, env->t_arW,
                   env->t_arW_rev, env->t_ar_tail, env->arNZ, env->t_scr_sh, env->t_scr_tw, env->t_scrC1, env->t_scrW1, env->t_scrW1T, env->t_scrC2, env->t_scrW2, env->t_scrW2T,
-                  env->screens, env->act, env->bufA, env->bufB, env->bufC, env->bufR, env->coef,
+                  env->screens, env->act, env->sqrt_cn2, env->bufA, env->bufB, env->bufC, env->bufR, env->coef,
                   env->strehl_part, env->arZ, env->act_in, env->noise_in, env->o_pack,
                   env->t_sh_mla, env->t_sh_C, env->t_sh_CT,
                   env->t_sh_off, env->t_sh_pix, env->t_sh_px, env->t_sh_py, env->t_sh_offset, env->t_sh_recon,
@@ -705,7 +709,7 @@ int aog_generate_screens(aog_env* env, void* stream) {
       k_scr_fft_rows<<<dim3(240 / FFT_LINES, nB), FFT_THREADS, FFT_SMEM, st>>>(Ctab, env->t_scr_sh, env->t_scr_tw, T, sB, e0, seed,
                                                                        (unsigned long long)c.env_id_base, draw_base);
       AOG_LAUNCH_CHECK();
-      k_scr_fft_cols<<<dim3(240 / FFT_LINES, nB), FFT_THREADS, FFT_SMEM, st>>>(T, sB, env->t_scr_tw, env->screens, P, e0, c.sqrt_cn2, accumulate,
+      k_scr_fft_cols<<<dim3(240 / FFT_LINES, nB), FFT_THREADS, FFT_SMEM, st>>>(T, sB, env->t_scr_tw, env->screens, P, e0, env->sqrt_cn2, accumulate,
                                                                        nullptr, 0.0, 0.0);
       AOG_LAUNCH_CHECK();
       return AOG_OK;
@@ -725,7 +729,7 @@ int aog_generate_screens(aog_env* env, void* stream) {
     }
     // with the FFT form this is the last writer of the screens: it also refreshes the phase tiles
     const bool wt = fft_form && accumulate && env->phase_tiles != nullptr;
-    k_scr_combine4<<<dim3(cdiv(Q, 256), nB), 256, 0, st>>>(env->screens, Pq, Np, sP, e0, c.sqrt_cn2, accumulate,
+    k_scr_combine4<<<dim3(cdiv(Q, 256), nB), 256, 0, st>>>(env->screens, Pq, Np, sP, e0, env->sqrt_cn2, accumulate,
                                                            wt ? env->phase_tiles : nullptr,
                                                            1.0 / (c.wavelength_wfs * 3.14159265358979323846), env->phase_tiles_unit);
     AOG_LAUNCH_CHECK();
@@ -751,7 +755,7 @@ int aog_generate_screens(aog_env* env, void* stream) {
     k_zgemm<<<dim3(cdiv(Np, 64), cdiv(Np, 64), nB), 256, 0, st>>>(env->bufB, env->t_scrW1T, env->bufC, Np, Np, Np, Np,
                                                                    Np, Np, sB, 0, sC);
     AOG_LAUNCH_CHECK();
-    k_scr_combine<<<dim3(cdiv(P, 256), nB), 256, 0, st>>>(env->screens, env->bufC, P, sC, e0, c.sqrt_cn2, 0);
+    k_scr_combine<<<dim3(cdiv(P, 256), nB), 256, 0, st>>>(env->screens, env->bufC, P, sC, e0, env->sqrt_cn2, 0);
     AOG_LAUNCH_CHECK();
     // scale 2: X2 [N2 x N2] -> W2 X2 W2^T
     k_scr_noise<<<dim3(cdiv(N2 * N2 / 2, 256), nB), 256, 0, st>>>(env->t_scrC2, env->bufA, N2 * N2, (long long)P, e0, seed,
@@ -763,11 +767,39 @@ int aog_generate_screens(aog_env* env, void* stream) {
     k_zgemm<<<dim3(cdiv(Np, 64), cdiv(Np, 64), nB), 256, 0, st>>>(env->bufB, env->t_scrW2T, env->bufC, Np, Np, N2, N2,
                                                                    Np, Np, sB, 0, sC);
     AOG_LAUNCH_CHECK();
-    k_scr_combine<<<dim3(cdiv(P, 256), nB), 256, 0, st>>>(env->screens, env->bufC, P, sC, e0, c.sqrt_cn2, 1);
+    k_scr_combine<<<dim3(cdiv(P, 256), nB), 256, 0, st>>>(env->screens, env->bufC, P, sC, e0, env->sqrt_cn2, 1);
     AOG_LAUNCH_CHECK();
   }
   env->cnt.column_origin = 0;
   if (c.precision != AOG_PRECISION_F64 && !tiles_done) return aog_tensor_screens_updated(env);
+  return AOG_OK;
+}
+
+int aog_set_turbulence(aog_env* env, const double* sqrt_cn2_host, int rescale, void* stream) {
+  if (!env || !sqrt_cn2_host) return AOG_ERR_INVALID;
+  const aog_config& c = env->cfg;
+  const int B = c.num_envs;
+  for (int b = 0; b < B; ++b)
+    if (!std::isfinite(sqrt_cn2_host[b]) || !(sqrt_cn2_host[b] > 0.0))
+      AOG_FAIL(AOG_ERR_INVALID, "sqrt_cn2 of env " + std::to_string(b) + " is not finite and positive");
+  AOG_DEVICE(c.device);
+  cudaStream_t st = (cudaStream_t)stream;
+  // [new values | new / old]: one upload (pageable source: staged before cudaMemcpyAsync returns)
+  std::vector<double> h(rescale ? 2 * (size_t)B : (size_t)B);
+  for (int b = 0; b < B; ++b) {
+    h[b] = sqrt_cn2_host[b];
+    if (rescale) h[B + b] = sqrt_cn2_host[b] / env->sqrt_cn2_host[b];
+  }
+  AOG_CUDA(cudaMemcpyAsync(env->sqrt_cn2, h.data(), h.size() * sizeof(double), cudaMemcpyHostToDevice, st));
+  env->sqrt_cn2_host.assign(sqrt_cn2_host, sqrt_cn2_host + B);
+  if (!rescale) return AOG_OK;
+  // the screens are a linear function of sqrt(Cn^2) (synthesis and AR extrusion alike): the same realisation at the new
+  // strength.  Elementwise, so the ring origin does not matter.
+  const double* factor = env->sqrt_cn2 + B;
+  if (env->phase_tiles) return aog_tensor_rescale_screens(env, factor, st);
+  const size_t total = (size_t)B * env->P;
+  k_scale_screens<<<(unsigned)((total + 255) / 256), 256, 0, st>>>(env->screens, factor, env->P, total);
+  AOG_LAUNCH_CHECK();
   return AOG_OK;
 }
 

@@ -4,6 +4,7 @@
 #include <cuda_fp16.h>
 #include <stdint.h>
 #include <string>
+#include <vector>
 #include "aogym.h"
 
 #define AOG_MAX_LP 8       // guided fibre modes kept in registers (reference config: 3)
@@ -79,6 +80,9 @@ struct aog_env {
   double* screens = nullptr;       // [B][Np x][Np y] COLUMN-major (a pupil column is contiguous: the extrusion reads and
                                    // writes whole columns), ring-buffered along x (column_origin)
   double* act = nullptr;           // [B][K] DM actuators (after normalisation)
+  double* sqrt_cn2 = nullptr;      // [2 B] turbulence strength sqrt(Cn^2) of each env (read by the screen synthesis and
+                                   // the extrusion noise), then the factors of the last aog_set_turbulence rescale
+  std::vector<double> sqrt_cn2_host;   // [B] host copy of the first half (the old values of a rescale)
 
   // ---- scratch for one chunk of envs ----
   int chunk = 0;

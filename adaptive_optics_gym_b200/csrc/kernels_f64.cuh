@@ -581,8 +581,9 @@ __device__ __forceinline__ void ar_normals4(unsigned long long seed, unsigned lo
 
 static __global__ void k_ar_gather(const double* __restrict__ screens, const int* __restrict__ stencil,
                             const double* __restrict__ noise, double* __restrict__ Z, int P, int Np, int Ns,
-                            int env0, int col_origin, int flipped, double sqrt_cn2, long long noise_stride,
-                            unsigned long long seed, unsigned long long env_id_base, unsigned long long draw_index) {
+                            int env0, int col_origin, int flipped, const double* __restrict__ sqrt_cn2,
+                            long long noise_stride, unsigned long long seed, unsigned long long env_id_base,
+                            unsigned long long draw_index) {
   const int b = blockIdx.y;
   const int j = blockIdx.x * blockDim.x + threadIdx.x;
   if (j >= Ns + Np) return;
@@ -605,7 +606,7 @@ static __global__ void k_ar_gather(const double* __restrict__ screens, const int
       ar_normals4(seed, env_id_base + env0 + b, draw_index, i >> 2, z);
       xi = (double)z[i & 3];
     }
-    v = sqrt_cn2 * xi;
+    v = sqrt_cn2[env0 + b] * xi;
   }
   Z[(size_t)b * (Ns + Np) + j] = v;
 }
@@ -614,11 +615,12 @@ static __global__ void k_ar_gather(const double* __restrict__ screens, const int
 // NZ[(e nB + b) Np + i], e < next;  the same Philox draws as k_ar_gather (extrusion e uses draw index draw0 + e), one
 // block per four normals, or the injected normals noise[(env0 + b) noise_stride + e Np + i].
 static __global__ void k_ar_noise(const double* __restrict__ noise, double* __restrict__ NZ, int Np, int nB, int next,
-                                  int env0, double sqrt_cn2, long long noise_stride, unsigned long long seed,
+                                  int env0, const double* __restrict__ sqrt_cn2, long long noise_stride, unsigned long long seed,
                                   unsigned long long env_id_base, unsigned long long draw0) {
   const int b = blockIdx.y, e = blockIdx.z;
   const int j = blockIdx.x * blockDim.x + threadIdx.x, i = 4 * j;
   if (i >= Np) return;
+  const double s = sqrt_cn2[env0 + b];         // loaded first: its latency hides under the Philox rounds
   double v[4];
   if (noise) {
     const double* src = noise + (size_t)(env0 + b) * noise_stride + (size_t)e * Np + i;
@@ -633,7 +635,7 @@ static __global__ void k_ar_noise(const double* __restrict__ noise, double* __re
   double* dst = NZ + ((size_t)e * nB + b) * Np + i;
 #pragma unroll
   for (int k = 0; k < 4; ++k)
-    if (i + k < Np) dst[k] = sqrt_cn2 * v[k];
+    if (i + k < Np) dst[k] = s * v[k];
 }
 
 // new column = Z . W (hcipy _extrude: A z + B xi for every env) on the FP64 tensor cores, with the scatter into the
@@ -1008,12 +1010,14 @@ k_scr_fft_rows(const double* __restrict__ C, const double2* __restrict__ sh, con
 }
 static __global__ void __launch_bounds__(FFT_THREADS)
 k_scr_fft_cols(const double2* __restrict__ T, long long sT, const double2* __restrict__ tw, double* __restrict__ screens,
-               int P, int env0, double scale, int accumulate, int32_t* __restrict__ tiles, double inv_w, double phi_one) {
+               int P, int env0, const double* __restrict__ sqrt_cn2, int accumulate, int32_t* __restrict__ tiles,
+               double inv_w, double phi_one) {
   constexpr int N = 240;
   extern __shared__ __align__(16) double2 fft_smem[];
   double2* buf = fft_smem;                       // [16 columns][FFT_LD]
   double2* tw_s = fft_smem + FFT_LINES * FFT_LD;
   const int b = blockIdx.y, x0 = blockIdx.x * FFT_LINES, t = threadIdx.x;
+  const double scale = sqrt_cn2[env0 + b];
   for (int i = t; i < N; i += FFT_THREADS) tw_s[i] = tw[i];
   const double2* tb = T + (size_t)b * sT;
   {
@@ -1074,7 +1078,7 @@ static __global__ void k_scr_noise_planes(const double* __restrict__ C, double* 
 // tiles != null (the last writer of a synthesis): also the fixed-point phase tiles of the tensor / fused paths
 // (TensorState::hwt, as k_ar_step's epilogue writes them; column origin 0)
 static __global__ void k_scr_combine4(double* __restrict__ screens, const double* __restrict__ Pq, int Np,
-                                      long long strideP, int env0, double scale, int accumulate,
+                                      long long strideP, int env0, const double* __restrict__ sqrt_cn2, int accumulate,
                                       int32_t* __restrict__ tiles, double inv_w, double phi_one) {
   const int Nh = Np / 2, Q = Nh * Nh;
   const int b = blockIdx.y;
@@ -1088,6 +1092,7 @@ static __global__ void k_scr_combine4(double* __restrict__ screens, const double
   const size_t idx[4] = {(size_t)x * Np + y, (size_t)(Np - 1 - x) * Np + y, (size_t)x * Np + (Np - 1 - y),
                          (size_t)(Np - 1 - x) * Np + (Np - 1 - y)};
   const size_t env = (size_t)env0 + b;
+  const double scale = sqrt_cn2[env];
   const int l = (int)(env & 31);
 #pragma unroll
   for (int c = 0; c < 4; ++c) {
@@ -1103,8 +1108,16 @@ static __global__ void k_scr_combine4(double* __restrict__ screens, const double
   }
 }
 
+// aog_set_turbulence's rescale on an FP64 handle: screens[b][*] *= factor[b] (the tensor / fused handles do this in
+// k_screens_to_tiles, which also rewrites the phase tiles)
+static __global__ void k_scale_screens(double* __restrict__ screens, const double* __restrict__ factor, int P,
+                                       size_t total) {
+  const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < total) screens[i] *= factor[i / P];
+}
+
 static __global__ void k_scr_combine(double* __restrict__ screens, const double2* __restrict__ Y, int P, long long strideY,
-                              int env0, double scale, int accumulate) {
+                              int env0, const double* __restrict__ sqrt_cn2, int accumulate) {
   const int b = blockIdx.y;
   const int p = blockIdx.x * blockDim.x + threadIdx.x;
   if (p >= P) return;
@@ -1112,7 +1125,7 @@ static __global__ void k_scr_combine(double* __restrict__ screens, const double2
   int Np = 1;
   while (Np * Np < P) ++Np;
   const int x = p / Np, y = p - x * Np;
-  const double v = scale * Y[(size_t)b * strideY + (size_t)y * Np + x].x;
+  const double v = sqrt_cn2[env0 + b] * Y[(size_t)b * strideY + (size_t)y * Np + x].x;
   double* s = screens + (size_t)(env0 + b) * P + p;
   *s = accumulate ? (*s + v) : v;
 }

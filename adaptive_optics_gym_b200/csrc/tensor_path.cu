@@ -1737,14 +1737,16 @@ __global__ void k_act_pack(const double* __restrict__ act, __half* __restrict__ 
 }
 
 // screens FP64 [B][xp][y] -> tiled fixed-point phase at lambda_wfs (layout: TensorState::hwt).
-// One thread per output int, output-ordered (coalesced writes, strided reads).
+// One thread per output int, output-ordered (coalesced writes, strided reads).  factor != null (aog_set_turbulence's
+// rescale): each env's screen is first multiplied in place by factor[env], and the tile is that of the product, so it
+// equals what a later plain conversion of the rescaled screens would write.
 __device__ __forceinline__ int32_t phase_fixed(double S, double inv) {
   double a = S * inv * (double)PHI_ONE;                  // half-turns x 2^22
   a = fmin(fmax(a, -2147483000.0), 2147483000.0);        // +-512 half-turns (1600 rad) of range
   return (int32_t)__double2ll_rn(a);
 }
-__global__ void k_screens_to_tiles(const double* __restrict__ src, int32_t* __restrict__ hwt, int Np, int B,
-                                   size_t total, double inv_w) {
+__global__ void k_screens_to_tiles(double* __restrict__ src, int32_t* __restrict__ hwt, int Np, int B,
+                                   size_t total, double inv_w, const double* __restrict__ factor) {
   const size_t o = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (o >= total) return;
   const int e = o & 3, piece = (o >> 2) & 3, l = (o >> 4) & 31;
@@ -1755,7 +1757,12 @@ __global__ void k_screens_to_tiles(const double* __restrict__ src, int32_t* __re
   const size_t env = (t2 / Np) * 32 + l;
   const int y = ci * 16 + ((piece ^ ((l >> 1) & 3)) << 2) + e;
   int32_t v = 0;
-  if (env < (size_t)B) v = phase_fixed(src[(env * Np + xp) * Np + y], inv_w);      // screens are [env][x][y]
+  if (env < (size_t)B) {
+    double* s = src + (env * Np + xp) * Np + y;                                      // screens are [env][x][y]
+    double S = *s;
+    if (factor) *s = S = S * factor[env];
+    v = phase_fixed(S, inv_w);
+  }
   hwt[o] = v;
 }
 
@@ -2221,9 +2228,20 @@ int aog_tensor_screens_updated(aog_env* env) {
   const double pi = 3.14159265358979323846;
   const size_t total = (size_t)((B + 127) / 128) * 4 * Np * (Np / 16) * 512;
   k_screens_to_tiles<<<(unsigned)((total + 255) / 256), 256>>>(env->screens, ts->hwt, Np, B, total,
-                                                              1.0 / (env->cfg.wavelength_wfs * pi));
+                                                              1.0 / (env->cfg.wavelength_wfs * pi), nullptr);
   AOG_LAUNCH_CHECK();
   AOG_CUDA(cudaDeviceSynchronize());
+  return AOG_OK;
+}
+
+int aog_tensor_rescale_screens(aog_env* env, const double* factor_dev, cudaStream_t st) {
+  TensorState* ts = TS(env);
+  const int Np = env->cfg.num_pupil_pixels, B = env->cfg.num_envs;
+  const double pi = 3.14159265358979323846;
+  const size_t total = (size_t)((B + 127) / 128) * 4 * Np * (Np / 16) * 512;
+  k_screens_to_tiles<<<(unsigned)((total + 255) / 256), 256, 0, st>>>(env->screens, ts->hwt, Np, B, total,
+                                                                     1.0 / (env->cfg.wavelength_wfs * pi), factor_dev);
+  AOG_LAUNCH_CHECK();
   return AOG_OK;
 }
 

@@ -6,6 +6,8 @@ int aog_tensor_create(aog_env* env);
 void aog_tensor_destroy(aog_env* env);
 int aog_tensor_table_updated(aog_env* env, int which, const void* host);
 int aog_tensor_screens_updated(aog_env* env);
+// every env's screen times factor_dev[env] (device [B]) and its phase tiles rewritten, stream-ordered on st
+int aog_tensor_rescale_screens(aog_env* env, const double* factor_dev, cudaStream_t st);
 int aog_tensor_optics(aog_env* env, bool flat_dm, bool with_reward, const aog_outputs& out, cudaStream_t st);
 int aog_tensor_check(aog_env* env);
 int aog_tensor_actuators(aog_env* env, const void* actions_dev, int act_dtype, cudaStream_t st);

@@ -20,7 +20,7 @@ import numpy as np
 
 from . import _lib
 from ._gym_compat import Env, spaces
-from .tables import AOConfig, build_sh_tables, build_tables, synthesize_screens
+from .tables import FRIED_MIN, AOConfig, build_sh_tables, build_tables, sqrt_cn2_from_fried, synthesize_screens
 
 
 def _coerce_velocity(atm_type, velocity_value):
@@ -34,6 +34,25 @@ def _coerce_velocity(atm_type, velocity_value):
         print('therefore velocity value is changed to 1 m/s')
         velocity_value = 1
     return velocity_value
+
+
+def fried_values(r0, num_envs):
+    """A Fried parameter given per env -> (float64 [num_envs], was a scalar).  ``r0``: a scalar (broadcast), or a
+    sequence, NumPy array or tensor (a CUDA tensor is copied to the host) of ``num_envs`` values, each finite and at
+    least ``FRIED_MIN`` m (below it the fixed-point phase of the tensor / fused paths could saturate)."""
+    if hasattr(r0, 'detach'):
+        r0 = r0.detach().cpu().numpy()
+    a = np.asarray(r0, dtype=np.float64)
+    scalar = a.ndim == 0
+    if scalar:
+        a = np.full(num_envs, float(a))
+    if a.shape != (num_envs,):
+        raise ValueError(f'atm_fried must be a scalar or {num_envs} values (one per env), got shape {a.shape}')
+    if not np.all(np.isfinite(a)) or np.any(a <= 0):
+        raise ValueError('atm_fried values must be finite and positive')
+    if np.any(a < FRIED_MIN):
+        raise ValueError(f'atm_fried values must be >= {FRIED_MIN} m (the fixed-point phase saturates below it)')
+    return a, scalar
 
 
 class _AOCore:
@@ -58,8 +77,11 @@ class _AOCore:
         self.rew_threshold = rew_threshold
         self.SH_operation = SH_operation
         self.num_envs = int(num_envs)
+        # a scalar keeps the handle-wide value of cfg.sqrt_cn2; a sequence is validated here, before any device call
+        fried = None if np.ndim(atm_fried) == 0 else fried_values(atm_fried, self.num_envs)[0]
         velocity = _coerce_velocity(atm_type, atm_vel)
-        cfg = AOConfig(atm_type=atm_type, velocity=float(velocity), fried_parameter=float(atm_fried),
+        cfg = AOConfig(atm_type=atm_type, velocity=float(velocity),
+                       fried_parameter=float(atm_fried) if fried is None else float(fried[0]),
                        act_type=act_type, num_modes=int(act_dim), obs_dim=int(obs_dim), rew_type=rew_type,
                        max_steps=int(timesteps_per_episode), num_pupil_pixels=int(num_pupil_pixels),
                        num_focal_pixels_fiber=int(num_focal_pixels_fiber))
@@ -69,6 +91,8 @@ class _AOCore:
                   'delta_t', 'max_steps', 'velocity', 'fried_parameter', 'outer_scale',
                   'singlemode_fiber_core_radius', 'multimode_fiber_core_radius'):
             setattr(self, k, getattr(cfg, k))
+        if fried is not None:
+            self.fried_parameter = fried.copy()
         self.num_focal_pixels_fiber = cfg.num_focal_pixels_fiber
         self.num_focal_pixels_fiber_subsample = cfg.obs_dim
         # The reference draws its screens and noise from NumPy's unseeded global generator (every construction is a
@@ -134,6 +158,8 @@ class _AOCore:
             for name in _lib.TABLE_IDS:
                 if name.startswith('sh_'):
                     self._h.set_table(name, sh[name])
+        if fried is not None:
+            self._h.set_turbulence(sqrt_cn2_from_fried(fried, cfg.wavelength_sci))
         # initial screen(s) (hcipy draws one at construction; AO_env.py:370)
         if initial_screens is not None:
             s = np.asarray(initial_screens)
@@ -150,6 +176,23 @@ class _AOCore:
         self.timestep_render = 0
 
     # ---- state shared by both front ends
+    def _stream(self):
+        return 0
+
+    def _set_fried(self, r0, rescale):
+        """New per-env Fried parameters for every later screen synthesis and extrusion; ``rescale`` also scales each
+        env's current screen by (r0_old / r0_new)^(5/6): the same realisation at the new strength."""
+        vals, scalar = fried_values(r0, self.num_envs)
+        self._h.set_turbulence(sqrt_cn2_from_fried(vals, self.wavelength_sci), rescale, self._stream())
+        self.fried_parameter = float(vals[0]) if scalar else vals
+
+    def _reset_options(self, options):
+        """``options={'atm_fried': r0}`` of ``reset``: semi_dynamic draws this reset's screens at the new strength;
+        quasi_static and dynamic rescale the screens they keep (for dynamic the AR process is linear in sqrt(Cn^2),
+        so later extrusions continue it consistently)."""
+        if options and 'atm_fried' in options:
+            self._set_fried(options['atm_fried'], rescale=self.atm_type != 'semi_dynamic')
+
     def _sync_counters(self):
         c = self._h.counters()
         self.timestep, self.timestep_render, self.episode_no = c.timestep, c.timestep_render, c.episode_no
@@ -161,13 +204,16 @@ class _AOCore:
         c = self._h.counters()
         st = dict(screens=self._h.get_screens(), actuators=self._h.get_actuators(),
                   timestep=c.timestep, timestep_render=c.timestep_render, episode_no=c.episode_no,
-                  extrusions=c.extrusions, screen_draws=c.screen_draws, sh_draws=c.sh_draws, seed=self._seed)
+                  extrusions=c.extrusions, screen_draws=c.screen_draws, sh_draws=c.sh_draws, seed=self._seed,
+                  fried_parameter=np.copy(self.fried_parameter) if np.ndim(self.fried_parameter) else self.fried_parameter)
         if self.SH_operation:
             st['sh_actuators'] = self._h.get_sh_actuators()
         return st
 
     def set_state(self, state):
         self._h.set_counters(column_origin=0)
+        if 'fried_parameter' in state:       # dicts written before per-env strengths existed leave them untouched
+            self._set_fried(state['fried_parameter'], rescale=False)
         self._h.set_screens(state['screens'])
         self._h.set_actuators(state['actuators'])
         if 'seed' in state:
@@ -207,7 +253,7 @@ class AOEnv(_AOCore, Env):
                  precision=None, tables=None, initial_screen=None, num_pupil_pixels=240,
                  num_focal_pixels_fiber=128, env_id_base=0):
         super().__init__()
-        self._setup(atm_type=atm_type, atm_vel=atm_vel, atm_fried=atm_fried, act_type=act_type, act_dim=act_dim,
+        self._setup(atm_type=atm_type, atm_vel=atm_vel, atm_fried=float(atm_fried), act_type=act_type, act_dim=act_dim,
                     obs_dim=obs_dim, rew_type=rew_type, rew_threshold=rew_threshold,
                     timesteps_per_episode=timesteps_per_episode,
                     flat_mirror_start_per_episode=flat_mirror_start_per_episode, SH_operation=SH_operation,
@@ -225,10 +271,12 @@ class AOEnv(_AOCore, Env):
     def reset(self, seed=None, options=None):
         """AO_env.py:74-103 -> (float16 obs [obs_dim^2], {}).  The reference ignores ``seed`` (its noise comes from
         NumPy's global generator); here ``seed=s`` re-keys the device's random streams first, so everything drawn from
-        this reset on (a ``semi_dynamic`` screen, extrusion noise, photon noise) is reproducible.  ``options`` is
-        ignored as in the reference."""
+        this reset on (a ``semi_dynamic`` screen, extrusion noise, photon noise) is reproducible.  The reference
+        ignores ``options``; here ``options={'atm_fried': r0}`` (a scalar) sets a new Fried parameter from this reset
+        on (see ``AOVecEnv.reset``)."""
         if seed is not None:
             self._reseed(seed)
+        self._reset_options(options)
         h = self._h.reset_host()
         self._sync_counters()
         self.last_obs_f64 = h['obs_f64'][0].copy()
@@ -308,6 +356,13 @@ class AOVecEnv(_AOCore):
     with ``env_id_base = rank * num_envs`` (RNG stream = global env id); no collective on the
     step path.
 
+    ``atm_fried`` is a scalar (every env sees the same turbulence) or one Fried parameter per env (a sequence, NumPy
+    array or tensor of ``num_envs`` values, each >= ``tables.FRIED_MIN`` = 1 cm): domain randomisation or evaluation
+    across seeing in one batch.  ``fried_parameter`` is then an ``np.ndarray``.  ``reset(options={'atm_fried': r0})``
+    changes the values from that episode on.  A sharded run passes each rank its slice ``r0[first:first + count]`` of
+    ``sharding.shard_range`` with ``env_id_base = first``, so that env i sees the same r0 and random streams as in one
+    handle.
+
     The tensors returned by ``reset`` / ``step`` / ``SH_step`` (``obs``, ``reward``, ``power``, ``sh_action``, the
     ``done`` masks) are VIEWS OF REUSED OUTPUT BUFFERS: the next call overwrites them in place.  A caller that keeps
     them across calls (a replay buffer, ``next_obs`` bookkeeping) must ``.clone()`` them -- ``rollout.py`` does.
@@ -354,8 +409,12 @@ class AOVecEnv(_AOCore):
         return self._torch.cuda.current_stream(self.device).cuda_stream
 
     def reset(self, seed=None, options=None):
+        """-> (obs, {}).  ``options={'atm_fried': r0}``: new Fried parameters from this episode on, r0 a scalar or
+        ``num_envs`` values (sequence, array or tensor).  semi_dynamic draws this reset's screens at them; quasi_static
+        and dynamic keep their screens, scaled per env by (r0_old / r0_new)^(5/6)."""
         if seed is not None:
             self._reseed(seed)
+        self._reset_options(options)
         self._h.reset_device(self._out, self._stream())
         self._sync_counters()
         return self.obs, {}

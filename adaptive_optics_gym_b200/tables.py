@@ -194,6 +194,21 @@ def cn2_from_fried(r0, wavelength):
     return r0 ** (-5.0 / 3) / (0.423 * (2 * np.pi / wavelength) ** 2)
 
 
+# Smallest Fried parameter accepted per env.  The tensor / fused paths hold the phase S / lambda_wfs as int32 fixed point
+# that saturates at +-512 half-turns (1608 rad).  A screen scales as r0^(-5/6); at r0 = 0.20 m the largest |S| / lambda_wfs
+# of 400 synthesised 240 x 240 screens is 33 rad (piston included: the 10 m outer scale gives each screen an offset of
+# ~11 rad RMS).  Budgeting 100 rad at 0.20 m (3x that, and 9 sigma of the offset), the clamp is reached at
+# r0 = 0.20 (100 / 1608)^(6/5) = 7.1 mm; the floor rounds that up to 1 cm, where the observed maximum (400 rad) is 4x
+# below the clamp.
+FRIED_MIN = 0.01
+
+
+def sqrt_cn2_from_fried(r0s, wavelength):
+    """sqrt(Cn^2) of each r0, converted one Python float at a time: entry i equals, bit for bit, the value a handle built
+    with the scalar r0s[i] uses (a vectorised power may round the last bit differently)."""
+    return np.array([float(np.sqrt(cn2_from_fried(float(r), wavelength))) for r in r0s], dtype=np.float64)
+
+
 def von_karman_covariance(r, r0, L0):
     r = r + 1e-10
     q = 2 * np.pi * r / L0

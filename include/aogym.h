@@ -183,6 +183,12 @@ AOG_API int aog_get_screens(aog_env* env, double* host_out, int first_env, int c
 /* new von-Karman screens for all envs from the on-device generator (semi_dynamic reset) */
 AOG_API int aog_generate_screens(aog_env* env, void* stream);
 
+/* per-env turbulence strength sqrt(Cn^2) [N] FP64 (host pointer), used by every later screen synthesis and
+   extrusion; rescale != 0 also multiplies each env's current screen by new/old and refreshes its phase tiles.
+   Values must be finite and > 0 (else AOG_ERR_INVALID, nothing changed).  aog_create starts every env at
+   cfg.sqrt_cn2.  Stream-ordered on `stream`: no device synchronisation. */
+AOG_API int aog_set_turbulence(aog_env* env, const double* sqrt_cn2_host, int rescale, void* stream);
+
 /* number of column extrusions the next aog_step will perform (sizes `noise`) */
 AOG_API int aog_next_extrusions(const aog_env* env);
 
