@@ -102,6 +102,7 @@ def load():
         'aog_get_field': (C.c_int, [P, C.c_int, C.c_int, P, C.c_size_t]),
         'aog_debug_poisson': (C.c_int, [C.c_int, C.c_double, C.c_int, C.c_uint64, P]),
         'aog_debug_poisson_f32': (C.c_int, [C.c_int, C.c_double, C.c_int, C.c_uint64, P]),
+        'aog_debug_normals': (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int, P, P, P]),
         'aog_launch_count': (C.c_int64, [P]),
         'aog_chunk_size': (C.c_int, [P]),
         'aog_set_timing': (C.c_int, [P, C.c_int]),

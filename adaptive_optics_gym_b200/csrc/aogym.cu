@@ -1295,6 +1295,13 @@ int aog_debug_poisson_f32(int device, double lambda, int n, uint64_t seed, doubl
   return aog_tensor_debug_poisson(device, lambda, n, seed, host_out);
 }
 
+int aog_debug_normals(int device, int generator, int philox, int n, const uint32_t* words_in, uint32_t* raw_out,
+                      float* normals_out) {
+  if (!words_in || !normals_out || (philox && !raw_out) || n < 1 || (generator != 0 && generator != 1))
+    return AOG_ERR_INVALID;
+  return aog_tensor_debug_normals(device, generator, philox, n, words_in, raw_out, normals_out);
+}
+
 int64_t aog_launch_count(const aog_env* env) { return env ? env->launches : -1; }
 
 int aog_chunk_size(const aog_env* env) { return env ? env->chunk : AOG_ERR_INVALID; }

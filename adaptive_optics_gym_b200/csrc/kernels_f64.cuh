@@ -559,9 +559,10 @@ __device__ __forceinline__ uint4 aog_philox4x32_10(uint4 c, uint2 k) {
   }
   return c;
 }
-// four standard normals from one block: two Box-Muller transforms in FP32 on the SFU (24-bit uniforms; a deviate good
-// to ~1e-6, |z| <= 5.9).  The draws only have to be normal and reproducible from (seed, env, index) -- parity with the
-// reference is through injected noise -- and curand's FP64 Box-Muller cost 58 us per step of 4096 envs at 20 m/s.
+// four standard normals from one block: two Box-Muller transforms in FP32 on the SFU (24-bit uniforms in (0, 1]; over all
+// of them within 3.5e-5 of an FP64 Box-Muller on B200, |z| <= 5.9: tests/test_device_noise_gpu.py).  The draws only
+// have to be normal and reproducible from (seed, env, index) -- parity with the reference is through injected noise --
+// and curand's FP64 Box-Muller cost 58 us per step of 4096 envs at 20 m/s.
 __device__ __forceinline__ void aog_normals4(uint4 r, float (&z)[4]) {
   const float u0 = ((float)(r.x >> 8) + 0.5f) * (1.0f / 16777216.0f), u1 = ((float)(r.y >> 8) + 0.5f) * (1.0f / 16777216.0f);
   const float u2 = ((float)(r.z >> 8) + 0.5f) * (1.0f / 16777216.0f), u3 = ((float)(r.w >> 8) + 0.5f) * (1.0f / 16777216.0f);

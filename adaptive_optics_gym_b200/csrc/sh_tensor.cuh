@@ -342,7 +342,7 @@ __device__ __forceinline__ uint4 philox4x32_10(uint4 c, uint2 k) {
   }
   return c;
 }
-__device__ __forceinline__ float u01(uint32_t r) { return ((float)(r >> 8) + 0.5f) * (1.0f / 16777216.0f); }   // (0, 1)
+__device__ __forceinline__ float u01(uint32_t r) { return ((float)(r >> 8) + 0.5f) * (1.0f / 16777216.0f); }   // (0, 1]: the top words round to 1 - 2^-23 and 1.0
 
 // Photon count at rate lam (hcipy large_poisson, AO_env.py:274) in FP32 arithmetic:
 //   lam > 1e6      rounded normal, as large_poisson itself does
@@ -565,6 +565,30 @@ __global__ void k_debug_poisson_f32(float lam, int n, unsigned long long seed, d
   float z[4];
   normals4(philox4x32_10(ctr, key), z);
   out[i] = (double)(lam >= 10.f ? poisson_large_f32(lam, z[i & 3]) : poisson_small_f32(lam, ctr, key, i & 3));
+}
+
+// test hook (aog_debug_normals): block i -> raw[i] = Philox-4x32-10 of (counter words[6 i .. 6 i + 3], key
+// words[6 i + 4 .. 6 i + 5]) when `philox`, else raw[i] = words[4 i .. 4 i + 3]; z[4 i ..] = the four normals of raw[i]
+// by the extrusion / synthesis generator (cam = 0: aog_philox4x32_10, aog_normals4) or the camera's (cam = 1)
+__global__ void k_debug_normals(const uint32_t* __restrict__ words, int n, int philox, int cam,
+                                uint32_t* __restrict__ raw, float* __restrict__ z) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  uint4 r;
+  if (philox) {
+    const uint32_t* w = words + (size_t)6 * i;
+    const uint4 c = make_uint4(w[0], w[1], w[2], w[3]);
+    const uint2 k = make_uint2(w[4], w[5]);
+    r = cam ? philox4x32_10(c, k) : aog_philox4x32_10(c, k);
+    raw[4 * (size_t)i] = r.x; raw[4 * (size_t)i + 1] = r.y; raw[4 * (size_t)i + 2] = r.z; raw[4 * (size_t)i + 3] = r.w;
+  } else {
+    const uint32_t* w = words + (size_t)4 * i;
+    r = make_uint4(w[0], w[1], w[2], w[3]);
+  }
+  float o[4];
+  if (cam) normals4(r, o); else aog_normals4(r, o);
+#pragma unroll
+  for (int k = 0; k < 4; ++k) z[4 * (size_t)i + k] = o[k];
 }
 
 // ----------------------------------------------------------------------------- host side
@@ -885,6 +909,24 @@ int aog_tensor_debug_poisson(int device, double lambda, int n, uint64_t seed, do
   if (cudaMalloc((void**)&d, (size_t)n * sizeof(double)) != cudaSuccess) return AOG_ERR_CUDA;
   k_debug_poisson_f32<<<cdiv(n, 256), 256>>>((float)lambda, n, (unsigned long long)seed, d);
   const cudaError_t e = cudaMemcpy(host_out, d, (size_t)n * sizeof(double), cudaMemcpyDeviceToHost);
+  cudaFree(d);
+  return e == cudaSuccess ? AOG_OK : AOG_ERR_CUDA;
+}
+
+int aog_tensor_debug_normals(int device, int generator, int philox, int n, const uint32_t* words_in, uint32_t* raw_out,
+                             float* normals_out) {
+  DeviceGuard guard(device);
+  if (guard.err != cudaSuccess) return AOG_ERR_CUDA;
+  const size_t nw = (size_t)n * (philox ? 6 : 4), nr = philox ? (size_t)n * 4 : 0, nz = (size_t)n * 4;
+  uint32_t* d = nullptr;                                          // [words | raw | normals]
+  if (cudaMalloc((void**)&d, (nw + nr + nz) * sizeof(uint32_t)) != cudaSuccess) return AOG_ERR_CUDA;
+  float* dz = reinterpret_cast<float*>(d + nw + nr);
+  cudaError_t e = cudaMemcpy(d, words_in, nw * sizeof(uint32_t), cudaMemcpyHostToDevice);
+  if (e == cudaSuccess) {
+    k_debug_normals<<<cdiv(n, 256), 256>>>(d, n, philox, generator, d + nw, dz);
+    e = cudaMemcpy(normals_out, dz, nz * sizeof(float), cudaMemcpyDeviceToHost);
+  }
+  if (e == cudaSuccess && philox) e = cudaMemcpy(raw_out, d + nw, nr * sizeof(uint32_t), cudaMemcpyDeviceToHost);
   cudaFree(d);
   return e == cudaSuccess ? AOG_OK : AOG_ERR_CUDA;
 }

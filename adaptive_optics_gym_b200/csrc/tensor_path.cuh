@@ -18,3 +18,5 @@ int aog_tensor_sh_step(aog_env* env, int noise_mode, double* action_out_dev, cud
 // noise-free camera image of one env through the tensor-core kernels (tests)
 int aog_tensor_sh_image(aog_env* env, int env_index, double* host_out, size_t count);
 int aog_tensor_debug_poisson(int device, double lambda, int n, uint64_t seed, double* host_out);
+int aog_tensor_debug_normals(int device, int generator, int philox, int n, const uint32_t* words_in, uint32_t* raw_out,
+                             float* normals_out);

@@ -271,19 +271,25 @@ def screen_synthesis_tables(n, delta, L0, oversampling=16):
 def synthesize_screens(tabs, num, cn2, rng):
     """Host-side screen synthesis from ``screen_synthesis_tables`` (construction time and
     CPU tests; the per-episode ``semi_dynamic`` regeneration runs on the GPU)."""
-    C1, W1, C2, W2 = tabs['scr_C1'], tabs['scr_W1'], tabs['scr_C2'], tabs['scr_W2']
-    n = C1.shape[0]
-    out = np.empty((num, n * n))
+    C1, C2 = tabs['scr_C1'], tabs['scr_C2']
+    out = np.empty((num, C1.size))
     for i in range(num):
         z1 = rng.standard_normal(C1.shape) + 1j * rng.standard_normal(C1.shape)
         z2 = rng.standard_normal(C2.shape) + 1j * rng.standard_normal(C2.shape)
-        # W1 is a (shifted) DFT: use the FFT for the fine grid
-        k1 = np.fft.fftfreq(n, d=1.0 / n)
-        sh = W1[0, :]                                  # exp(2 pi i f_k x_0)
-        s = (np.fft.ifft2(C1 * z1 * sh[None, :] * sh[:, None]) * n * n).real
-        s += (W2 @ (C2 * z2) @ W2.T).real
-        out[i] = s.ravel() * np.sqrt(cn2)
+        out[i] = synthesize_screen(tabs, z1, z2, np.sqrt(cn2))
     return out
+
+
+def synthesize_screen(tabs, z1, z2, sqrt_cn2):
+    """One screen [y][x] (flattened) of ``synthesize_screens`` from given complex normals: z1 [n][n] and z2 [n2][n2],
+    indexed [ky][kx] like the tables."""
+    C1, W1, C2, W2 = tabs['scr_C1'], tabs['scr_W1'], tabs['scr_C2'], tabs['scr_W2']
+    n = C1.shape[0]
+    # W1 is a (shifted) DFT: use the FFT for the fine grid
+    sh = W1[0, :]                                      # exp(2 pi i f_k x_0)
+    s = (np.fft.ifft2(C1 * z1 * sh[None, :] * sh[:, None]) * n * n).real
+    s += (W2 @ (C2 * z2) @ W2.T).real
+    return s.ravel() * sqrt_cn2
 
 
 # ---------------------------------------------------------------- everything

@@ -240,6 +240,13 @@ AOG_API int aog_debug_poisson(int device, double lambda, int n, uint64_t seed, d
 /* the FP32 photon-noise sampler of the tensor / fused handles' Shack-Hartmann camera (same test hook) */
 AOG_API int aog_debug_poisson_f32(int device, double lambda, int n, uint64_t seed, double* host_out);
 
+/* test hook: n Philox-4x32-10 blocks and the four standard normals the device makes of each.  philox != 0: words_in
+ * holds n groups (counter[4], key[2]) and raw_out [n][4] receives the generator's words; philox == 0: words_in holds n
+ * raw blocks [n][4] (raw_out unused).  generator 0: the extrusion noise and screen synthesis (aog_normals4), 1: the
+ * Shack-Hartmann camera (normals4).  normals_out [n][4] */
+AOG_API int aog_debug_normals(int device, int generator, int philox, int n, const uint32_t* words_in, uint32_t* raw_out,
+                              float* normals_out);
+
 /* kernels launched by this handle since creation (bench.py's gpu_launches) */
 AOG_API int64_t aog_launch_count(const aog_env* env);
 /* environments processed per kernel sequence (num_envs is walked in chunks of this size) */
