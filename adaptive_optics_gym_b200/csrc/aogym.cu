@@ -13,20 +13,10 @@
 
 namespace {
 
-template <typename T>
-int dev_alloc(aog_env* env, T** p, size_t count) {
-  if (*p) { cudaFree(*p); *p = nullptr; }
-  if (count == 0) return AOG_OK;
-  AOG_CUDA(cudaMalloc((void**)p, count * sizeof(T)));
-  return AOG_OK;
-}
-
 int ensure_pinned(aog_env* env, size_t bytes) {
   if (bytes <= env->h_pinned_cap) return AOG_OK;
-  if (env->h_pinned) cudaFreeHost(env->h_pinned);
-  env->h_pinned = nullptr;
   env->h_pinned_cap = 0;
-  AOG_CUDA(cudaMallocHost(&env->h_pinned, bytes));
+  if (int rc = env->h_pinned.alloc(env, bytes)) return rc;
   env->h_pinned_cap = bytes;
   return AOG_OK;
 }
@@ -99,7 +89,7 @@ int extrude_direct(aog_env* env, bool positive, int n, const double* noise_dev, 
   const int flipped = positive ? 1 : 0;
   { int rc = dmma_configure(env); if (rc) return rc; }
   if (n > env->arNZ_cap) {
-    int rc = dev_alloc(env, &env->arNZ, (size_t)n * env->chunk * Np);
+    int rc = env->arNZ.alloc(env, (size_t)n * env->chunk * Np);
     if (rc) return rc;
     env->arNZ_cap = n;
   }
@@ -164,7 +154,7 @@ int optics_chunk_f64(aog_env* env, int e0, int nB, bool flat_dm, bool with_rewar
         flat_dm ? 1 : 0);
     AOG_LAUNCH_CHECK();
   }
-  if (env->timing) { AOG_CUDA(cudaEventRecord(env->ev0, st)); }
+  if (env->timing) { AOG_CUDA(cudaEventRecord(env->ev0.get(), st)); }
   {  // T = M1 . E    [Nf x Np] . [Np x Np]
     dim3 g(cdiv(Np, 64), cdiv(Nf, 64), nB);
     k_zgemm<<<g, 256, 0, st>>>(env->t_m1f, env->bufA, env->bufB, Nf, Np, Np, Np, Np, Np, 0, (long long)P,
@@ -177,7 +167,7 @@ int optics_chunk_f64(aog_env* env, int e0, int nB, bool flat_dm, bool with_rewar
                                (long long)env->NF2);
     AOG_LAUNCH_CHECK();
   }
-  if (env->timing) { AOG_CUDA(cudaEventRecord(env->ev1, st)); env->ev_valid = true; }
+  if (env->timing) { AOG_CUDA(cudaEventRecord(env->ev1.get(), st)); env->ev_valid = true; }
   const double2 norm = make_double2(c.mft_norm_re, c.mft_norm_im);
   if (with_reward) {
     k_fiber_f64<<<nB, 256, 0, st>>>(env->bufC, env->t_lpw, env->coef, env->NF2, J, (long long)env->NF2, norm);
@@ -224,7 +214,7 @@ int alloc_host_outputs(aog_env* env) {
   if (env->o_pack) return AOG_OK;
   const size_t bytes = B * n2 * sizeof(double) + 4 * B * sizeof(double) + B * n2 * sizeof(uint16_t);
   int rc;
-  if ((rc = dev_alloc(env, &env->o_pack, bytes))) return rc;
+  if ((rc = env->o_pack.alloc(env, bytes))) return rc;
   env->o_pack_bytes = bytes;
   AOG_CUDA(cudaMemset(env->o_pack, 0, bytes));
   char* p = env->o_pack;
@@ -270,9 +260,9 @@ int ensure_f64_scratch(aog_env* env) {
   const aog_config& c = env->cfg;
   const size_t ch = env->chunk, P = env->P;
   int rc;
-  if ((rc = dev_alloc(env, &env->bufA, ch * P))) return rc;
-  if ((rc = dev_alloc(env, &env->bufB, ch * (size_t)c.num_pupil_pixels * std::max(c.num_focal_pixels, c.num_pupil_pixels)))) return rc;
-  if ((rc = dev_alloc(env, &env->bufC, ch * std::max<size_t>(env->NF2, P)))) return rc;
+  if ((rc = env->bufA.alloc(env, ch * P))) return rc;
+  if ((rc = env->bufB.alloc(env, ch * (size_t)c.num_pupil_pixels * std::max(c.num_focal_pixels, c.num_pupil_pixels)))) return rc;
+  if ((rc = env->bufC.alloc(env, ch * std::max<size_t>(env->NF2, P)))) return rc;
   return AOG_OK;
 }
 
@@ -321,73 +311,70 @@ int aog_create(const aog_config* cfg, aog_env** out) {
   const size_t P = env->P, B = c.num_envs;
   int rc;
 #define A(expr) if ((rc = (expr))) return rc
-  A(dev_alloc(env, &env->t_aperture, P));
-  A(dev_alloc(env, &env->t_modes, (size_t)K * P));
-  A(dev_alloc(env, &env->t_gram, (size_t)K * K));
-  A(dev_alloc(env, &env->t_m1f, (size_t)Nf * Np));
-  A(dev_alloc(env, &env->t_m2f, (size_t)Np * Nf));
-  A(dev_alloc(env, &env->t_m1o, (size_t)n * Np));
-  A(dev_alloc(env, &env->t_m2o, (size_t)Np * n));
-  A(dev_alloc(env, &env->t_lpw, (size_t)J * env->NF2));
-  A(dev_alloc(env, &env->t_lpphase, (size_t)J));
-  A(dev_alloc(env, &env->t_lpgram, (size_t)J * J));
+  A(env->t_aperture.alloc(env, P));
+  A(env->t_modes.alloc(env, (size_t)K * P));
+  A(env->t_gram.alloc(env, (size_t)K * K));
+  A(env->t_m1f.alloc(env, (size_t)Nf * Np));
+  A(env->t_m2f.alloc(env, (size_t)Np * Nf));
+  A(env->t_m1o.alloc(env, (size_t)n * Np));
+  A(env->t_m2o.alloc(env, (size_t)Np * n));
+  A(env->t_lpw.alloc(env, (size_t)J * env->NF2));
+  A(env->t_lpphase.alloc(env, (size_t)J));
+  A(env->t_lpgram.alloc(env, (size_t)J * J));
   if (c.num_stencil > 0) {
-    A(dev_alloc(env, &env->t_stencil, (size_t)c.num_stencil));
-    A(dev_alloc(env, &env->t_arA, (size_t)Np * c.num_stencil));
-    A(dev_alloc(env, &env->t_arB, (size_t)Np * Np));
-    A(dev_alloc(env, &env->t_arW, (size_t)(c.num_stencil + Np) * Np));
-    A(dev_alloc(env, &env->t_arW_rev, (size_t)(c.num_stencil + Np) * Np));
+    A(env->t_stencil.alloc(env, (size_t)c.num_stencil));
+    A(env->t_arA.alloc(env, (size_t)Np * c.num_stencil));
+    A(env->t_arB.alloc(env, (size_t)Np * Np));
+    A(env->t_arW.alloc(env, (size_t)(c.num_stencil + Np) * Np));
+    A(env->t_arW_rev.alloc(env, (size_t)(c.num_stencil + Np) * Np));
   }
   if (c.num_screen_fine > 0) {
     const size_t N2 = c.num_screen_fine;
-    A(dev_alloc(env, &env->t_scrC1, P));
-    A(dev_alloc(env, &env->t_scrW1, P));
-    A(dev_alloc(env, &env->t_scrW1T, P));
-    A(dev_alloc(env, &env->t_scrC2, N2 * N2));
-    A(dev_alloc(env, &env->t_scrW2, (size_t)Np * N2));
-    A(dev_alloc(env, &env->t_scrW2T, (size_t)Np * N2));
+    A(env->t_scrC1.alloc(env, P));
+    A(env->t_scrW1.alloc(env, P));
+    A(env->t_scrW1T.alloc(env, P));
+    A(env->t_scrC2.alloc(env, N2 * N2));
+    A(env->t_scrW2.alloc(env, (size_t)Np * N2));
+    A(env->t_scrW2T.alloc(env, (size_t)Np * N2));
   }
-  A(dev_alloc(env, &env->screens, B * P));
+  A(env->screens.alloc(env, B * P));
   AOG_CUDA(cudaMemset(env->screens, 0, B * P * sizeof(double)));
-  A(dev_alloc(env, &env->act, B * K));
+  A(env->act.alloc(env, B * K));
   AOG_CUDA(cudaMemset(env->act, 0, B * K * sizeof(double)));
-  A(dev_alloc(env, (double**)&env->act_in, B * K));
+  A(env->act_in.alloc(env, B * K));
   // every env starts at the configured strength (aog_set_turbulence changes it per env)
   env->sqrt_cn2_host.assign(B, c.sqrt_cn2);
-  A(dev_alloc(env, &env->sqrt_cn2, 2 * B));
+  A(env->sqrt_cn2.alloc(env, 2 * B));
   AOG_CUDA(cudaMemcpy(env->sqrt_cn2, env->sqrt_cn2_host.data(), B * sizeof(double), cudaMemcpyHostToDevice));
   env->chunk = (int)std::min<size_t>(B, 4096);
   env->strehl_blocks = cdiv(env->P, 128);
   const size_t ch = env->chunk;
   if (c.precision == AOG_PRECISION_F64 || c.num_screen_fine > 0) {
-    A(dev_alloc(env, &env->bufA, ch * P));
-    A(dev_alloc(env, &env->bufB, ch * (size_t)Np * std::max(Nf, Np)));
-    A(dev_alloc(env, &env->bufC, ch * std::max<size_t>(env->NF2, P)));
+    A(env->bufA.alloc(env, ch * P));
+    A(env->bufB.alloc(env, ch * (size_t)Np * std::max(Nf, Np)));
+    A(env->bufC.alloc(env, ch * std::max<size_t>(env->NF2, P)));
   }
-  A(dev_alloc(env, &env->bufR, ch * (size_t)Np * n));
-  A(dev_alloc(env, &env->coef, ch * (size_t)J));
-  A(dev_alloc(env, &env->strehl_part, ch * (size_t)env->strehl_blocks));
+  A(env->bufR.alloc(env, ch * (size_t)Np * n));
+  A(env->coef.alloc(env, ch * (size_t)J));
+  A(env->strehl_part.alloc(env, ch * (size_t)env->strehl_blocks));
   if (c.num_stencil > 0) {
-    A(dev_alloc(env, &env->arZ, ch * (size_t)(c.num_stencil + Np)));
+    A(env->arZ.alloc(env, ch * (size_t)(c.num_stencil + Np)));
   }
   A(alloc_host_outputs(env));
   if (c.precision != AOG_PRECISION_F64) A(aog_tensor_create(env));
 #undef A
-  AOG_CUDA(cudaStreamCreate(&env->own_stream));   // blocking: ordered with the default stream
+  AOG_CUDA(cuda_create(env->own_stream, cudaStreamCreate));   // blocking: ordered with the default stream
   {
     // highest priority: its (few, compute-bound) blocks are placed as soon as an SM has room, next to the HBM-bound
     // blocks of the kernels they overlap with
     int lo = 0, hi = 0;
     AOG_CUDA(cudaDeviceGetStreamPriorityRange(&lo, &hi));
-    AOG_CUDA(cudaStreamCreateWithPriority(&env->side_stream, cudaStreamNonBlocking, hi));
+    AOG_CUDA(cuda_create(env->side_stream, cudaStreamCreateWithPriority, cudaStreamNonBlocking, hi));
   }
-  AOG_CUDA(cudaEventCreateWithFlags(&env->ev_sh_phase, cudaEventDisableTiming));
-  AOG_CUDA(cudaEventCreateWithFlags(&env->ev_ext_done, cudaEventDisableTiming));
-  AOG_CUDA(cudaEventCreate(&env->ev0));
-  AOG_CUDA(cudaEventCreate(&env->ev1));
-  AOG_CUDA(cudaEventCreate(&env->evf));
-  AOG_CUDA(cudaEventCreate(&env->evm));
-  for (auto& e : env->tev) AOG_CUDA(cudaEventCreate(&e));
+  AOG_CUDA(cuda_create(env->ev_sh_phase, cudaEventCreateWithFlags, cudaEventDisableTiming));
+  AOG_CUDA(cuda_create(env->ev_ext_done, cudaEventCreateWithFlags, cudaEventDisableTiming));
+  for (EventPtr* ev : {&env->ev0, &env->ev1, &env->evf, &env->evm}) AOG_CUDA(cuda_create(*ev, cudaEventCreateWithFlags, cudaEventDefault));
+  for (EventPtr& ev : env->tev) AOG_CUDA(cuda_create(ev, cudaEventCreateWithFlags, cudaEventDefault));
   return AOG_OK;
 }
 
@@ -395,32 +382,6 @@ void aog_destroy(aog_env* env) {
   if (!env) return;
   DeviceGuard guard(env->cfg.device);
   cudaDeviceSynchronize();
-  aog_tensor_destroy(env);
-  void* ptrs[] = {env->t_aperture, env->t_modes, env->t_gram, env->t_m1f, env->t_m2f, env->t_m1o, env->t_m2o,
-                  env->t_lpw, env->t_lpphase, env->t_lpgram, env->t_stencil, env->t_stencil_perm, env->t_arA, env->t_arB, env->t_arW,
-                  env->t_arW_rev, env->t_ar_tail, env->arNZ, env->t_scr_sh, env->t_scr_tw, env->t_scrC1, env->t_scrW1, env->t_scrW1T, env->t_scrC2, env->t_scrW2, env->t_scrW2T,
-                  env->screens, env->act, env->sqrt_cn2, env->bufA, env->bufB, env->bufC, env->bufR, env->coef,
-                  env->strehl_part, env->arZ, env->act_in, env->noise_in, env->o_pack,
-                  env->t_sh_mla, env->t_sh_C, env->t_sh_CT,
-                  env->t_sh_off, env->t_sh_pix, env->t_sh_px, env->t_sh_py, env->t_sh_offset, env->t_sh_recon,
-                  env->t_sh_act0, env->act_sh, env->o_action, env->sh_noisy_in, env->t_sh_Cf[0], env->t_sh_Cf[1],
-                  env->t_sh_Cf[2], env->t_sh_Cf[3], env->t_scrWst[0], env->t_scrWst[1], env->t_scrWrT[0], env->t_scrWrT[1],
-                  env->t_scrWiT[0], env->t_scrWiT[1]};
-  for (void* p : ptrs)
-    if (p) cudaFree(p);
-  if (env->h_pinned) cudaFreeHost(env->h_pinned);
-  if (env->h_act) cudaFreeHost(env->h_act);
-  if (env->step_graph) cudaGraphExecDestroy(env->step_graph);
-  if (env->own_stream) cudaStreamDestroy(env->own_stream);
-  if (env->side_stream) cudaStreamDestroy(env->side_stream);
-  if (env->ev_sh_phase) cudaEventDestroy(env->ev_sh_phase);
-  if (env->ev_ext_done) cudaEventDestroy(env->ev_ext_done);
-  if (env->ev0) cudaEventDestroy(env->ev0);
-  if (env->ev1) cudaEventDestroy(env->ev1);
-  if (env->evf) cudaEventDestroy(env->evf);
-  if (env->evm) cudaEventDestroy(env->evm);
-  for (auto& e : env->tev)
-    if (e) cudaEventDestroy(e);
   delete env;
 }
 
@@ -477,7 +438,7 @@ int aog_set_table(aog_env* env, int which, const void* host, size_t count) {
       return ka < kb;
     });
     for (size_t j = 0; j < Ns; ++j) sorted[j] = st[perm[j]];
-    int rc = dev_alloc(env, &env->t_stencil_perm, Ns);
+    int rc = env->t_stencil_perm.alloc(env, Ns);
     if (rc) return rc;
     AOG_CUDA(cudaMemcpy(env->t_stencil_perm, perm.data(), Ns * sizeof(int), cudaMemcpyHostToDevice));
     AOG_CUDA(cudaMemcpy(dst, sorted.data(), Ns * sizeof(int), cudaMemcpyHostToDevice));
@@ -492,7 +453,7 @@ int aog_set_table(aog_env* env, int which, const void* host, size_t count) {
     }
     env->ar_direct = direct;
     if (direct) {
-      rc = dev_alloc(env, &env->t_ar_tail, tail.size());
+      rc = env->t_ar_tail.alloc(env, tail.size());
       if (rc) return rc;
       AOG_CUDA(cudaMemcpy(env->t_ar_tail, tail.data(), tail.size() * sizeof(int), cudaMemcpyHostToDevice));
     }
@@ -500,7 +461,7 @@ int aog_set_table(aog_env* env, int which, const void* host, size_t count) {
     AOG_CUDA(cudaMemcpy(dst, host, want * esz, cudaMemcpyHostToDevice));
   }
   env->have[which] = true;
-  if (env->step_graph) { cudaGraphExecDestroy(env->step_graph); env->step_graph = nullptr; }   // captured launches hold table-derived arguments
+  env->step_graph.reset();   // captured launches hold table-derived arguments
   if ((which == AOG_TABLE_AR_A || which == AOG_TABLE_AR_B || which == AOG_TABLE_AR_STENCIL) && env->have[AOG_TABLE_AR_A] &&
       env->have[AOG_TABLE_AR_B] && env->have[AOG_TABLE_AR_STENCIL]) {
     const int tot = (int)((Ns + Np) * Np);
@@ -534,8 +495,8 @@ int aog_set_table(aog_env* env, int which, const void* host, size_t count) {
     env->scr_fft = fft && res <= 1e-11;
     if (env->scr_fft) {
       int rc;
-      if ((rc = dev_alloc(env, &env->t_scr_sh, N))) return rc;
-      if ((rc = dev_alloc(env, &env->t_scr_tw, (size_t)240))) return rc;
+      if ((rc = env->t_scr_sh.alloc(env, N))) return rc;
+      if ((rc = env->t_scr_tw.alloc(env, (size_t)240))) return rc;
       AOG_CUDA(cudaMemcpy(env->t_scr_sh, m, N * sizeof(double2), cudaMemcpyHostToDevice));       // row x = 0
       AOG_CUDA(cudaMemcpy(env->t_scr_tw, tw.data(), 240 * sizeof(double2), cudaMemcpyHostToDevice));
     }
@@ -565,9 +526,9 @@ int aog_set_table(aog_env* env, int which, const void* host, size_t count) {
           wiT[k * Nh + x] = im;
         }
       int rc;
-      if ((rc = dev_alloc(env, &env->t_scrWst[sidx], N * Nk))) return rc;
-      if ((rc = dev_alloc(env, &env->t_scrWrT[sidx], Nk * Nh))) return rc;
-      if ((rc = dev_alloc(env, &env->t_scrWiT[sidx], Nk * Nh))) return rc;
+      if ((rc = env->t_scrWst[sidx].alloc(env, N * Nk))) return rc;
+      if ((rc = env->t_scrWrT[sidx].alloc(env, Nk * Nh))) return rc;
+      if ((rc = env->t_scrWiT[sidx].alloc(env, Nk * Nh))) return rc;
       AOG_CUDA(cudaMemcpy(env->t_scrWst[sidx], wst.data(), wst.size() * sizeof(double), cudaMemcpyHostToDevice));
       AOG_CUDA(cudaMemcpy(env->t_scrWrT[sidx], wrT.data(), wrT.size() * sizeof(double), cudaMemcpyHostToDevice));
       AOG_CUDA(cudaMemcpy(env->t_scrWiT[sidx], wiT.data(), wiT.size() * sizeof(double), cudaMemcpyHostToDevice));
@@ -603,7 +564,7 @@ int aog_set_table(aog_env* env, int which, const void* host, size_t count) {
           }
         }
       for (int k = 0; k < 4; ++k) {
-        int rc = dev_alloc(env, &env->t_sh_Cf[k], Nh * Nh);
+        int rc = env->t_sh_Cf[k].alloc(env, Nh * Nh);
         if (rc) return rc;
         AOG_CUDA(cudaMemcpy(env->t_sh_Cf[k], &t[(size_t)k * 2 * Nh * Nh], Nh * Nh * sizeof(double2), cudaMemcpyHostToDevice));
       }
@@ -638,11 +599,11 @@ int aog_set_screens(aog_env* env, const void* src, int dtype, int src_on_device,
     // the caller's screens are [y][x] (hcipy Field order); the device keeps them column-major
     const size_t esz = dtype == AOG_DTYPE_F64 ? sizeof(double) : sizeof(float);
     const void* s = src;
-    void* tmp = nullptr;
+    DevArray<char> tmp;
     if (!src_on_device) {
-      AOG_CUDA(cudaMalloc(&tmp, nel * esz));
+      if (int rc = tmp.alloc(env, nel * esz)) return rc;
       cudaError_t e = cudaMemcpy(tmp, src, nel * esz, cudaMemcpyHostToDevice);
-      if (e != cudaSuccess) { cudaFree(tmp); env->err = cudaGetErrorString(e); return AOG_ERR_CUDA; }
+      if (e != cudaSuccess) { env->err = cudaGetErrorString(e); return AOG_ERR_CUDA; }
       s = tmp;
     }
     const unsigned grid = (unsigned)((nel + 255) / 256);
@@ -650,7 +611,6 @@ int aog_set_screens(aog_env* env, const void* src, int dtype, int src_on_device,
     else k_screens_in<float><<<grid, 256>>>((const float*)s, dst, c.num_pupil_pixels, nel);
     env->launches++;
     cudaError_t e = cudaDeviceSynchronize();
-    if (tmp) cudaFree(tmp);
     if (e != cudaSuccess) { env->err = cudaGetErrorString(e); return AOG_ERR_CUDA; }
   }
   if (c.precision != AOG_PRECISION_F64) return aog_tensor_screens_updated(env);
@@ -697,9 +657,9 @@ int aog_generate_screens(aog_env* env, void* stream) {
   auto synth_real = [&](int sidx, int Nk, const double* Ctab, unsigned long long draw_base, int e0, int nB,
                         int accumulate) -> int {
     const int Nh = Np / 2, Q = Nh * Nh;
-    double* X = reinterpret_cast<double*>(env->bufA);
-    double* O = reinterpret_cast<double*>(env->bufB);
-    double* Pq = reinterpret_cast<double*>(env->bufC);
+    double* X = reinterpret_cast<double*>(env->bufA.get());
+    double* O = reinterpret_cast<double*>(env->bufB.get());
+    double* Pq = reinterpret_cast<double*>(env->bufC.get());
     const long long sX = 2LL * P, sO = 2 * sB, sP = 2 * sC;
     { int rc = dmma_configure(env); if (rc) return rc; }
     if (sidx == 0 && fft_form) {
@@ -833,11 +793,11 @@ int aog_reset(aog_env* env, const aog_outputs* out_dev, void* stream) {
 int aog_reset_host(aog_env* env, const aog_outputs* out_host) {
   if (!env) return AOG_ERR_INVALID;
   aog_outputs d = device_outputs(env);
-  int rc = aog_reset(env, &d, env->own_stream);
+  int rc = aog_reset(env, &d, env->own_stream.get());
   if (rc) return rc;
   aog_outputs h{};
   if (out_host) { h.obs_f16 = out_host->obs_f16; h.obs_f64 = out_host->obs_f64; }
-  return copy_outputs_to_host(env, &h, env->own_stream);
+  return copy_outputs_to_host(env, &h, env->own_stream.get());
 }
 
 int aog_step(aog_env* env, const void* actions_dev, int act_dtype, const double* noise_dev,
@@ -868,24 +828,24 @@ int aog_step(aog_env* env, const void* actions_dev, int act_dtype, const double*
   const int64_t old_t = env->cnt.timestep;
   env->cnt.timestep += 1;
   env->cnt.timestep_render += 1;
-  if (env->timing) AOG_CUDA(cudaEventRecord(env->tev[0], st));
+  if (env->timing) AOG_CUDA(cudaEventRecord(env->tev[0].get(), st));
   const int64_t ext_before = env->cnt.extrusions;
   int rc;
   if (env->sh_phase_pending && env->sh_phase_stream == st && c.velocity != 0.0 && !env->timing) {
     // SH_step's phase kernel was the last reader of the screens: extrude on the side stream, under SH_step's
     // remaining kernels (which are still running or queued on `st`), and join before the optics
-    AOG_CUDA(cudaStreamWaitEvent(env->side_stream, env->ev_sh_phase, 0));
-    rc = evolve_to(env, env->cnt.timestep, old_t, noise_dev, env->side_stream);
+    AOG_CUDA(cudaStreamWaitEvent(env->side_stream.get(), env->ev_sh_phase.get(), 0));
+    rc = evolve_to(env, env->cnt.timestep, old_t, noise_dev, env->side_stream.get());
     if (rc) return rc;
-    AOG_CUDA(cudaEventRecord(env->ev_ext_done, env->side_stream));
-    AOG_CUDA(cudaStreamWaitEvent(st, env->ev_ext_done, 0));
+    AOG_CUDA(cudaEventRecord(env->ev_ext_done.get(), env->side_stream.get()));
+    AOG_CUDA(cudaStreamWaitEvent(st, env->ev_ext_done.get(), 0));
   } else {
     rc = evolve_to(env, env->cnt.timestep, old_t, noise_dev, st);
     if (rc) return rc;
   }
   env->sh_phase_pending = false;
   if (env->timing) {
-    AOG_CUDA(cudaEventRecord(env->tev[1], st));
+    AOG_CUDA(cudaEventRecord(env->tev[1].get(), st));
     env->last_extrusions = (int)(env->cnt.extrusions - ext_before);
     env->tev_ext_valid = true;
   }
@@ -906,7 +866,7 @@ int aog_step_host(aog_env* env, const void* actions_host, int act_dtype, const d
   if (!env || !actions_host) return AOG_ERR_INVALID;
   const aog_config& c = env->cfg;
   AOG_DEVICE(c.device);
-  cudaStream_t st = env->own_stream;
+  cudaStream_t st = env->own_stream.get();
   if (act_dtype != AOG_DTYPE_F32 && act_dtype != AOG_DTYPE_F64) AOG_FAIL(AOG_ERR_INVALID, "act_dtype");
   const size_t esz = act_dtype == AOG_DTYPE_F32 ? sizeof(float) : sizeof(double);
   const size_t abytes = (size_t)c.num_envs * c.num_modes * esz;
@@ -916,7 +876,7 @@ int aog_step_host(aog_env* env, const void* actions_host, int act_dtype, const d
   if (c.num_envs <= 256 && c.precision != AOG_PRECISION_F64 && c.velocity == 0.0 && !noise_host && !env->timing &&
       !env->graph_failed && !no_graph && tables_ready(env)) {
     int rc;
-    if (!env->h_act) AOG_CUDA(cudaMallocHost(&env->h_act, (size_t)c.num_envs * c.num_modes * sizeof(double)));
+    if (!env->h_act && (rc = env->h_act.alloc(env, (size_t)c.num_envs * c.num_modes))) return rc;
     if ((rc = ensure_pinned(env, env->o_pack_bytes))) return rc;
     std::memcpy(env->h_act, actions_host, abytes);
     aog_outputs d = device_outputs(env);
@@ -927,10 +887,10 @@ int aog_step_host(aog_env* env, const void* actions_host, int act_dtype, const d
       int done = 0;
       if (env->cnt.timestep_render == c.max_steps) { done = 1; env->cnt.episode_no += 1; }
       if (done_out) *done_out = done;
-      AOG_CUDA(cudaGraphLaunch(env->step_graph, st));
+      AOG_CUDA(cudaGraphLaunch(env->step_graph.get(), st));
       env->launches += env->graph_launches;
     } else if (env->graph_warm >= 1) {
-      if (env->step_graph) { cudaGraphExecDestroy(env->step_graph); env->step_graph = nullptr; }
+      env->step_graph.reset();
       cudaGraph_t graph = nullptr;
       const int64_t l0 = env->launches;
       AOG_CUDA(cudaStreamBeginCapture(st, cudaStreamCaptureModeThreadLocal));
@@ -939,10 +899,9 @@ int aog_step_host(aog_env* env, const void* actions_host, int act_dtype, const d
       if (rc == AOG_OK) e = cudaMemcpyAsync(env->h_pinned, env->o_pack, env->o_pack_bytes, cudaMemcpyDeviceToHost, st);
       const cudaError_t e2 = cudaStreamEndCapture(st, &graph);
       if (rc != AOG_OK || e != cudaSuccess || e2 != cudaSuccess || !graph ||
-          cudaGraphInstantiate(&env->step_graph, graph, 0) != cudaSuccess) {
+          cuda_create(env->step_graph, cudaGraphInstantiateWithFlags, graph, 0ull) != cudaSuccess) {
         if (graph) cudaGraphDestroy(graph);
         cudaGetLastError();
-        env->step_graph = nullptr;
         env->graph_failed = true;                      // this handle keeps to plain launches
         if (rc != AOG_OK) return rc;                   // (aog_step's own error; its bookkeeping has not been undone)
         AOG_FAIL(AOG_ERR_CUDA, "CUDA graph capture of the step failed");
@@ -950,7 +909,7 @@ int aog_step_host(aog_env* env, const void* actions_host, int act_dtype, const d
       cudaGraphDestroy(graph);
       env->graph_dtype = act_dtype;
       env->graph_launches = (int)(env->launches - l0);
-      AOG_CUDA(cudaGraphLaunch(env->step_graph, st));  // the capture recorded the work, this runs it
+      AOG_CUDA(cudaGraphLaunch(env->step_graph.get(), st));  // the capture recorded the work, this runs it
     } else {
       env->graph_warm++;                               // first call: plain launches (function attributes, lazy set-up)
       AOG_CUDA(cudaMemcpyAsync(env->act_in, env->h_act, abytes, cudaMemcpyHostToDevice, st));
@@ -968,7 +927,7 @@ int aog_step_host(aog_env* env, const void* actions_host, int act_dtype, const d
     const size_t cnt = (size_t)c.num_envs * n_ext * c.num_pupil_pixels;
     if (cnt > 0) {
       if (cnt > env->noise_in_cap) {
-        int rc = dev_alloc(env, &env->noise_in, cnt);
+        int rc = env->noise_in.alloc(env, cnt);
         if (rc) return rc;
         env->noise_in_cap = cnt;
       }
@@ -994,18 +953,18 @@ int aog_sh_configure(aog_env* env, int num_sub, int num_pix, double amplitude, d
   env->sh_weight_dt = weight_dt;
   int rc;
 #define A(expr) if ((rc = (expr))) return rc
-  A(dev_alloc(env, &env->t_sh_mla, P));
-  A(dev_alloc(env, &env->t_sh_C, P));
-  A(dev_alloc(env, &env->t_sh_CT, P));
-  A(dev_alloc(env, &env->t_sh_off, (size_t)num_sub + 1));
-  A(dev_alloc(env, &env->t_sh_pix, (size_t)num_pix));
-  A(dev_alloc(env, &env->t_sh_px, (size_t)num_pix));
-  A(dev_alloc(env, &env->t_sh_py, (size_t)num_pix));
-  A(dev_alloc(env, &env->t_sh_offset, 2 * (size_t)num_sub));
-  A(dev_alloc(env, &env->t_sh_recon, K * 2 * (size_t)num_sub));
-  A(dev_alloc(env, &env->t_sh_act0, K));
-  A(dev_alloc(env, &env->act_sh, B * K));
-  A(dev_alloc(env, &env->o_action, B * K));
+  A(env->t_sh_mla.alloc(env, P));
+  A(env->t_sh_C.alloc(env, P));
+  A(env->t_sh_CT.alloc(env, P));
+  A(env->t_sh_off.alloc(env, (size_t)num_sub + 1));
+  A(env->t_sh_pix.alloc(env, (size_t)num_pix));
+  A(env->t_sh_px.alloc(env, (size_t)num_pix));
+  A(env->t_sh_py.alloc(env, (size_t)num_pix));
+  A(env->t_sh_offset.alloc(env, 2 * (size_t)num_sub));
+  A(env->t_sh_recon.alloc(env, K * 2 * (size_t)num_sub));
+  A(env->t_sh_act0.alloc(env, K));
+  A(env->act_sh.alloc(env, B * K));
+  A(env->o_action.alloc(env, B * K));
 #undef A
   AOG_CUDA(cudaMemset(env->act_sh, 0, B * K * sizeof(double)));
   for (int t = AOG_TABLE_SH_MLA_PHASE; t <= AOG_TABLE_SH_ACT0; ++t) env->have[t] = false;
@@ -1093,13 +1052,13 @@ int aog_sh_step_host(aog_env* env, int noise_mode, const double* noisy_image_hos
   if (!env || !action_out_host) return AOG_ERR_INVALID;
   const aog_config& c = env->cfg;
   AOG_DEVICE(c.device);
-  cudaStream_t st = env->own_stream;
+  cudaStream_t st = env->own_stream.get();
   const size_t B = c.num_envs, K = c.num_modes, P = env->P;
   if (!env->o_action) AOG_FAIL(AOG_ERR_STATE, "aog_sh_configure not called");
   const double* noisy = nullptr;
   if (noise_mode == AOG_SH_NOISE_INJECTED) {
     if (!noisy_image_host) AOG_FAIL(AOG_ERR_INVALID, "noisy image missing");
-    if (!env->sh_noisy_in) { int rc = dev_alloc(env, &env->sh_noisy_in, B * P); if (rc) return rc; }
+    if (!env->sh_noisy_in) { int rc = env->sh_noisy_in.alloc(env, B * P); if (rc) return rc; }
     AOG_CUDA(cudaMemcpyAsync(env->sh_noisy_in, noisy_image_host, B * P * sizeof(double), cudaMemcpyHostToDevice, st));
     noisy = env->sh_noisy_in;
   }
@@ -1215,7 +1174,7 @@ int aog_get_field(aog_env* env, int which, int env_index, double* host_out, size
     int rc = ensure_f64_scratch(env);
     if (rc) return rc;
     const int Np = c.num_pupil_pixels, K = c.num_modes;
-    cudaStream_t st = env->own_stream;
+    cudaStream_t st = env->own_stream.get();
     k_sh_field_f64<1><<<dim3(cdiv((int)P, 128), 1), 128, K * sizeof(double), st>>>(
         env->screens, env->act_sh, env->t_modes, env->t_aperture, env->t_sh_mla, env->bufA, (int)P, Np, K, env_index,
         1, (int)env->cnt.column_origin, c.wavelength_wfs, env->sh_amplitude);
@@ -1243,10 +1202,10 @@ int aog_get_field(aog_env* env, int which, int env_index, double* host_out, size
   none.obs_f64 = d.obs_f64;   // optics_chunk_f64 applies the env offset itself
   const bool timing = env->timing;
   env->timing = false;
-  int rc = optics_chunk_f64(env, env_index, 1, false, false, none, env->own_stream);
+  int rc = optics_chunk_f64(env, env_index, 1, false, false, none, env->own_stream.get());
   env->timing = timing;
   if (rc) return rc;
-  AOG_CUDA(cudaStreamSynchronize(env->own_stream));
+  AOG_CUDA(cudaStreamSynchronize(env->own_stream.get()));
   if (which == AOG_FIELD_PUPIL) {
     if (count != 2 * P) AOG_FAIL(AOG_ERR_INVALID, "count");
     AOG_CUDA(cudaMemcpy(host_out, env->bufA, count * sizeof(double), cudaMemcpyDeviceToHost));
@@ -1282,11 +1241,10 @@ int aog_debug_poisson(int device, double lambda, int n, uint64_t seed, double* h
   if (!host_out || n < 1 || !(lambda >= 0.0)) return AOG_ERR_INVALID;
   DeviceGuard guard(device);
   if (guard.err != cudaSuccess) return AOG_ERR_CUDA;
-  double* d = nullptr;
-  if (cudaMalloc((void**)&d, (size_t)n * sizeof(double)) != cudaSuccess) return AOG_ERR_CUDA;
+  DevArray<double> d;
+  if (d.alloc(n) != cudaSuccess) return AOG_ERR_CUDA;
   k_debug_poisson<<<cdiv(n, 256), 256>>>(lambda, n, (unsigned long long)seed, d);
   const cudaError_t e = cudaMemcpy(host_out, d, (size_t)n * sizeof(double), cudaMemcpyDeviceToHost);
-  cudaFree(d);
   return e == cudaSuccess ? AOG_OK : AOG_ERR_CUDA;
 }
 
@@ -1317,11 +1275,11 @@ int aog_set_timing(aog_env* env, int enabled) {
 int aog_last_kernel_ms(aog_env* env, double* field_ms, double* stage1_ms, double* stage2_ms) {
   if (!env) return AOG_ERR_INVALID;
   if (!env->ev_valid || env->cfg.precision == AOG_PRECISION_F64) AOG_FAIL(AOG_ERR_STATE, "no timed tensor-path step yet");
-  AOG_CUDA(cudaEventSynchronize(env->ev1));
+  AOG_CUDA(cudaEventSynchronize(env->ev1.get()));
   float a = 0.f, b = 0.f, c = 0.f;
-  AOG_CUDA(cudaEventElapsedTime(&a, env->evf, env->ev0));
-  AOG_CUDA(cudaEventElapsedTime(&b, env->ev0, env->evm));
-  AOG_CUDA(cudaEventElapsedTime(&c, env->evm, env->ev1));
+  AOG_CUDA(cudaEventElapsedTime(&a, env->evf.get(), env->ev0.get()));
+  AOG_CUDA(cudaEventElapsedTime(&b, env->ev0.get(), env->evm.get()));
+  AOG_CUDA(cudaEventElapsedTime(&c, env->evm.get(), env->ev1.get()));
   if (field_ms) *field_ms = a;
   if (stage1_ms) *stage1_ms = b;
   if (stage2_ms) *stage2_ms = c;
@@ -1333,15 +1291,15 @@ int aog_last_timings(aog_env* env, double* out_ms, int n) {
   for (int i = 0; i < n; ++i) out_ms[i] = -1.0;
   float ms = 0.f;
   if (env->tev_ext_valid) {
-    AOG_CUDA(cudaEventSynchronize(env->tev[1]));
-    AOG_CUDA(cudaEventElapsedTime(&ms, env->tev[0], env->tev[1]));
+    AOG_CUDA(cudaEventSynchronize(env->tev[1].get()));
+    AOG_CUDA(cudaEventElapsedTime(&ms, env->tev[0].get(), env->tev[1].get()));
     out_ms[0] = ms;
     out_ms[1] = (double)env->last_extrusions;
   }
   if (env->tev_sh_valid) {
-    AOG_CUDA(cudaEventSynchronize(env->tev[7]));
+    AOG_CUDA(cudaEventSynchronize(env->tev[7].get()));
     for (int k = 0; k < 5; ++k) {
-      AOG_CUDA(cudaEventElapsedTime(&ms, env->tev[2 + k], env->tev[3 + k]));
+      AOG_CUDA(cudaEventElapsedTime(&ms, env->tev[2 + k].get(), env->tev[3 + k].get()));
       out_ms[2 + k] = ms;
     }
   }
@@ -1350,9 +1308,9 @@ int aog_last_timings(aog_env* env, double* out_ms, int n) {
 
 double aog_last_mft_ms(aog_env* env) {
   if (!env || !env->ev_valid) return -1.0;
-  if (cudaEventSynchronize(env->ev1) != cudaSuccess) return -1.0;
+  if (cudaEventSynchronize(env->ev1.get()) != cudaSuccess) return -1.0;
   float ms = 0.f;
-  if (cudaEventElapsedTime(&ms, env->ev0, env->ev1) != cudaSuccess) return -1.0;
+  if (cudaEventElapsedTime(&ms, env->ev0.get(), env->ev1.get()) != cudaSuccess) return -1.0;
   return (double)ms;
 }
 

@@ -3,6 +3,8 @@
 #pragma once
 #include "fft240.cuh"
 #include "common.cuh"
+#include "finalize.cuh"
+#include "philox.cuh"
 #include <curand_kernel.h>
 
 // --------------------------------------------------------------------------------------
@@ -235,48 +237,9 @@ static __global__ void k_obs_rows_f64(const double2* __restrict__ E, const doubl
 // --------------------------------------------------------------------------------------
 // Per-env epilogue: obs power (second contraction + |.|^2 w), fibre power, Strehl, SSIM,
 // reward, threshold (AO_env.py:142-153, 468-503).  k_finalize (FP64 path, block per env) reads R and coef;
-// k_finalize_tcw (tensor / fused paths, warp per env) reads R4 and the partial sums and actuators described below.
+// k_finalize_tcw (tensor / fused paths, warp per env, tensor_path.cu) reads R4 and the partial sums and actuators
+// described in finalize.cuh.
 // --------------------------------------------------------------------------------------
-struct FinalizeArgs {
-  const double2* R; const float2* R4; const double2* m1o; const double2* coef; const double* coef4; const double2* lpphase; const double* lpgram;
-  const double2* strehl_part; int strehl_blocks;
-  int Np, n, J, rew_type, has_thr, compute_reward;
-  int coef_is_raw;     // 2: coef4 holds [re|im][2 partials]; 3: fib_part holds [fib_slots][fib_stride] partial sums
-                       // per env;  both x coef_scale
-  const double2* fib_part; int fib_slots, fib_stride;
-  // the phase kernel's CTA c takes work items [c slot_ipc, (c + 1) slot_ipc) and the 128-env block eb owns items
-  // [eb slot_items, (eb + 1) slot_items), so only slots 0 .. last - first of an env are written (and summed): no
-  // clearing pass
-  int slot_ipc, slot_items;
-  // the env's normalised actuators [K].  An all-zero action makes them 0/0 = NaN (AO_env.py:119-120) and the
-  // reference then returns NaN observations, reward and power; the fixed-point phase arithmetic of the tensor / fused
-  // kernels would swallow the NaN, so it is re-applied here.
-  const double* act; int K;
-  double2 coef_scale;
-  double thr, obs_weight, strehl_scale, ssim_peak;
-  double2 norm;
-  uint16_t* obs16; double* obs64; double* reward; double* power; double* strehl; double* ssim;
-};
-
-__device__ __forceinline__ double ssim_1d(const double* x, int len, int ref_idx, double peak) {
-  // skimage.metrics.structural_similarity 0.22 on 1-D data against peak * onehot(ref_idx):
-  // win 7, uniform filter, sample covariance, K1 = .01, K2 = .03, crop 3, mean.
-  const double C1 = (0.01 * peak) * (0.01 * peak), C2 = (0.03 * peak) * (0.03 * peak);
-  const double cov_norm = 7.0 / 6.0;
-  double tot = 0.0;
-  for (int c = 3; c < len - 3; ++c) {
-    double sx = 0, sxx = 0, sy = 0, syy = 0, sxy = 0;
-    for (int i = c - 3; i <= c + 3; ++i) {
-      const double a = x[i], r = (i == ref_idx) ? peak : 0.0;
-      sx += a; sxx += a * a; sy += r; syy += r * r; sxy += a * r;
-    }
-    const double ux = sx / 7, uy = sy / 7, uxx = sxx / 7, uyy = syy / 7, uxy = sxy / 7;
-    const double vx = cov_norm * (uxx - ux * ux), vy = cov_norm * (uyy - uy * uy), vxy = cov_norm * (uxy - ux * uy);
-    tot += ((2 * ux * uy + C1) * (2 * vxy + C2)) / ((ux * ux + uy * uy + C1) * (vx + vy + C2));
-  }
-  return tot / (double)(len - 6);
-}
-
 static __global__ void k_finalize(FinalizeArgs a) {
   __shared__ double obs[AOG_MAX_OBS * AOG_MAX_OBS];
   const int b = blockIdx.x;
@@ -334,245 +297,11 @@ static __global__ void k_finalize(FinalizeArgs a) {
   if (a.power) a.power[b] = power;
 }
 
-// k_finalize_tcw<N, PARTS>: the epilogue of the tensor / fused paths, R4 holding PARTS partial column sums per
-// contraction index, with ONE WARP per env and no block-level barrier.  The kernel is bound by the LATENCY of fetching
-// the env's column partial sums (28.8 KB for the 5x5 detector), not by its arithmetic (DESIGN 4.6), so the partial
-// sums stream through shared memory: every warp keeps a
-// double-buffered ring of tiles (8 XS pupil columns = ~6 KB each, 16-byte cp.async, one commit group per tile) in
-// flight ahead of its arithmetic -- 16 warps per SM x 6-12 KB outstanding.
-// Lane (xs, b) = (lane / N, lane % N) owns column b of the column sums and the pupil columns x = xs, xs + XS, ...
-// (XS = 32 / N): per x it adds the PARTS partial sums of R[x][b] in FP64 and multiplies them with the N table
-// entries m[a][x] (broadcast loads), i.e. N complex accumulators per lane instead of N^2 -- no lane computes anything
-// twice.  The XS partial results per detector pixel meet in shared memory, summed in a fixed order by the lane that owns
-// the pixel.  Slot sums (fibre projections, Strehl) are loaded before the contraction and reduced after it.
-// Summation order depends on the env's data only: a batched env equals its single-env twin bit for bit.
-constexpr int FIN_WARPS = 8;
-template <int N, int PARTS> struct FinCfg {
-  static constexpr int XS = 32 / N, LANES = XS * N, N2 = N * N, N2P = N2 < 7 ? 7 : N2;
-  static constexpr int ITER = N >= 6 ? 4 : 8, TILE_X = XS * ITER, ROW = PARTS * N /* float2 per pupil column */;
-  static constexpr int TAB_MAX = N * 512 * 16;           // the [N][Np] table, Np <= 512 on the tensor / fused paths
-  static constexpr int TILE_BYTES = TILE_X * ROW * 8, WARP_BYTES = 2 * TILE_BYTES, SMEM = FIN_WARPS * WARP_BYTES;
-  static constexpr int RED_LD = 33;
-  static_assert(TILE_BYTES % 16 == 0, "tile size");
-  static_assert((2 * N * RED_LD + 2 * N2P) * 8 <= WARP_BYTES, "the reduction scratch aliases the tile ring");
-};
-template <int N, int PARTS>
-static __global__ void __launch_bounds__(FIN_WARPS * 32, 2) k_finalize_tcw(FinalizeArgs a, int num_envs) {
-  using Cfg = FinCfg<N, PARTS>;
-  constexpr int XS = Cfg::XS, LANES = Cfg::LANES, N2 = Cfg::N2, ITER = Cfg::ITER, TILE_X = Cfg::TILE_X, ROW = Cfg::ROW;
-  extern __shared__ __align__(16) unsigned char fin_smem[];
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int b = blockIdx.x * FIN_WARPS + warp;
-  unsigned char* wbase = fin_smem + warp * Cfg::WARP_BYTES;
-  double2* tab_s = reinterpret_cast<double2*>(fin_smem + FIN_WARPS * Cfg::WARP_BYTES);   // [N][Np] second obs-arm table
-  constexpr unsigned FULL = 0xffffffffu;
-  const int ntiles = (a.Np + TILE_X - 1) / TILE_X;
-  const float2* r4 = a.R4 + (size_t)b * a.Np * ROW;
-  auto issue = [&](int t, int buf) {
-    const int cols = min(TILE_X, a.Np - t * TILE_X);
-    const int nchunks = cols * ROW / 2;                                // 16-byte pieces (cols is even)
-    const unsigned char* src = reinterpret_cast<const unsigned char*>(r4 + (size_t)t * TILE_X * ROW);
-    const unsigned dst = (unsigned)__cvta_generic_to_shared(wbase + buf * Cfg::TILE_BYTES);
-    for (int c = lane; c < nchunks; c += 32)
-      asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(dst + c * 16), "l"(src + (size_t)c * 16) : "memory");
-    asm volatile("cp.async.commit_group;" ::: "memory");
-  };
-  if (b < num_envs) {
-    issue(0, 0);
-    if (ntiles > 1) issue(1, 1);
-  }
-  // the table is read N times per (pupil column, lane): from global memory those loads were the kernel's stall
-  // (L1 hit rate 39 % next to 184 KB of shared memory; ncu: long scoreboard 6 of 14 warp-cycles per issue)
-  for (int i = threadIdx.x; i < N * a.Np; i += FIN_WARPS * 32) tab_s[i] = __ldg(a.m1o + i);
-  __syncthreads();
-  if (b >= num_envs) return;                            // warps are independent from here on
-  if (a.act) {
-    int bad = 0;
-    for (int k = lane; k < a.K; k += 32) bad |= isfinite(a.act[(size_t)b * a.K + k]) ? 0 : 1;   // inf: exp(i inf) = NaN too
-    if (__any_sync(FULL, bad)) {
-      asm volatile("cp.async.wait_group 0;" ::: "memory");
-      const double qnan = __longlong_as_double(0x7ff8000000000000LL);
-      for (int t = lane; t < N2; t += 32) {
-        if (a.obs64) a.obs64[(size_t)b * N2 + t] = qnan;
-        if (a.obs16) a.obs16[(size_t)b * N2 + t] = 0x7e00;
-      }
-      if (lane == 0 && a.compute_reward) {
-        if (a.reward) a.reward[b] = qnan;
-        if (a.power) a.power[b] = qnan;
-        if (a.strehl) a.strehl[b] = qnan;
-        if (a.ssim) a.ssim[b] = qnan;
-      }
-      return;
-    }
-  }
-  // per-lane partial slot sums (reduced after the contraction)
-  double2 cj[AOG_MAX_LP];
-  double2 sp = make_double2(0.0, 0.0);
-#pragma unroll
-  for (int j = 0; j < AOG_MAX_LP; ++j) cj[j] = make_double2(0.0, 0.0);
-  if (a.compute_reward) {
-    const int eb = b >> 7;
-    const int nslots = ((eb + 1) * a.slot_items - 1) / a.slot_ipc - (eb * a.slot_items) / a.slot_ipc + 1;
-    if (a.coef_is_raw == 2) {
-      if (lane == 0) {
-#pragma unroll
-        for (int j = 0; j < AOG_MAX_LP; ++j)
-          if (j < a.J) {
-            const double* c4 = a.coef4 + ((size_t)b * a.J + j) * 4;
-            cj[j] = make_double2(c4[0] + c4[1], c4[2] + c4[3]);
-          }
-      }
-    } else {
-      const double2* fp = a.fib_part + (size_t)b * a.fib_slots * a.fib_stride;
-      for (int i = lane; i < nslots; i += 32) {
-#pragma unroll
-        for (int j = 0; j < AOG_MAX_LP; ++j)
-          if (j < a.J) { const double2 v = fp[i * a.fib_stride + j]; cj[j].x += v.x; cj[j].y += v.y; }
-      }
-    }
-    if (a.rew_type == AOG_REW_STREHL_RATIO) {
-      const double2* spp = a.strehl_part + (size_t)b * a.strehl_blocks;
-      for (int i = lane; i < nslots; i += 32) { const double2 v = spp[i]; sp.x += v.x; sp.y += v.y; }
-    }
-  }
-  // contraction over the pupil columns
-  const int xs = lane / N, bb = lane - xs * N;
-  double are[N], aim[N];
-#pragma unroll
-  for (int v = 0; v < N; ++v) are[v] = aim[v] = 0.0;
-  for (int t = 0; t < ntiles; ++t) {
-    if (t + 1 < ntiles) asm volatile("cp.async.wait_group 1;" ::: "memory");
-    else                asm volatile("cp.async.wait_group 0;" ::: "memory");
-    __syncwarp();
-    const float2* tile = reinterpret_cast<const float2*>(wbase + (t & 1) * Cfg::TILE_BYTES);
-    if (lane < LANES) {
-#pragma unroll
-      for (int i = 0; i < ITER; ++i) {
-        const int xl = xs + XS * i, x = t * TILE_X + xl;
-        if (x < a.Np) {
-          double ex = 0.0, ey = 0.0;
-#pragma unroll
-          for (int qq = 0; qq < PARTS; ++qq) {
-            const float2 t4 = tile[(xl * PARTS + qq) * N + bb];
-            ex += (double)t4.x;
-            ey += (double)t4.y;
-          }
-#pragma unroll
-          for (int v = 0; v < N; ++v) {
-            const double2 m = tab_s[v * a.Np + x];
-            are[v] = fma(m.x, ex, fma(-m.y, ey, are[v]));
-            aim[v] = fma(m.x, ey, fma(m.y, ex, aim[v]));
-          }
-        }
-      }
-    }
-    __syncwarp();
-    if (t + 2 < ntiles) issue(t + 2, t & 1);
-  }
-  double* red = reinterpret_cast<double*>(wbase);               // [2 N][RED_LD]; the tile ring is drained
-  double* obs_s = red + 2 * N * Cfg::RED_LD;
-  double* win_s = obs_s + Cfg::N2P;
-#pragma unroll
-  for (int v = 0; v < N; ++v) { red[(2 * v) * Cfg::RED_LD + lane] = are[v]; red[(2 * v + 1) * Cfg::RED_LD + lane] = aim[v]; }
-  __syncwarp();
-  for (int t = lane; t < N2; t += 32) {
-    const int v = t / N, u = t - v * N;
-    double re = 0.0, im = 0.0;
-#pragma unroll
-    for (int s = 0; s < XS; ++s) { re += red[(2 * v) * Cfg::RED_LD + s * N + u]; im += red[(2 * v + 1) * Cfg::RED_LD + s * N + u]; }
-    const double fr = re * a.norm.x - im * a.norm.y, fi = re * a.norm.y + im * a.norm.x;
-    const double pw = (fr * fr + fi * fi) * a.obs_weight;
-    const int to = u * N + v;          // R4 and the table (M2o^T) hold the transposed contraction
-    obs_s[to] = pw;
-    if (a.obs64) a.obs64[(size_t)b * N2 + to] = pw;
-    if (a.obs16) a.obs16[(size_t)b * N2 + to] = __half_as_ushort(__double2half(pw));
-  }
-  __syncwarp();
-  if (!a.compute_reward) return;
-  // fibre: out = M (c e^{i beta L});  total power = c'^H G c'
-  double2 c[AOG_MAX_LP];
-#pragma unroll
-  for (int j = 0; j < AOG_MAX_LP; ++j) {
-    if (j < a.J) {
-      double2 s = make_double2(warp_sum(cj[j].x), warp_sum(cj[j].y));
-      s = make_double2(s.x * a.coef_scale.x - s.y * a.coef_scale.y, s.x * a.coef_scale.y + s.y * a.coef_scale.x);
-      const double2 ph = a.lpphase[j];
-      c[j] = make_double2(s.x * ph.x - s.y * ph.y, s.x * ph.y + s.y * ph.x);
-    } else {
-      c[j] = make_double2(0.0, 0.0);
-    }
-  }
-  double power = 0.0;
-#pragma unroll
-  for (int j = 0; j < AOG_MAX_LP; ++j)
-#pragma unroll
-    for (int k = 0; k < AOG_MAX_LP; ++k)
-      if (j < a.J && k < a.J) power += a.lpgram[j * a.J + k] * (c[j].x * c[k].x + c[j].y * c[k].y);
-  double reward;
-  if (a.rew_type == AOG_REW_STREHL_RATIO) {
-    const double sr = warp_sum(sp.x), si = warp_sum(sp.y);
-    const double strehl = a.strehl_scale * (sr * sr + si * si);
-    if (lane == 0 && a.strehl) a.strehl[b] = strehl;
-    reward = -(100.0 - strehl);
-  } else {
-    // skimage SSIM on 1-D data (ssim_1d above), one window per lane, summed in window order
-    const double peak = a.ssim_peak, C1 = (0.01 * peak) * (0.01 * peak), C2 = (0.03 * peak) * (0.03 * peak);
-    const double cov_norm = 7.0 / 6.0;
-    constexpr int ref_idx = N2 / 2;
-    for (int cw = 3 + lane; cw < N2 - 3; cw += 32) {
-      double sx = 0, sxx = 0, sy = 0, syy = 0, sxy = 0;
-      for (int i = cw - 3; i <= cw + 3; ++i) {
-        const double x = obs_s[i], r = (i == ref_idx) ? peak : 0.0;
-        sx += x; sxx += x * x; sy += r; syy += r * r; sxy += x * r;
-      }
-      const double ux = sx / 7, uy = sy / 7, uxx = sxx / 7, uyy = syy / 7, uxy = sxy / 7;
-      const double vx = cov_norm * (uxx - ux * ux), vy = cov_norm * (uyy - uy * uy), vxy = cov_norm * (uxy - ux * uy);
-      win_s[cw] = ((2 * ux * uy + C1) * (2 * vxy + C2)) / ((ux * ux + uy * uy + C1) * (vx + vy + C2));
-    }
-    __syncwarp();
-    double tot = 0.0;
-    for (int cw = 3; cw < N2 - 3; ++cw) tot += win_s[cw];      // same summation order as ssim_1d
-    const double sv = tot / (double)(N2 - 6);
-    if (lane == 0 && a.ssim) a.ssim[b] = sv;
-    reward = 0.8 * power + (1.0 - 0.8) * sv;
-  }
-  if (lane != 0) return;
-  if (a.has_thr && reward < a.thr) reward = -1.0;
-  if (a.reward) a.reward[b] = reward;
-  if (a.power) a.power[b] = power;
-}
-
 // --------------------------------------------------------------------------------------
 // Autoregressive column extrusion (hcipy InfiniteAtmosphericLayer._extrude; AO_env.py:125).
 // gather: Z[b] = [ screen[stencil] (on the 180-degree rotated screen when moving +x) ,
 //                  sqrt(Cn2) xi ];  GEMM: new = Z . [A^T ; B^T];  scatter: ring slot.
 // --------------------------------------------------------------------------------------
-// Philox-4x32-10 (Salmon et al. 2011), one counter block per call
-__device__ __forceinline__ uint4 aog_philox4x32_10(uint4 c, uint2 k) {
-#pragma unroll
-  for (int r = 0; r < 10; ++r) {
-    const uint32_t h0 = __umulhi(0xD2511F53u, c.x), l0 = 0xD2511F53u * c.x;
-    const uint32_t h1 = __umulhi(0xCD9E8D57u, c.z), l1 = 0xCD9E8D57u * c.z;
-    c = make_uint4(h1 ^ c.y ^ k.x, l1, h0 ^ c.w ^ k.y, l0);
-    k.x += 0x9E3779B9u;
-    k.y += 0xBB67AE85u;
-  }
-  return c;
-}
-// four standard normals from one block: two Box-Muller transforms in FP32 on the SFU (24-bit uniforms in (0, 1]; over all
-// of them within 3.5e-5 of an FP64 Box-Muller on B200, |z| <= 5.9: tests/test_device_noise_gpu.py).  The draws only
-// have to be normal and reproducible from (seed, env, index) -- parity with the reference is through injected noise --
-// and curand's FP64 Box-Muller cost 58 us per step of 4096 envs at 20 m/s.
-__device__ __forceinline__ void aog_normals4(uint4 r, float (&z)[4]) {
-  const float u0 = ((float)(r.x >> 8) + 0.5f) * (1.0f / 16777216.0f), u1 = ((float)(r.y >> 8) + 0.5f) * (1.0f / 16777216.0f);
-  const float u2 = ((float)(r.z >> 8) + 0.5f) * (1.0f / 16777216.0f), u3 = ((float)(r.w >> 8) + 0.5f) * (1.0f / 16777216.0f);
-  const float ra = sqrtf(-2.f * __logf(u0)), rb = sqrtf(-2.f * __logf(u2));
-  float sn, cs;
-  __sincosf(6.28318530718f * u1, &sn, &cs);
-  z[0] = ra * cs; z[1] = ra * sn;
-  __sincosf(6.28318530718f * u3, &sn, &cs);
-  z[2] = rb * cs; z[3] = rb * sn;
-}
 // extrusion noise: normals 4 j .. 4 j + 3 of extrusion `draw` of env `env_id`
 __device__ __forceinline__ void ar_normals4(unsigned long long seed, unsigned long long env_id, unsigned long long draw,
                                             int j, float (&z)[4]) {
@@ -1375,12 +1104,4 @@ static __global__ void k_build_arW(const double* __restrict__ A, const double* _
   int js = j;
   if (reverse_cols && j < 2 * Np) js = (j / Np) * Np + (Np - 1 - j % Np);
   W[i] = (j < Ns) ? A[(size_t)y * Ns + perm[js]] : Bm[(size_t)y * Np + (j - Ns)];
-}
-
-static __global__ void k_focal_power(const double2* __restrict__ F, double* __restrict__ out, int n, double2 norm, double w) {
-  int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= n) return;
-  const double2 f = F[i];
-  const double fr = f.x * norm.x - f.y * norm.y, fi = f.x * norm.y + f.y * norm.x;
-  out[i] = (fr * fr + fi * fi) * w;
 }

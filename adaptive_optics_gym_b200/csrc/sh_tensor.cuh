@@ -646,8 +646,8 @@ int build_sh_operator(aog_env* env, TensorState* ts, int stage, const std::vecto
         row_im[kr] = im;  row_im[ki] = re;
       }
   int rc;
-  if ((rc = talloc(env, &ts->shCE_hi[stage], t.size()))) return rc;
-  if ((rc = talloc(env, &ts->shCE_lo[stage], t.size()))) return rc;
+  if ((rc = ts->shCE_hi[stage].alloc(env, t.size()))) return rc;
+  if ((rc = ts->shCE_lo[stage].alloc(env, t.size()))) return rc;
   if ((rc = upload_split(env, t, ts->shCE_hi[stage], ts->shCE_lo[stage]))) return rc;
   if ((rc = make_map(env, &ts->tmShCE_hi[stage], ts->shCE_hi[stage], 4 * SH_HP, SH_HP, SH_K, KB))) return rc;
   if ((rc = make_map(env, &ts->tmShCE_lo[stage], ts->shCE_lo[stage], 4 * SH_HP, SH_HP, SH_K, KB))) return rc;
@@ -713,8 +713,8 @@ int build_sh_tensor_tables(aog_env* env, TensorState* ts) {
     }
   }
   ts->shX0 = X0; ts->shdX = dX; ts->shY0 = Y0; ts->shdY = dY;
-  if ((rc = talloc(env, &ts->shSlot, slot.size()))) return rc;
-  if ((rc = talloc(env, &ts->shSlotC, slotc.size()))) return rc;
+  if ((rc = ts->shSlot.alloc(env, slot.size()))) return rc;
+  if ((rc = ts->shSlotC.alloc(env, slotc.size()))) return rc;
   AOG_CUDA(cudaMemcpy(ts->shSlot, slot.data(), slot.size() * sizeof(int16_t), cudaMemcpyHostToDevice));
   AOG_CUDA(cudaMemcpy(ts->shSlotC, slotc.data(), slotc.size() * sizeof(double), cudaMemcpyHostToDevice));
   ts->sh_unsupported = false;
@@ -729,14 +729,14 @@ int ensure_sh_tensor_buffers(aog_env* env, TensorState* ts) {
   const size_t rows = ch * 4 * SH_HP, nel = rows * SH_K;
   int rc;
   if (!ts->phi) {
-    if ((rc = talloc(env, &ts->phi, ch * P))) return rc;
+    if ((rc = ts->phi.alloc(env, ch * P))) return rc;
     AOG_CUDA(cudaMemset(ts->phi, 0, ch * P * sizeof(float)));
   }
-  if ((rc = talloc(env, &ts->shEB_hi, nel))) return rc;
-  if ((rc = talloc(env, &ts->shEB_lo, nel))) return rc;
-  if ((rc = talloc(env, &ts->shYB_hi, nel))) return rc;
-  if ((rc = talloc(env, &ts->shYB_lo, nel))) return rc;
-  if ((rc = talloc(env, &ts->shG, nel))) return rc;
+  if ((rc = ts->shEB_hi.alloc(env, nel))) return rc;
+  if ((rc = ts->shEB_lo.alloc(env, nel))) return rc;
+  if ((rc = ts->shYB_hi.alloc(env, nel))) return rc;
+  if ((rc = ts->shYB_lo.alloc(env, nel))) return rc;
+  if ((rc = ts->shG.alloc(env, nel))) return rc;
   // padding rows / columns of the operands are never written: they must be zero (and finite)
   AOG_CUDA(cudaMemset(ts->shEB_hi, 0, nel * sizeof(__half)));
   AOG_CUDA(cudaMemset(ts->shEB_lo, 0, nel * sizeof(__half)));
@@ -759,7 +759,7 @@ int ensure_sh_tensor_buffers(aog_env* env, TensorState* ts) {
 int sh_tensor_optics(aog_env* env, TensorState* ts, int e0, int nB, cudaStream_t st) {
   const aog_config& c = env->cfg;
   const int Np = TC_NP, K = c.num_modes;
-  if (env->timing) AOG_CUDA(cudaEventRecord(env->tev[2], st));
+  if (env->timing) AOG_CUDA(cudaEventRecord(env->tev[2].get(), st));
   {   // the SH mirror's actuators -> half-turns of DM phase per unit mode, split fp16 (the DM GEMM's A operand)
     const int rows = cdiv(nB, 128) * 128;
     k_act_pack<<<cdiv(rows * ts->kpad, 256), 256, 0, st>>>(env->act_sh, ts->act_hi, ts->act_lo, K, ts->kpad, e0, nB, rows,
@@ -782,17 +782,17 @@ int sh_tensor_optics(aog_env* env, TensorState* ts, int e0, int nB, cudaStream_t
     // nothing after this kernel reads the screens or the phase tiles: the next aog_step may extrude concurrently
     // (single-chunk handles; see aog_step)
     if (nB == c.num_envs) {
-      AOG_CUDA(cudaEventRecord(env->ev_sh_phase, st));
+      AOG_CUDA(cudaEventRecord(env->ev_sh_phase.get(), st));
       env->sh_phase_pending = true;
       env->sh_phase_stream = st;
     }
   }
-  if (env->timing) AOG_CUDA(cudaEventRecord(env->tev[3], st));
+  if (env->timing) AOG_CUDA(cudaEventRecord(env->tev[3].get(), st));
   // k_sh_fold materialises the folded field and the first product streams it by TMA (forming it on chip inside the
   // first product was measured slower: DESIGN.md 4.4)
   k_sh_fold<<<dim3(SH_NKB, nB), 128, 0, st>>>(ts->phi, ts->apmask, ts->shEB_hi, ts->shEB_lo, nB);
   AOG_LAUNCH_CHECK();
-  if (env->timing) AOG_CUDA(cudaEventRecord(env->tev[4], st));
+  if (env->timing) AOG_CUDA(cudaEventRecord(env->tev[4].get(), st));
   ShGemmParams gp{};
   gp.num_envs = nB;
   gp.G = ts->shG;
@@ -803,11 +803,11 @@ int sh_tensor_optics(aog_env* env, TensorState* ts, int e0, int nB, cudaStream_t
   k_sh_gemm<1><<<2 * clusters, SG_THREADS, SG_SMEM_BYTES, st>>>(ts->tmShCE_hi[0], ts->tmShCE_lo[0], ts->tmShEB_hi, ts->tmShEB_lo,
                                                                 ts->tmShYout_hi, ts->tmShYout_lo, gp);
   AOG_LAUNCH_CHECK();
-  if (env->timing) AOG_CUDA(cudaEventRecord(env->tev[5], st));
+  if (env->timing) AOG_CUDA(cudaEventRecord(env->tev[5].get(), st));
   k_sh_gemm<2><<<2 * clusters, SG_THREADS, SG_SMEM_BYTES, st>>>(ts->tmShCE_hi[1], ts->tmShCE_lo[1], ts->tmShYB_hi, ts->tmShYB_lo,
                                                          ts->tmShYout_hi, ts->tmShYout_lo, gp);
   AOG_LAUNCH_CHECK();
-  if (env->timing) AOG_CUDA(cudaEventRecord(env->tev[6], st));
+  if (env->timing) AOG_CUDA(cudaEventRecord(env->tev[6].get(), st));
   return AOG_OK;
 }
 
@@ -819,7 +819,7 @@ double sh_image_scale(const aog_env* env, const TensorState* ts) {
 }  // namespace
 
 int aog_tensor_sh_table(aog_env* env, int which, const void* host) {
-  TensorState* ts = TS(env);
+  TensorState* ts = env->tensor.get();
   if (!ts || env->cfg.num_pupil_pixels != TC_NP) return AOG_OK;
   const size_t P = env->P;
   const double* d = static_cast<const double*>(host);
@@ -839,7 +839,7 @@ int aog_tensor_sh_table(aog_env* env, int which, const void* host) {
 }
 
 int aog_tensor_sh_step(aog_env* env, int noise_mode, double* action_out_dev, cudaStream_t st) {
-  TensorState* ts = TS(env);
+  TensorState* ts = env->tensor.get();
   if (!ts || !ts->sh_ready || noise_mode == AOG_SH_NOISE_INJECTED) return AOG_ERR_UNSUPPORTED;
   if (!(ts->have_modes && ts->have_ap)) AOG_FAIL(AOG_ERR_STATE, "tensor path tables incomplete");
   const aog_config& c = env->cfg;
@@ -863,18 +863,18 @@ int aog_tensor_sh_step(aog_env* env, int noise_mode, double* action_out_dev, cud
     cp.draw = (unsigned long long)env->sh_draws;
     k_sh_camera_tc<<<nB, CAM_THREADS, (size_t)Nsub * (3 * sizeof(unsigned long long) + 2 * sizeof(double)), st>>>(cp);
     AOG_LAUNCH_CHECK();
-    if (env->timing) { AOG_CUDA(cudaEventRecord(env->tev[7], st)); env->tev_sh_valid = true; }
+    if (env->timing) { AOG_CUDA(cudaEventRecord(env->tev[7].get(), st)); env->tev_sh_valid = true; }
   }
   return AOG_OK;
 }
 
 int aog_tensor_sh_image(aog_env* env, int env_index, double* host_out, size_t count) {
-  TensorState* ts = TS(env);
+  TensorState* ts = env->tensor.get();
   if (!ts || !ts->sh_ready) AOG_FAIL(AOG_ERR_UNSUPPORTED, "tensor-core Shack-Hartmann path not available: " + (ts ? ts->sh_why : std::string("no tensor state")));
   if (count != (size_t)env->P) AOG_FAIL(AOG_ERR_INVALID, "count");
   int rc = ensure_sh_tensor_buffers(env, ts);
   if (rc) return rc;
-  cudaStream_t st = env->own_stream;
+  cudaStream_t st = env->own_stream.get();
   // the phase kernel works on whole 128-env blocks of the tiled screens: run the block that holds env_index
   const int e0 = env_index & ~127, nB = std::min(128, env->cfg.num_envs - e0);
   if ((rc = sh_tensor_optics(env, ts, e0, nB, st))) return rc;
@@ -905,11 +905,10 @@ int aog_tensor_sh_image(aog_env* env, int env_index, double* host_out, size_t co
 int aog_tensor_debug_poisson(int device, double lambda, int n, uint64_t seed, double* host_out) {
   DeviceGuard guard(device);
   if (guard.err != cudaSuccess) return AOG_ERR_CUDA;
-  double* d = nullptr;
-  if (cudaMalloc((void**)&d, (size_t)n * sizeof(double)) != cudaSuccess) return AOG_ERR_CUDA;
+  DevArray<double> d;
+  if (d.alloc(n) != cudaSuccess) return AOG_ERR_CUDA;
   k_debug_poisson_f32<<<cdiv(n, 256), 256>>>((float)lambda, n, (unsigned long long)seed, d);
   const cudaError_t e = cudaMemcpy(host_out, d, (size_t)n * sizeof(double), cudaMemcpyDeviceToHost);
-  cudaFree(d);
   return e == cudaSuccess ? AOG_OK : AOG_ERR_CUDA;
 }
 
@@ -918,8 +917,8 @@ int aog_tensor_debug_normals(int device, int generator, int philox, int n, const
   DeviceGuard guard(device);
   if (guard.err != cudaSuccess) return AOG_ERR_CUDA;
   const size_t nw = (size_t)n * (philox ? 6 : 4), nr = philox ? (size_t)n * 4 : 0, nz = (size_t)n * 4;
-  uint32_t* d = nullptr;                                          // [words | raw | normals]
-  if (cudaMalloc((void**)&d, (nw + nr + nz) * sizeof(uint32_t)) != cudaSuccess) return AOG_ERR_CUDA;
+  DevArray<uint32_t> d;                                           // [words | raw | normals]
+  if (d.alloc(nw + nr + nz) != cudaSuccess) return AOG_ERR_CUDA;
   float* dz = reinterpret_cast<float*>(d + nw + nr);
   cudaError_t e = cudaMemcpy(d, words_in, nw * sizeof(uint32_t), cudaMemcpyHostToDevice);
   if (e == cudaSuccess) {
@@ -927,6 +926,5 @@ int aog_tensor_debug_normals(int device, int generator, int philox, int n, const
     e = cudaMemcpy(normals_out, dz, nz * sizeof(float), cudaMemcpyDeviceToHost);
   }
   if (e == cudaSuccess && philox) e = cudaMemcpy(raw_out, d + nw, nr * sizeof(uint32_t), cudaMemcpyDeviceToHost);
-  cudaFree(d);
   return e == cudaSuccess ? AOG_OK : AOG_ERR_CUDA;
 }

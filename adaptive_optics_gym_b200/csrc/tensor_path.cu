@@ -7,7 +7,7 @@
 //                   column sums, Strehl sum, fibre-coupling coefficients as inner products with the fibre modes
 //                   propagated back to the pupil (G_j = M1^T (mode_j w) M2^T).  Nothing but partial sums leaves the SM.
 //   k_small_fused   the same optics chain with a thread per pixel for batches of at most 8 envs (one env = configs[0])
-//   k_finalize_tcw  detector powers, fibre power, Strehl, SSIM, reward: one warp per env (kernels_f64.cuh)
+//   k_finalize_tcw  detector powers, fibre power, Strehl, SSIM, reward: one warp per env
 //
 // AOG_PRECISION_TENSOR -- the fibre arm through the matrix Fourier transform, three kernels per chunk:
 //   k_dm_phase_tc   DM surface as a tcgen05 GEMM over blocks of 128 envs; epilogue = total wavefront phase
@@ -30,7 +30,8 @@
 // split by the field warps, the stage-1 product by the stage-1 epilogue.  The stage-2 epilogue never writes the focal
 // plane: it projects it on the fibre modes (AO_env.py:471) out of TMEM.
 #include "tensor_path.cuh"
-#include "kernels_f64.cuh"
+#include "finalize.cuh"
+#include "philox.cuh"
 #include "fp32x2.cuh"
 #include "phase_round.cuh"
 
@@ -42,29 +43,19 @@
 #include <string>
 #include <vector>
 
-namespace {
-
-constexpr int TC_NP = 240;          // pupil pixels per side this path is built for
-constexpr int TC_NF = 128;          // focal pixels per side
-constexpr int TC_K = 2 * TC_NP;     // real-embedded contraction length (480)
-constexpr int KB = 32;              // K elements per pipeline stage (64 B rows, SWIZZLE_64B)
-constexpr int NUM_KB = TC_K / KB;   // 15
-constexpr int A_TILE = 128 * KB * 2;            // 8 KB: 128 rows x 64 B
-constexpr float PHI_ONE = 4194304.f;   // 2^22 fixed-point units per half-turn of phase
-
 struct TensorState {
   // operands (device)
-  __half* A1_hi = nullptr; __half* A1_lo = nullptr;   // [256][480]  stage-1 constant
-  __half* B2_hi = nullptr; __half* B2_lo = nullptr;   // [256][480]  stage-2 constant (N-major rows, K contiguous)
-  __half* T_hi = nullptr; __half* T_lo = nullptr;     // [chunk][128][480]  stage-1 product
-  float* lpw = nullptr;                               // [J][128][128] fibre modes * weight / max
-  float* lpwr = nullptr;                              // the same, [rank][v / 16][J][(v / 4) % 4][64 u][4 v] (stage-2 epilogue tiles)
-  double* coef4 = nullptr;                            // [chunk][J][re|im][rank] raw projection sums
+  DevArray<__half> A1_hi, A1_lo;                      // [256][480]  stage-1 constant
+  DevArray<__half> B2_hi, B2_lo;                      // [256][480]  stage-2 constant (N-major rows, K contiguous)
+  DevArray<__half> T_hi, T_lo;                        // [chunk][128][480]  stage-1 product
+  DevArray<float> lpw;                                // [J][128][128] fibre modes * weight / max
+  DevArray<float> lpwr;                               // the same, [rank][v / 16][J][(v / 4) % 4][64 u][4 v] (stage-2 epilogue tiles)
+  DevArray<double> coef4;                             // [chunk][J][re|im][rank] raw projection sums
   // atmospheric phase at lambda_wfs, UNREDUCED, int32 fixed point in units of 2^-22 half-turns (PHI_ONE per
   // half-turn; +-512 half-turns of range), tiled for the phase kernel's bulk prefetch:
   // [env / 32][Np xp][Np / 16 chunks][32 envs][16 pixels], ring-buffered in xp, the four 16-byte pieces of
   // each env row pre-swizzled (piece j at j ^ ((env >> 1) & 3)) so the shared-memory image is conflict free.
-  int32_t* hwt = nullptr;
+  DevArray<int32_t> hwt;
   // the same tiles as a 5-D tensor [env / 32][Np xp][Np / 16][32][16]: one box = the four 32-env tiles of a 128-env
   // block at one (column, chunk), 8 KB, for the shared prefetch of the phase kernel's lane groups
   CUtensorMap tmHwt;
@@ -72,33 +63,33 @@ struct TensorState {
   // [chunk][Np / 16 (y chunk)][Np x][16 y] (the 120 columns x 16 pixels one CTA needs per K block are one
   // contiguous 7.5 KB run): written by the phase kernel, read by the stage-1 kernel's field warps, which form
   // the pupil field on chip -- the field itself never goes to HBM.
-  float* phi = nullptr;
+  DevArray<float> phi;
   CUtensorMap tmPhi;
-  __half* modesK_hi = nullptr; __half* modesK_lo = nullptr;   // [Np x][Np y][KPAD] DM modes, k contiguous (GEMM B operand)
-  __half* act_hi = nullptr; __half* act_lo = nullptr;         // [chunk rows padded to 128][KPAD] actuators * 4 / lambda_wfs
-  uint16_t* apmask = nullptr;                         // [Np x][Np / 16] aperture bits of each 16-pixel column chunk
-  float2* R4 = nullptr;                               // [chunk][Np x][FK_PARTS][n] obs-arm column partial sums
-  float2* m1o32 = nullptr;                            // [n][Np] first obs-arm table in FP32
+  DevArray<__half> modesK_hi, modesK_lo;              // [Np x][Np y][KPAD] DM modes, k contiguous (GEMM B operand)
+  DevArray<__half> act_hi, act_lo;                    // [chunk rows padded to 128][KPAD] actuators * 4 / lambda_wfs
+  DevArray<uint16_t> apmask;                          // [Np x][Np / 16] aperture bits of each 16-pixel column chunk
+  DevArray<float2> R4;                                // [chunk][Np x][FK_PARTS][n] obs-arm column partial sums
+  DevArray<float2> m1o32;                             // [n][Np] first obs-arm table in FP32
   int kpad = 64;
   int act_rows = 128;
-  double2* m2oT = nullptr;                            // [n][Np] transposed obs table
-  int* err_flag = nullptr;                            // device alias of err_flag_host, set by a timed-out barrier wait
-  int* err_flag_host = nullptr;
+  DevArray<double2> m2oT;                             // [n][Np] transposed obs table
+  int* err_flag = nullptr;                            // not owned: device alias of err_flag_host, set by a timed-out barrier wait
+  PinnedArray<int> err_flag_host;
   // AOG_PRECISION_FUSED: per-pixel records [Np x][Np / 16][16 y][FK_NT(n)] float2 = [obs-arm twiddles m1o[v][y] |
   // fibre modes propagated back to the pupil, G_j = M1^T (mode_j w) M2^T / max|G| | (aperture, 0)], all times the
   // aperture: the 16 records of a column chunk are one contiguous run for the bulk prefetch
   bool fused = false;
   bool packed_valid = false;                          // act_hi / act_lo already hold this step's actuators (k_actuators_pack)
-  float2* gfib = nullptr;
+  DevArray<float2> gfib;
   double gfib_scale = 0.0;
-  double2* fib_part = nullptr;                        // [chunk][FK_SLOTS][FK_JT] partial projection sums
+  DevArray<double2> fib_part;                         // [chunk][FK_SLOTS][FK_JT] partial projection sums
   bool have_gfib = false, have_G = false;
   std::vector<double> h_m1, h_m2, h_lp, h_G, h_m1o, h_ap;   // host copies of the tables the records are built from
   // symmetric tables (kernel MODE 2, see FK_NF): G_j = e^{i theta_j} R_j; lpphase_f[j] = e^{i beta_j L} e^{i theta_j}
   bool sym = false, g_real = false, have_lpphase = false;
   double theta[AOG_MAX_LP] = {0};
   std::vector<double> h_lpphase;
-  double2* lpphase_f = nullptr;
+  DevArray<double2> lpphase_f;
   CUtensorMap tmA1_hi, tmA1_lo, tmB2_hi, tmB2_lo;
   CUtensorMap tmT128_hi, tmT128_lo;
   CUtensorMap tmTout_hi, tmTout_lo;                   // stage-1 epilogue stores: 128 rows x 16 columns, SWIZZLE_32B                   // stage-1 product, one env (128 rows) per box
@@ -109,13 +100,13 @@ struct TensorState {
   bool sh_have[6] = {false, false, false, false, false, false};   // fresnel, mla, offsets, index, x, y
   bool sh_ready = false, sh_unsupported = false;
   std::string sh_why;                                 // why the tables do not qualify (the FP64 kernels run instead)
-  __half* shCE_hi[2] = {nullptr, nullptr};            // [stage][2 parities][re | im][128 rows][256 K] operator embeddings
-  __half* shCE_lo[2] = {nullptr, nullptr};
-  __half* shEB_hi = nullptr; __half* shEB_lo = nullptr;   // [chunk][p][q][128 x][256 K] folded field
-  __half* shYB_hi = nullptr; __half* shYB_lo = nullptr;   // [chunk][q][p][128 i'][256 K] first product
-  float* shG = nullptr;                               // [chunk][p][q][128 i'][re 128 | im 128] second product
-  int16_t* shSlot = nullptr;                          // [P] lenslet slot of each camera pixel
-  double* shSlotC = nullptr;                          // [Nsub][3]
+  DevArray<__half> shCE_hi[2];                        // [stage][2 parities][re | im][128 rows][256 K] operator embeddings
+  DevArray<__half> shCE_lo[2];
+  DevArray<__half> shEB_hi, shEB_lo;                  // [chunk][p][q][128 x][256 K] folded field
+  DevArray<__half> shYB_hi, shYB_lo;                  // [chunk][q][p][128 i'][256 K] first product
+  DevArray<float> shG;                                // [chunk][p][q][128 i'][re 128 | im 128] second product
+  DevArray<int16_t> shSlot;                           // [P] lenslet slot of each camera pixel
+  DevArray<double> shSlotC;                           // [Nsub][3]
   double shScale[2] = {1.0, 1.0};                     // power-of-two scales of the two operator tables
   double shX0 = 0, shdX = 0, shY0 = 0, shdY = 0;
   CUtensorMap tmShCE_hi[2], tmShCE_lo[2], tmShEB_hi, tmShEB_lo, tmShYB_hi, tmShYB_lo, tmShYout_hi, tmShYout_lo;
@@ -126,7 +117,17 @@ struct TensorState {
   bool have_m1 = false, have_m2 = false, have_lp = false, have_modes = false, have_ap = false, have_m2o = false, have_m1o = false;
 };
 
-TensorState* TS(aog_env* env) { return reinterpret_cast<TensorState*>(env->tensor_state); }
+void TensorStateDeleter::operator()(TensorState* ts) const { delete ts; }
+
+namespace {
+
+constexpr int TC_NP = 240;          // pupil pixels per side this path is built for
+constexpr int TC_NF = 128;          // focal pixels per side
+constexpr int TC_K = 2 * TC_NP;     // real-embedded contraction length (480)
+constexpr int KB = 32;              // K elements per pipeline stage (64 B rows, SWIZZLE_64B)
+constexpr int NUM_KB = TC_K / KB;   // 15
+constexpr int A_TILE = 128 * KB * 2;            // 8 KB: 128 rows x 64 B
+constexpr float PHI_ONE = 4194304.f;   // 2^22 fixed-point units per half-turn of phase
 
 // ----------------------------------------------------------------------------- PTX wrappers
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
@@ -1766,6 +1767,214 @@ __global__ void k_screens_to_tiles(double* __restrict__ src, int32_t* __restrict
   hwt[o] = v;
 }
 
+// k_finalize_tcw<N, PARTS>: the epilogue of the tensor / fused paths, R4 holding PARTS partial column sums per
+// contraction index, with ONE WARP per env and no block-level barrier.  The kernel is bound by the LATENCY of fetching
+// the env's column partial sums (28.8 KB for the 5x5 detector), not by its arithmetic (DESIGN 4.6), so the partial
+// sums stream through shared memory: every warp keeps a
+// double-buffered ring of tiles (8 XS pupil columns = ~6 KB each, 16-byte cp.async, one commit group per tile) in
+// flight ahead of its arithmetic -- 16 warps per SM x 6-12 KB outstanding.
+// Lane (xs, b) = (lane / N, lane % N) owns column b of the column sums and the pupil columns x = xs, xs + XS, ...
+// (XS = 32 / N): per x it adds the PARTS partial sums of R[x][b] in FP64 and multiplies them with the N table
+// entries m[a][x] (broadcast loads), i.e. N complex accumulators per lane instead of N^2 -- no lane computes anything
+// twice.  The XS partial results per detector pixel meet in shared memory, summed in a fixed order by the lane that owns
+// the pixel.  Slot sums (fibre projections, Strehl) are loaded before the contraction and reduced after it.
+// Summation order depends on the env's data only: a batched env equals its single-env twin bit for bit.
+constexpr int FIN_WARPS = 8;
+template <int N, int PARTS> struct FinCfg {
+  static constexpr int XS = 32 / N, LANES = XS * N, N2 = N * N, N2P = N2 < 7 ? 7 : N2;
+  static constexpr int ITER = N >= 6 ? 4 : 8, TILE_X = XS * ITER, ROW = PARTS * N /* float2 per pupil column */;
+  static constexpr int TAB_MAX = N * 512 * 16;           // the [N][Np] table, Np <= 512 on the tensor / fused paths
+  static constexpr int TILE_BYTES = TILE_X * ROW * 8, WARP_BYTES = 2 * TILE_BYTES, SMEM = FIN_WARPS * WARP_BYTES;
+  static constexpr int RED_LD = 33;
+  static_assert(TILE_BYTES % 16 == 0, "tile size");
+  static_assert((2 * N * RED_LD + 2 * N2P) * 8 <= WARP_BYTES, "the reduction scratch aliases the tile ring");
+};
+template <int N, int PARTS>
+__global__ void __launch_bounds__(FIN_WARPS * 32, 2) k_finalize_tcw(FinalizeArgs a, int num_envs) {
+  using Cfg = FinCfg<N, PARTS>;
+  constexpr int XS = Cfg::XS, LANES = Cfg::LANES, N2 = Cfg::N2, ITER = Cfg::ITER, TILE_X = Cfg::TILE_X, ROW = Cfg::ROW;
+  extern __shared__ __align__(16) unsigned char fin_smem[];
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int b = blockIdx.x * FIN_WARPS + warp;
+  unsigned char* wbase = fin_smem + warp * Cfg::WARP_BYTES;
+  double2* tab_s = reinterpret_cast<double2*>(fin_smem + FIN_WARPS * Cfg::WARP_BYTES);   // [N][Np] second obs-arm table
+  constexpr unsigned FULL = 0xffffffffu;
+  const int ntiles = (a.Np + TILE_X - 1) / TILE_X;
+  const float2* r4 = a.R4 + (size_t)b * a.Np * ROW;
+  auto issue = [&](int t, int buf) {
+    const int cols = min(TILE_X, a.Np - t * TILE_X);
+    const int nchunks = cols * ROW / 2;                                // 16-byte pieces (cols is even)
+    const unsigned char* src = reinterpret_cast<const unsigned char*>(r4 + (size_t)t * TILE_X * ROW);
+    const unsigned dst = (unsigned)__cvta_generic_to_shared(wbase + buf * Cfg::TILE_BYTES);
+    for (int c = lane; c < nchunks; c += 32)
+      asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(dst + c * 16), "l"(src + (size_t)c * 16) : "memory");
+    asm volatile("cp.async.commit_group;" ::: "memory");
+  };
+  if (b < num_envs) {
+    issue(0, 0);
+    if (ntiles > 1) issue(1, 1);
+  }
+  // the table is read N times per (pupil column, lane): from global memory those loads were the kernel's stall
+  // (L1 hit rate 39 % next to 184 KB of shared memory; ncu: long scoreboard 6 of 14 warp-cycles per issue)
+  for (int i = threadIdx.x; i < N * a.Np; i += FIN_WARPS * 32) tab_s[i] = __ldg(a.m1o + i);
+  __syncthreads();
+  if (b >= num_envs) return;                            // warps are independent from here on
+  if (a.act) {
+    int bad = 0;
+    for (int k = lane; k < a.K; k += 32) bad |= isfinite(a.act[(size_t)b * a.K + k]) ? 0 : 1;   // inf: exp(i inf) = NaN too
+    if (__any_sync(FULL, bad)) {
+      asm volatile("cp.async.wait_group 0;" ::: "memory");
+      const double qnan = __longlong_as_double(0x7ff8000000000000LL);
+      for (int t = lane; t < N2; t += 32) {
+        if (a.obs64) a.obs64[(size_t)b * N2 + t] = qnan;
+        if (a.obs16) a.obs16[(size_t)b * N2 + t] = 0x7e00;
+      }
+      if (lane == 0 && a.compute_reward) {
+        if (a.reward) a.reward[b] = qnan;
+        if (a.power) a.power[b] = qnan;
+        if (a.strehl) a.strehl[b] = qnan;
+        if (a.ssim) a.ssim[b] = qnan;
+      }
+      return;
+    }
+  }
+  // per-lane partial slot sums (reduced after the contraction)
+  double2 cj[AOG_MAX_LP];
+  double2 sp = make_double2(0.0, 0.0);
+#pragma unroll
+  for (int j = 0; j < AOG_MAX_LP; ++j) cj[j] = make_double2(0.0, 0.0);
+  if (a.compute_reward) {
+    const int eb = b >> 7;
+    const int nslots = ((eb + 1) * a.slot_items - 1) / a.slot_ipc - (eb * a.slot_items) / a.slot_ipc + 1;
+    if (a.coef_is_raw == 2) {
+      if (lane == 0) {
+#pragma unroll
+        for (int j = 0; j < AOG_MAX_LP; ++j)
+          if (j < a.J) {
+            const double* c4 = a.coef4 + ((size_t)b * a.J + j) * 4;
+            cj[j] = make_double2(c4[0] + c4[1], c4[2] + c4[3]);
+          }
+      }
+    } else {
+      const double2* fp = a.fib_part + (size_t)b * a.fib_slots * a.fib_stride;
+      for (int i = lane; i < nslots; i += 32) {
+#pragma unroll
+        for (int j = 0; j < AOG_MAX_LP; ++j)
+          if (j < a.J) { const double2 v = fp[i * a.fib_stride + j]; cj[j].x += v.x; cj[j].y += v.y; }
+      }
+    }
+    if (a.rew_type == AOG_REW_STREHL_RATIO) {
+      const double2* spp = a.strehl_part + (size_t)b * a.strehl_blocks;
+      for (int i = lane; i < nslots; i += 32) { const double2 v = spp[i]; sp.x += v.x; sp.y += v.y; }
+    }
+  }
+  // contraction over the pupil columns
+  const int xs = lane / N, bb = lane - xs * N;
+  double are[N], aim[N];
+#pragma unroll
+  for (int v = 0; v < N; ++v) are[v] = aim[v] = 0.0;
+  for (int t = 0; t < ntiles; ++t) {
+    if (t + 1 < ntiles) asm volatile("cp.async.wait_group 1;" ::: "memory");
+    else                asm volatile("cp.async.wait_group 0;" ::: "memory");
+    __syncwarp();
+    const float2* tile = reinterpret_cast<const float2*>(wbase + (t & 1) * Cfg::TILE_BYTES);
+    if (lane < LANES) {
+#pragma unroll
+      for (int i = 0; i < ITER; ++i) {
+        const int xl = xs + XS * i, x = t * TILE_X + xl;
+        if (x < a.Np) {
+          double ex = 0.0, ey = 0.0;
+#pragma unroll
+          for (int qq = 0; qq < PARTS; ++qq) {
+            const float2 t4 = tile[(xl * PARTS + qq) * N + bb];
+            ex += (double)t4.x;
+            ey += (double)t4.y;
+          }
+#pragma unroll
+          for (int v = 0; v < N; ++v) {
+            const double2 m = tab_s[v * a.Np + x];
+            are[v] = fma(m.x, ex, fma(-m.y, ey, are[v]));
+            aim[v] = fma(m.x, ey, fma(m.y, ex, aim[v]));
+          }
+        }
+      }
+    }
+    __syncwarp();
+    if (t + 2 < ntiles) issue(t + 2, t & 1);
+  }
+  double* red = reinterpret_cast<double*>(wbase);               // [2 N][RED_LD]; the tile ring is drained
+  double* obs_s = red + 2 * N * Cfg::RED_LD;
+  double* win_s = obs_s + Cfg::N2P;
+#pragma unroll
+  for (int v = 0; v < N; ++v) { red[(2 * v) * Cfg::RED_LD + lane] = are[v]; red[(2 * v + 1) * Cfg::RED_LD + lane] = aim[v]; }
+  __syncwarp();
+  for (int t = lane; t < N2; t += 32) {
+    const int v = t / N, u = t - v * N;
+    double re = 0.0, im = 0.0;
+#pragma unroll
+    for (int s = 0; s < XS; ++s) { re += red[(2 * v) * Cfg::RED_LD + s * N + u]; im += red[(2 * v + 1) * Cfg::RED_LD + s * N + u]; }
+    const double fr = re * a.norm.x - im * a.norm.y, fi = re * a.norm.y + im * a.norm.x;
+    const double pw = (fr * fr + fi * fi) * a.obs_weight;
+    const int to = u * N + v;          // R4 and the table (M2o^T) hold the transposed contraction
+    obs_s[to] = pw;
+    if (a.obs64) a.obs64[(size_t)b * N2 + to] = pw;
+    if (a.obs16) a.obs16[(size_t)b * N2 + to] = __half_as_ushort(__double2half(pw));
+  }
+  __syncwarp();
+  if (!a.compute_reward) return;
+  // fibre: out = M (c e^{i beta L});  total power = c'^H G c'
+  double2 c[AOG_MAX_LP];
+#pragma unroll
+  for (int j = 0; j < AOG_MAX_LP; ++j) {
+    if (j < a.J) {
+      double2 s = make_double2(warp_sum(cj[j].x), warp_sum(cj[j].y));
+      s = make_double2(s.x * a.coef_scale.x - s.y * a.coef_scale.y, s.x * a.coef_scale.y + s.y * a.coef_scale.x);
+      const double2 ph = a.lpphase[j];
+      c[j] = make_double2(s.x * ph.x - s.y * ph.y, s.x * ph.y + s.y * ph.x);
+    } else {
+      c[j] = make_double2(0.0, 0.0);
+    }
+  }
+  double power = 0.0;
+#pragma unroll
+  for (int j = 0; j < AOG_MAX_LP; ++j)
+#pragma unroll
+    for (int k = 0; k < AOG_MAX_LP; ++k)
+      if (j < a.J && k < a.J) power += a.lpgram[j * a.J + k] * (c[j].x * c[k].x + c[j].y * c[k].y);
+  double reward;
+  if (a.rew_type == AOG_REW_STREHL_RATIO) {
+    const double sr = warp_sum(sp.x), si = warp_sum(sp.y);
+    const double strehl = a.strehl_scale * (sr * sr + si * si);
+    if (lane == 0 && a.strehl) a.strehl[b] = strehl;
+    reward = -(100.0 - strehl);
+  } else {
+    // skimage SSIM on 1-D data (ssim_1d, finalize.cuh), one window per lane, summed in window order
+    const double peak = a.ssim_peak, C1 = (0.01 * peak) * (0.01 * peak), C2 = (0.03 * peak) * (0.03 * peak);
+    const double cov_norm = 7.0 / 6.0;
+    constexpr int ref_idx = N2 / 2;
+    for (int cw = 3 + lane; cw < N2 - 3; cw += 32) {
+      double sx = 0, sxx = 0, sy = 0, syy = 0, sxy = 0;
+      for (int i = cw - 3; i <= cw + 3; ++i) {
+        const double x = obs_s[i], r = (i == ref_idx) ? peak : 0.0;
+        sx += x; sxx += x * x; sy += r; syy += r * r; sxy += x * r;
+      }
+      const double ux = sx / 7, uy = sy / 7, uxx = sxx / 7, uyy = syy / 7, uxy = sxy / 7;
+      const double vx = cov_norm * (uxx - ux * ux), vy = cov_norm * (uyy - uy * uy), vxy = cov_norm * (uxy - ux * uy);
+      win_s[cw] = ((2 * ux * uy + C1) * (2 * vxy + C2)) / ((ux * ux + uy * uy + C1) * (vx + vy + C2));
+    }
+    __syncwarp();
+    double tot = 0.0;
+    for (int cw = 3; cw < N2 - 3; ++cw) tot += win_s[cw];      // same summation order as ssim_1d
+    const double sv = tot / (double)(N2 - 6);
+    if (lane == 0 && a.ssim) a.ssim[b] = sv;
+    reward = 0.8 * power + (1.0 - 0.8) * sv;
+  }
+  if (lane != 0) return;
+  if (a.has_thr && reward < a.thr) reward = -1.0;
+  if (a.reward) a.reward[b] = reward;
+  if (a.power) a.power[b] = power;
+}
+
 // ----------------------------------------------------------------------------- host helpers
 typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
                                   const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
@@ -1834,13 +2043,6 @@ int make_map_hwt(aog_env* env, CUtensorMap* map, const int32_t* ptr, uint64_t bl
   return AOG_OK;
 }
 
-template <typename T>
-int talloc(aog_env* env, T** p, size_t count) {
-  if (*p) { cudaFree(*p); *p = nullptr; }
-  AOG_CUDA(cudaMalloc((void**)p, count * sizeof(T)));
-  return AOG_OK;
-}
-
 void split_half(double x, __half* hi, __half* lo) {
   const __half h = __float2half_rn((float)x);
   *hi = h;
@@ -1869,8 +2071,8 @@ int aog_tensor_create(aog_env* env) {
       !((NPc == 128 || NPc == 256 || NPc == 512) && (c.obs_dim == 2 || c.obs_dim == 5)))
     AOG_FAIL(AOG_ERR_UNSUPPORTED, "precision='fused' supports num_pupil_pixels=240 (any obs_dim <= 8) and 128 / 256 / 512 "
                                   "(obs_dim 2 or 5), with any focal grid; use precision='f64' for other grids");
-  TensorState* ts = new TensorState();
-  env->tensor_state = ts;
+  env->tensor.reset(new TensorState());
+  TensorState* ts = env->tensor.get();
   ts->fused = c.precision == AOG_PRECISION_FUSED;
   if (ts->fused && c.num_lp_modes > FK_JT)
     AOG_FAIL(AOG_ERR_UNSUPPORTED, "fused precision path holds at most 3 guided fibre modes; use precision='tensor'");
@@ -1881,50 +2083,50 @@ int aog_tensor_create(aog_env* env) {
   int rc;
 #define A(expr) if ((rc = (expr))) return rc
   if (!ts->fused) {
-    A(talloc(env, &ts->A1_hi, (size_t)256 * TC_K));
-    A(talloc(env, &ts->A1_lo, (size_t)256 * TC_K));
-    A(talloc(env, &ts->B2_hi, (size_t)256 * TC_K));
-    A(talloc(env, &ts->B2_lo, (size_t)256 * TC_K));
-    A(talloc(env, &ts->phi, ch * P));
+    A(ts->A1_hi.alloc(env, (size_t)256 * TC_K));
+    A(ts->A1_lo.alloc(env, (size_t)256 * TC_K));
+    A(ts->B2_hi.alloc(env, (size_t)256 * TC_K));
+    A(ts->B2_lo.alloc(env, (size_t)256 * TC_K));
+    A(ts->phi.alloc(env, ch * P));
     AOG_CUDA(cudaMemset(ts->phi, 0, ch * P * sizeof(float)));   // out-of-aperture chunks are never written (nor used)
     // stage-2 reads env pairs: keep one spare env of rows so the last odd pair stays in bounds
-    A(talloc(env, &ts->T_hi, (ch + 1) * 128 * TC_K));
-    A(talloc(env, &ts->T_lo, (ch + 1) * 128 * TC_K));
+    A(ts->T_hi.alloc(env, (ch + 1) * 128 * TC_K));
+    A(ts->T_lo.alloc(env, (ch + 1) * 128 * TC_K));
     AOG_CUDA(cudaMemset(ts->T_hi, 0, (ch + 1) * 128 * TC_K * sizeof(__half)));
     AOG_CUDA(cudaMemset(ts->T_lo, 0, (ch + 1) * 128 * TC_K * sizeof(__half)));
-    A(talloc(env, &ts->lpw, (size_t)c.num_lp_modes * env->NF2));
-    A(talloc(env, &ts->lpwr, (size_t)c.num_lp_modes * env->NF2));
-    A(talloc(env, &ts->coef4, ch * (size_t)c.num_lp_modes * 4));
+    A(ts->lpw.alloc(env, (size_t)c.num_lp_modes * env->NF2));
+    A(ts->lpwr.alloc(env, (size_t)c.num_lp_modes * env->NF2));
+    A(ts->coef4.alloc(env, ch * (size_t)c.num_lp_modes * 4));
   } else {
-    A(talloc(env, &ts->gfib, (size_t)P * FK_NT(c.obs_dim)));
+    A(ts->gfib.alloc(env, (size_t)P * FK_NT(c.obs_dim)));
     AOG_CUDA(cudaMemset(ts->gfib, 0, (size_t)P * FK_NT(c.obs_dim) * sizeof(float2)));
-    A(talloc(env, &ts->fib_part, ch * (size_t)FK_SLOTS * FK_JT));
-    A(talloc(env, &ts->lpphase_f, (size_t)AOG_MAX_LP));
+    A(ts->fib_part.alloc(env, ch * (size_t)FK_SLOTS * FK_JT));
+    A(ts->lpphase_f.alloc(env, (size_t)AOG_MAX_LP));
   }
   if (c.obs_dim > 8) AOG_FAIL(AOG_ERR_UNSUPPORTED, "tensor precision path supports obs_dim <= 8");
   ts->kpad = ((c.num_modes + 63) / 64) * 64;
   ts->act_rows = (int)((ch + 127) / 128) * 128;
   {
     const size_t tiles = ((B + 127) / 128) * 4 * NPc * (NPc / 16);       // whole 128-env blocks: the prefetch reads them all
-    A(talloc(env, &ts->hwt, tiles * 512));
+    A(ts->hwt.alloc(env, tiles * 512));
     AOG_CUDA(cudaMemset(ts->hwt, 0, tiles * 512 * sizeof(int32_t)));
     A(make_map_hwt(env, &ts->tmHwt, ts->hwt, tiles / ((size_t)NPc * (NPc / 16)), NPc));
     env->phase_tiles = ts->hwt;
     env->phase_tiles_unit = (double)PHI_ONE;
   }
-  A(talloc(env, &ts->modesK_hi, P * ts->kpad));
-  A(talloc(env, &ts->modesK_lo, P * ts->kpad));
-  A(talloc(env, &ts->act_hi, (size_t)ts->act_rows * ts->kpad));
-  A(talloc(env, &ts->act_lo, (size_t)ts->act_rows * ts->kpad));
+  A(ts->modesK_hi.alloc(env, P * ts->kpad));
+  A(ts->modesK_lo.alloc(env, P * ts->kpad));
+  A(ts->act_hi.alloc(env, (size_t)ts->act_rows * ts->kpad));
+  A(ts->act_lo.alloc(env, (size_t)ts->act_rows * ts->kpad));
   AOG_CUDA(cudaMemset(ts->act_hi, 0, (size_t)ts->act_rows * ts->kpad * sizeof(__half)));
   AOG_CUDA(cudaMemset(ts->act_lo, 0, (size_t)ts->act_rows * ts->kpad * sizeof(__half)));
-  A(talloc(env, &ts->apmask, (size_t)NPc * (NPc / 16)));
-  A(talloc(env, &ts->m1o32, (size_t)c.obs_dim * NPc));
-  A(talloc(env, &ts->R4, ch * NPc * FK_NSEG(NPc) * FK_PARTS * c.obs_dim));
-  A(talloc(env, &ts->m2oT, (size_t)c.obs_dim * NPc));
+  A(ts->apmask.alloc(env, (size_t)NPc * (NPc / 16)));
+  A(ts->m1o32.alloc(env, (size_t)c.obs_dim * NPc));
+  A(ts->R4.alloc(env, ch * NPc * FK_NSEG(NPc) * FK_PARTS * c.obs_dim));
+  A(ts->m2oT.alloc(env, (size_t)c.obs_dim * NPc));
   // barrier-timeout code: mapped pinned HOST memory, so that the host can still read it after the trap that follows
   // a timeout has poisoned the CUDA context (aog_health)
-  AOG_CUDA(cudaHostAlloc((void**)&ts->err_flag_host, sizeof(int), cudaHostAllocMapped));
+  AOG_CUDA(ts->err_flag_host.alloc(1, cudaHostAllocMapped));
   *ts->err_flag_host = 0;
   AOG_CUDA(cudaHostGetDevicePointer((void**)&ts->err_flag, ts->err_flag_host, 0));
   if (!ts->fused) {
@@ -1947,23 +2149,6 @@ int aog_tensor_create(aog_env* env) {
   AOG_CUDA(cudaFuncSetAttribute(k_mft2<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, M2_SMEM_BYTES));
   AOG_CUDA(cudaFuncSetAttribute(k_mft2<AOG_MAX_LP>, cudaFuncAttributeMaxDynamicSharedMemorySize, M2_SMEM_BYTES));
   return AOG_OK;
-}
-
-void aog_tensor_destroy(aog_env* env) {
-  TensorState* ts = TS(env);
-  if (!ts) return;
-  void* ptrs[] = {ts->A1_hi, ts->A1_lo, ts->B2_hi, ts->B2_lo, ts->phi, ts->T_hi, ts->T_lo, ts->lpw, ts->lpwr, ts->coef4,
-                  ts->hwt, ts->modesK_hi, ts->modesK_lo, ts->act_hi, ts->act_lo, ts->apmask, ts->m1o32, ts->R4,
-                  ts->m2oT, ts->gfib, ts->fib_part, ts->lpphase_f};
-  for (void* p : ptrs)
-    if (p) cudaFree(p);
-  void* shp[] = {ts->shCE_hi[0], ts->shCE_hi[1], ts->shCE_lo[0], ts->shCE_lo[1], ts->shEB_hi, ts->shEB_lo, ts->shYB_hi,
-                 ts->shYB_lo, ts->shG, ts->shSlot, ts->shSlotC};
-  for (void* p : shp)
-    if (p) cudaFree(p);
-  if (ts->err_flag_host) cudaFreeHost(ts->err_flag_host);
-  delete ts;
-  env->tensor_state = nullptr;
 }
 
 namespace {
@@ -2097,7 +2282,7 @@ int build_fused_records(aog_env* env, TensorState* ts) {
 int aog_tensor_sh_table(aog_env* env, int which, const void* host);   // sh_tensor.cuh
 
 int aog_tensor_table_updated(aog_env* env, int which, const void* host) {
-  TensorState* ts = TS(env);
+  TensorState* ts = env->tensor.get();
   const aog_config& c = env->cfg;
   const int Np = c.num_pupil_pixels, Nf = c.num_focal_pixels;     // the tensor-precision branches below run at 240 / 128 only
   if (which >= AOG_TABLE_SH_MLA_PHASE && which <= AOG_TABLE_SH_ACT0) return aog_tensor_sh_table(env, which, host);
@@ -2223,7 +2408,7 @@ int aog_tensor_table_updated(aog_env* env, int which, const void* host) {
 }
 
 int aog_tensor_screens_updated(aog_env* env) {
-  TensorState* ts = TS(env);
+  TensorState* ts = env->tensor.get();
   const int Np = env->cfg.num_pupil_pixels, B = env->cfg.num_envs;
   const double pi = 3.14159265358979323846;
   const size_t total = (size_t)((B + 127) / 128) * 4 * Np * (Np / 16) * 512;
@@ -2235,7 +2420,7 @@ int aog_tensor_screens_updated(aog_env* env) {
 }
 
 int aog_tensor_rescale_screens(aog_env* env, const double* factor_dev, cudaStream_t st) {
-  TensorState* ts = TS(env);
+  TensorState* ts = env->tensor.get();
   const int Np = env->cfg.num_pupil_pixels, B = env->cfg.num_envs;
   const double pi = 3.14159265358979323846;
   const size_t total = (size_t)((B + 127) / 128) * 4 * Np * (Np / 16) * 512;
@@ -2250,7 +2435,7 @@ int aog_tensor_rescale_screens(aog_env* env, const double* factor_dev, cudaStrea
 //   which = AOG_FIELD_TC_PUPIL : pupil field [y][x] complex (unit modulus x aperture)
 //   which = AOG_FIELD_TC_STAGE1: stage-1 product [v][x] complex (unit-modulus twiddles)
 int aog_tensor_get_field(aog_env* env, int which, int env_in_chunk, double* host_out, size_t count) {
-  TensorState* ts = TS(env);
+  TensorState* ts = env->tensor.get();
   if (!ts || ts->fused) AOG_FAIL(AOG_ERR_STATE, "handle has no matrix-Fourier-transform GEMM stages");
   if (env_in_chunk < 0 || env_in_chunk >= env->chunk) AOG_FAIL(AOG_ERR_INVALID, "env index outside the chunk");
   if (which == AOG_FIELD_TC_PUPIL) {          // phi [y / 16][x][16] radians -> out [y][x] = aperture exp(i phi)
@@ -2285,7 +2470,7 @@ int aog_tensor_get_field(aog_env* env, int which, int env_in_chunk, double* host
 // AO_env.py:115-120 for every env, with the DM-GEMM operand packed in the same kernel.  Returns AOG_ERR_UNSUPPORTED
 // (and launches nothing) when the handle runs more than one chunk or the Gram matrix does not fit shared memory.
 int aog_tensor_actuators(aog_env* env, const void* actions_dev, int act_dtype, cudaStream_t st) {
-  TensorState* ts = TS(env);
+  TensorState* ts = env->tensor.get();
   const aog_config& c = env->cfg;
   const int B = c.num_envs, K = c.num_modes;
   const size_t shm = ((size_t)K * K + 8 * (size_t)K) * sizeof(double);
@@ -2304,14 +2489,14 @@ int aog_tensor_actuators(aog_env* env, const void* actions_dev, int act_dtype, c
 }
 
 void aog_tensor_annotate_error(aog_env* env) {
-  TensorState* ts = env ? TS(env) : nullptr;
+  TensorState* ts = env ? env->tensor.get() : nullptr;
   if (!ts || !ts->err_flag_host) return;
   const int flag = *(volatile int*)ts->err_flag_host;
   if (flag) env->err += " [tensor pipeline barrier timeout, code " + std::to_string(flag) + ": the kernel trapped, this process's CUDA context is no longer usable]";
 }
 
 int aog_tensor_check(aog_env* env) {
-  TensorState* ts = TS(env);
+  TensorState* ts = env->tensor.get();
   if (!ts) return AOG_OK;
   const int flag = ts->err_flag_host ? *(volatile int*)ts->err_flag_host : 0;
   if (flag) AOG_FAIL(AOG_ERR_CUDA, "tensor pipeline barrier timeout, code " + std::to_string(flag) +
@@ -2404,7 +2589,7 @@ cudaError_t launch_finalize(int device, const FinalizeArgs& a, int nB, cudaStrea
 }  // namespace
 
 int aog_tensor_optics(aog_env* env, bool flat_dm, bool with_reward, const aog_outputs& out, cudaStream_t st) {
-  TensorState* ts = TS(env);
+  TensorState* ts = env->tensor.get();
   const aog_config& c = env->cfg;
   if (!(ts->have_m1 && ts->have_m2 && ts->have_lp && ts->have_modes && ts->have_ap && ts->have_m2o && ts->have_m1o) ||
       (ts->fused && !ts->have_gfib))
@@ -2418,7 +2603,7 @@ int aog_tensor_optics(aog_env* env, bool flat_dm, bool with_reward, const aog_ou
   int slot_ipc = 1;
   for (int e0 = 0; e0 < B; e0 += env->chunk) {
     const int nB = std::min(env->chunk, B - e0);
-    if (env->timing) { AOG_CUDA(cudaEventRecord(env->evf, st)); }
+    if (env->timing) { AOG_CUDA(cudaEventRecord(env->evf.get(), st)); }
     {
       // actuators -> half-turns of DM phase per unit mode (2 k s / pi = 4 s / lambda), split fp16
       const int rows = cdiv(nB, 128) * 128;
@@ -2451,7 +2636,7 @@ int aog_tensor_optics(aog_env* env, bool flat_dm, bool with_reward, const aog_ou
         sp.B = nB; sp.Np = Np; sp.kpad = ts->kpad; sp.col_origin = fp.col_origin; sp.env0 = e0;
         sp.ipc = cdiv(Np, std::min(ts->num_sms, FK_SLOTS));
         sp.sci_ratio_q32 = fp.sci_ratio_q32;
-        sp.hwt = ts->hwt; sp.apmask = ts->apmask; sp.gfib = reinterpret_cast<const float*>(ts->gfib);
+        sp.hwt = ts->hwt; sp.apmask = ts->apmask; sp.gfib = reinterpret_cast<const float*>(ts->gfib.get());
         sp.act_hi = ts->act_hi; sp.act_lo = ts->act_lo; sp.m_hi = ts->modesK_hi; sp.m_lo = ts->modesK_lo;
         sp.R4 = ts->R4; sp.strehl_part = env->strehl_part; sp.fib_part = ts->fib_part;
         slot_ipc = sp.ipc;
@@ -2462,7 +2647,7 @@ int aog_tensor_optics(aog_env* env, bool flat_dm, bool with_reward, const aog_ou
       else                  rc = strehl ? launch_phase_n<true, 0>(env, ts, fp, n, grid, st) : launch_phase_n<false, 0>(env, ts, fp, n, grid, st);
       if (rc) return rc;
     }
-    if (env->timing) { AOG_CUDA(cudaEventRecord(env->ev0, st)); }
+    if (env->timing) { AOG_CUDA(cudaEventRecord(env->ev0.get(), st)); }
     const int max_clusters = ts->num_sms / 2;
     int tc_dbg = 0;
     { const char* d = getenv("AOG_TC_DEBUG"); tc_dbg = d ? atoi(d) : 0; }
@@ -2481,7 +2666,7 @@ int aog_tensor_optics(aog_env* env, bool flat_dm, bool with_reward, const aog_ou
                                                                                    ts->tmTout_hi, ts->tmTout_lo, f1);
       AOG_LAUNCH_CHECK();
     }
-    if (env->timing) { AOG_CUDA(cudaEventRecord(env->evm, st)); }
+    if (env->timing) { AOG_CUDA(cudaEventRecord(env->evm.get(), st)); }
     if (with_reward && !fused) {
       TcParams p{};
       p.num_envs = nB;
@@ -2498,7 +2683,7 @@ int aog_tensor_optics(aog_env* env, bool flat_dm, bool with_reward, const aog_ou
             ts->tmB2_hi, ts->tmB2_lo, ts->tmT128_hi, ts->tmT128_lo, p);
       AOG_LAUNCH_CHECK();
     }
-    if (env->timing) { AOG_CUDA(cudaEventRecord(env->ev1, st)); env->ev_valid = true; }
+    if (env->timing) { AOG_CUDA(cudaEventRecord(env->ev1.get(), st)); env->ev_valid = true; }
     FinalizeArgs a{};
     a.R4 = ts->R4; a.m1o = ts->m2oT;
     {

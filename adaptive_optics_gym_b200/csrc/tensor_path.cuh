@@ -3,7 +3,6 @@
 #include "common.cuh"
 
 int aog_tensor_create(aog_env* env);
-void aog_tensor_destroy(aog_env* env);
 int aog_tensor_table_updated(aog_env* env, int which, const void* host);
 int aog_tensor_screens_updated(aog_env* env);
 // every env's screen times factor_dev[env] (device [B]) and its phase tiles rewritten, stream-ordered on st

@@ -1,8 +1,11 @@
 """CPU: libaogym.so loads and exports every symbol include/aogym.h declares; the ctypes structs
 mirror the header (no compute calls -- there is no GPU here)."""
+import collections
 import ctypes
 import os
 import re
+import shutil
+import subprocess
 
 import pytest
 
@@ -35,6 +38,20 @@ def test_every_declared_symbol_is_exported(lib):
     for s in declared_symbols():
         assert hasattr(lib, s), f'{s} declared in include/aogym.h but not exported by libaogym.so'
     assert b'sm_100a' in lib.aog_version()
+
+
+def test_each_kernel_is_compiled_once(lib):
+    """A header that defines kernels and is included by both translation units builds (and ships) each of them twice:
+    every kernel name must appear once in the library's SASS."""
+    from adaptive_optics_gym_b200 import _lib
+    cuobjdump = shutil.which('cuobjdump') or '/usr/local/cuda/bin/cuobjdump'
+    if not os.path.exists(cuobjdump):
+        pytest.skip('cuobjdump not found')
+    sass = subprocess.run([cuobjdump, '-sass', _lib.LIB_PATH], check=True, capture_output=True, text=True).stdout
+    names = re.findall(r'Function : (\S+)', sass)
+    assert names, 'no kernels found in the SASS dump'
+    twice = sorted(n for n, k in collections.Counter(names).items() if k > 1)
+    assert not twice, f'{len(twice)} kernels compiled more than once: {twice}'
 
 
 def test_ctypes_structs_mirror_header():

@@ -10,7 +10,7 @@ SYNTH_KEY_XOR = 0x9E3779B97F4A7C15          # aog_generate_screens: the synthesi
 
 def philox4x32_10(counter, key):
     """Philox-4x32-10 (Salmon et al. 2011) in uint64 arithmetic: counter [..., 4], key [..., 2] uint32 words ->
-    [..., 4] uint32, the rounds of aog_philox4x32_10 (csrc/kernels_f64.cuh)."""
+    [..., 4] uint32, the rounds of aog_philox4x32_10 (csrc/philox.cuh)."""
     c = np.asarray(counter, dtype=np.uint64)
     k = np.asarray(key, dtype=np.uint64)
     c0, c1, c2, c3 = (c[..., i].copy() for i in range(4))
